@@ -69,7 +69,41 @@ def parse_args():
     ap.add_argument("--sweep-worlds", type=int, default=65536, help="BASELINE config 5: total worlds of the sweep (0: skip)")
     ap.add_argument("--sweep-seconds", type=float, default=45.0, help="wall-clock box of the sweep per rank")
     ap.add_argument("--no-configs", action="store_true", help="skip the config 1 / 3 / 4 objects")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps write g and the dense Jacobian of the last k-iterate of the last step as "
+                         "DIR/g.npy and DIR/jac.npy (float64; rank 0's worlds, a fixed sample of them beyond 64 MB)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the b200 timed path")
+    return args
+
+
+DUMP_BYTES = 64 * 10 ** 6
+
+
+def dump_sample(nprob, m):
+    """Worlds whose g [m] and dense Jacobian [m, 7] --dump-outputs writes: all of them when they fit in DUMP_BYTES (less
+    room for the .npy headers), else a sorted sample drawn with a fixed seed, so that runs with the same arguments write
+    the same worlds."""
+    n = min(nprob, (DUMP_BYTES - 1024) // (8 * m * (1 + NF)))
+    if n < 1:
+        raise SystemExit(f"bench.py: g and the Jacobian of one world ({m} constraints) exceed {DUMP_BYTES} bytes")
+    if n == nprob:
+        return np.arange(nprob)
+    return np.sort(np.random.default_rng(0).choice(nprob, n, replace=False))
+
+
+def dump_outputs(out_dir, d_g, d_j):
+    """What the timed step hands its caller (g [nprob, m] and the dense Jacobian [nprob, m, 7] of its last k-iterate,
+    on the device) for the worlds of dump_sample, as float64 .npy files."""
+    import torch
+
+    sel = torch.as_tensor(dump_sample(*d_g.shape), device=d_g.device)
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "g.npy"), d_g[sel].cpu().numpy())
+    np.save(os.path.join(out_dir, "jac.npy"), d_j[sel].cpu().numpy())
 
 
 _WORLDS = None
@@ -741,6 +775,8 @@ def run_b200(args):
     per_rank_dev = list(timed.per_rank)
     clock_windows = [(c0, c1)]
     value = world * nprob * iters * args.steps / (ms_dev * 1e-3)
+    if args.dump_outputs and rank == 0:  # before anything below overwrites d_g / d_j
+        dump_outputs(args.dump_outputs, d_g, d_j)
 
     # verdicts of the last iterate (on the device), gathered as counts: the only cross-rank traffic
     d_ok = torch.empty(nprob, dtype=torch.int32, device=dev)
@@ -1013,6 +1049,7 @@ def run_b200(args):
 
 def main():
     args = parse_args()
+    sys.dont_write_bytecode = True  # the tree may be read-only: no __pycache__ beside the modules imported from here on
     if args.impl == "reference":
         return run_reference(args)
     return run_b200(args)
