@@ -11,8 +11,8 @@ _lib.load()  # no CPU fallback: a missing extension is an ImportError here
 
 from .planner import ReachSetEngine  # noqa: E402
 from .controller import RobustController  # noqa: E402
-from .armtd import ArmtdPlanner  # noqa: E402
+from .armtd import ArmtdBatch, ArmtdPlanner  # noqa: E402
 from . import worlds  # noqa: E402
 from . import sharding  # noqa: E402
 
-__all__ = ["ReachSetEngine", "RobustController", "ArmtdPlanner", "ArmourError", "NF", "worlds", "sharding"]
+__all__ = ["ReachSetEngine", "RobustController", "ArmtdPlanner", "ArmtdBatch", "ArmourError", "NF", "worlds", "sharding"]

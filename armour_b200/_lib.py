@@ -131,6 +131,16 @@ SIGNATURES.update({
     "armour_armtd_cost": (C.c_int, [C.c_void_p, dp, dp, dp, dp]),
     "armour_armtd_get_link_sliced_center": (C.c_int, [C.c_void_p, dp]),
     "armour_armtd_get_link_independent_generators": (C.c_int, [C.c_void_p, dp]),
+    "armour_armtd_batch_ctx_create": (C.c_int, [C.POINTER(Config), C.POINTER(C.c_void_p)]),
+    "armour_armtd_batch_build": (C.c_int, [C.c_void_p, C.c_int, dp, dp, dp, dp, dp, C.c_int]),
+    "armour_armtd_batch_build_device": (C.c_int, [C.c_void_p, C.c_int] + [C.c_void_p] * 5 + [C.c_int, C.c_void_p]),
+    "armour_armtd_batch_eval": (C.c_int, [C.c_void_p, C.c_int, dp, dp, dp]),
+    "armour_armtd_batch_eval_device": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "armour_armtd_batch_verdict_device": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "armour_armtd_batch_cost": (C.c_int, [C.c_void_p, C.c_int, dp, dp, dp, dp]),
+    "armour_armtd_batch_get_link_independent_generators": (C.c_int, [C.c_void_p, C.c_int, dp]),
+    "armour_armtd_batch_solve": (C.c_int, [C.c_void_p, C.c_int, dp, C.c_void_p, dp, ip, ip, ip]),
+    "armour_armtd_batch_solve_device": (C.c_int, [C.c_void_p, C.c_int] + [C.c_void_p] * 6),
 })
 
 

@@ -513,6 +513,10 @@ K1_DI PZ8 make_link_box(int top, int i) {
     top = end_of<SZ>(h);      \
     top_max = top > top_max ? top : top_max
 
+// FK_ONLY: the ARMTD comparison planner (B.jrs_ext set): forward kinematics only, as mg_task_list_fk in the latency
+// configuration; with an imported joint reachable set the Newton-Euler pass would run on meaningless Bezier models.  A template
+// parameter rather than a test of B.jrs_ext, so that the main planner's kernel is the same code as without the ARMTD path.
+template <bool FK_ONLY>
 K1_DI int build_unit(const Batch& B, int p, int t) {
     const RobotConstants& rc = c_robot;
     K1S& S = k1s();
@@ -553,6 +557,7 @@ K1_DI int build_unit(const Batch& B, int p, int t) {
             FK_R = FK_R2;
         }
     }
+    if (FK_ONLY) return top_max;
 
     // ---- recursive Newton-Euler, forward pass (KPR/Dynamics.cu:83-155) ----
     top = B0;
@@ -1080,7 +1085,9 @@ static_assert(!MG, "K1_JRS_GLOBAL is a knob of the throughput configuration");
 constexpr int K1_FIXED_BYTES = K1S_BYTES + JRS_WORDS * 8;  // per group: control block + joint reachable set region
 #endif
 
-__global__ void __launch_bounds__(NT * GROUPS, CTAS_PER_SM) k_reachsets(K1Params P) {
+// FK_ONLY (throughput configuration only): see build_unit; the latency configuration reads B.jrs_ext for its task list
+template <bool FK_ONLY>
+K1_DI void reachsets_body(const K1Params& P) {
 #ifndef ARMOUR_EMU
     // a kernel launched behind this one with programmatic stream serialisation (k_hyperplanes in the latency path) may
     // start as soon as every CTA of this grid is resident; it synchronises on P.unit_flag, not on this grid's end
@@ -1220,7 +1227,7 @@ __global__ void __launch_bounds__(NT * GROUPS, CTAS_PER_SM) k_reachsets(K1Params
 #ifdef K1_PROFILE
         const long long _u0 = clock64();
 #endif
-        const int tm = build_unit(P.B, p, t);
+        const int tm = build_unit<FK_ONLY>(P.B, p, t);
 #ifdef K1_PROFILE
         if (tid == 0) {
             g_k1prof[(size_t(t) * K1_PROF_SITES + K1_PROF_SITES - 1) * 2] += clock64() - _u0;
@@ -1274,6 +1281,12 @@ __global__ void __launch_bounds__(NT * GROUPS, CTAS_PER_SM) k_reachsets(K1Params
         atomicAdd(&P.stats[3], ndone);
     }
 }
+
+__global__ void __launch_bounds__(NT * GROUPS, CTAS_PER_SM) k_reachsets(K1Params P) { reachsets_body<false>(P); }
+#if !K1_MG
+// the ARMTD comparison planner's build (B.jrs_ext set) in the throughput configuration: forward kinematics only
+__global__ void __launch_bounds__(NT * GROUPS, CTAS_PER_SM) k_reachsets_fk(K1Params P) { reachsets_body<true>(P); }
+#endif
 
 #ifndef ARMOUR_EMU
 // ---- host side: scratch buffers and launch ----------------------------------------------------------
@@ -1350,6 +1363,10 @@ inline cudaError_t k1_scratch_create(K1Scratch* s, const armour_config& cfg, con
         if ((e = cudaMalloc(&s->mbox, size_t(s->grid) * MB_SLOTS * s->mbox_words * 8)) != cudaSuccess) return e;
     }
     if ((e = cudaMemsetAsync(s->stats, 0, 4 * sizeof(int), st)) != cudaSuccess) return e;
+#if !K1_MG
+    if ((e = cudaFuncSetAttribute(k_reachsets_fk, cudaFuncAttributeMaxDynamicSharedMemorySize, int(s->smem_bytes))) != cudaSuccess)
+        return e;
+#endif
     return cudaFuncSetAttribute(k_reachsets, cudaFuncAttributeMaxDynamicSharedMemorySize, int(s->smem_bytes));
 }
 
@@ -1377,6 +1394,13 @@ inline cudaError_t launch_reachsets(const Batch& B, K1Scratch& s, cudaStream_t s
     P.nunits = 0;
     const int ntiles = MG ? B.nprob * B.T : (B.nprob * B.T + GROUPS - 1) / GROUPS;
     const int grid = ntiles < s.grid ? ntiles : s.grid;
+#if !K1_MG
+    if (B.jrs_ext) {
+        k_reachsets_fk<<<grid, NT * GROUPS, s.smem_bytes, st>>>(P);
+        *nlaunch = 1;
+        return cudaGetLastError();
+    }
+#endif
     k_reachsets<<<grid, NT * GROUPS, s.smem_bytes, st>>>(P);
     *nlaunch = 1;
     return cudaGetLastError();

@@ -13,6 +13,11 @@
 // region (the CTA searches the most violated row, one thread does the 7 x 7 algebra of taking it in), then accepts /
 // rejects on (violation, cost).  Per iteration: k_constraints (g, J at x),
 // k_solver_step, k_constraints (g at the trial point), k_solver_accept.
+//
+// The kernels are templates over an NLP policy: m(B) rows per problem, row_bounds(B, p, i, ...) = bounds and acceptance
+// tolerance of row i, cost(B, p, q_des, k, grad) = cost and its gradient.  ArmourNlp below is the main planner's armtd_NLP;
+// ArmtdNlp (csrc/armtd.cuh) is the one of the ARMTD comparison planner, whose evaluation step assembles KPA's row layout
+// behind k_constraints.
 #pragma once
 #include <cuda_runtime.h>
 
@@ -110,6 +115,17 @@ __device__ __forceinline__ void solver_row_bounds(const Batch& B, int p, int i, 
     }
 }
 
+// the main planner's NLP (KPR/NLPclass.cu)
+struct ArmourNlp {
+    __device__ int m(const Batch& B) const { return B.m(); }
+    __device__ void row_bounds(const Batch& B, int p, int i, double ttol, double ctol, double* gl, double* gu, double* tol) const {
+        solver_row_bounds(B, p, i, ttol, ctol, gl, gu, tol);
+    }
+    __device__ double cost(const Batch& B, int p, const double* q_des, const double* k, double* grad) const {
+        return solver_cost(B, p, q_des, k, grad);
+    }
+};
+
 // block-wide maximum (all threads get it)
 __device__ inline double solver_block_max(double v, double* s_red) {
     for (int o = 16; o > 0; o >>= 1) v = fmax(v, __shfl_xor_sync(0xffffffffu, v, o));
@@ -121,12 +137,14 @@ __device__ inline double solver_block_max(double v, double* s_red) {
     return r;
 }
 // violation with the verdict's tolerances folded in: <= 0 means "finalize_solution would accept"
-__device__ inline double solver_violation(const Batch& B, int p, const double* g, double ttol, double ctol, double* s_red) {
-    const int m = B.m();
+template <class Nlp>
+__device__ inline double solver_violation(const Batch& B, const Nlp& nlp, int p, const double* g, double ttol, double ctol,
+                                          double* s_red) {
+    const int m = nlp.m(B);
     double v = -1e300;
     for (int i = threadIdx.x; i < m; i += SOLVER_THREADS) {
         double gl, gu, tol;
-        solver_row_bounds(B, p, i, ttol, ctol, &gl, &gu, &tol);
+        nlp.row_bounds(B, p, i, ttol, ctol, &gl, &gu, &tol);
         v = fmax(v, g[i] - gu - tol);
         if (gl > -1e18) v = fmax(v, gl - g[i] - tol);
     }
@@ -134,14 +152,15 @@ __device__ inline double solver_violation(const Batch& B, int p, const double* g
 }
 
 // start: x = 0 (armtd_NLP::get_starting_point), cost and violation there from g(0)
-__global__ void __launch_bounds__(SOLVER_THREADS) k_solver_start(Batch B, SolverState S, const double* __restrict__ g) {
+template <class Nlp>
+__global__ void __launch_bounds__(SOLVER_THREADS) k_solver_start(Batch B, Nlp nlp, SolverState S, const double* __restrict__ g) {
     const int p = blockIdx.x;
     __shared__ double s_red[SOLVER_THREADS / 32];
-    const double viol = solver_violation(B, p, g + size_t(p) * B.m(), S.torque_tol, S.collision_tol, s_red);
+    const double viol = solver_violation(B, nlp, p, g + size_t(p) * nlp.m(B), S.torque_tol, S.collision_tol, s_red);
     if (threadIdx.x == 0) {
         double x[NF];
         for (int j = 0; j < NF; j++) x[j] = S.x[size_t(p) * NF + j];
-        const double f = solver_cost(B, p, S.q_des + size_t(p) * NF, x, nullptr);
+        const double f = nlp.cost(B, p, S.q_des + size_t(p) * NF, x, nullptr);
         S.f[p] = f;
         S.viol[p] = viol;
         S.have_best[p] = viol <= 0;
@@ -172,14 +191,15 @@ __device__ __forceinline__ void solver_load_row(const double* rows, int i, doubl
 }
 
 // one SQP step from (g, J) at x: writes the trial point xt, or ends the problem (step below tolerance)
+template <class Nlp>
 __global__ void __launch_bounds__(SOLVER_THREADS)
-k_solver_step(Batch B, SolverState S, const double* __restrict__ g_all, const double* __restrict__ jac_all, int it) {
+k_solver_step(Batch B, Nlp nlp, SolverState S, const double* __restrict__ g_all, const double* __restrict__ jac_all, int it) {
     const int p = B.plist ? B.plist[blockIdx.x] : int(blockIdx.x), tid = threadIdx.x;
     if (S.status[p] != SOLVER_RUNNING) return;  // uniform per CTA
 #ifdef SOLVER_PROFILE
     const long long pc0 = clock64();
 #endif
-    const int m = B.m();
+    const int m = nlp.m(B);
     const double* g = g_all + size_t(p) * m;
     const double* J = jac_all + size_t(p) * m * NF;
     __shared__ double s_x[NF], s_gf[NF], s_h, s_delta;
@@ -188,14 +208,14 @@ k_solver_step(Batch B, SolverState S, const double* __restrict__ g_all, const do
         double x[NF], gf[NF], xt[NF];
         for (int j = 0; j < NF; j++) x[j] = S.x[size_t(p) * NF + j];
         const double* qd = S.q_des + size_t(p) * NF;
-        solver_cost(B, p, qd, x, gf);
+        nlp.cost(B, p, qd, x, gf);
         // curvature of the cost along the gradient from one extra evaluation (exact for the planner's quadratic cost)
         double h = 1.0, gn2 = 0;
         for (int j = 0; j < NF; j++) gn2 += gf[j] * gf[j];
         if (gn2 > 0) {
             const double eps = 1e-3 / sqrt(gn2);
             for (int j = 0; j < NF; j++) xt[j] = x[j] - eps * gf[j];
-            const double f2 = solver_cost(B, p, qd, xt, nullptr);
+            const double f2 = nlp.cost(B, p, qd, xt, nullptr);
             const double curv = 2.0 * (f2 - S.f[p] + eps * gn2) / (eps * eps * gn2);
             if (curv > 1e-8) h = curv;
         }
@@ -229,7 +249,7 @@ k_solver_step(Batch B, SolverState S, const double* __restrict__ g_all, const do
             pu[q] = pl[q] = false;
             if (st0 + q < steps && i < m) {
                 double gl, gu, tol;
-                solver_row_bounds(B, p, i, S.torque_tol, S.collision_tol, &gl, &gu, &tol);
+                nlp.row_bounds(B, p, i, S.torque_tol, S.collision_tol, &gl, &gu, &tol);
                 tol *= 0.5;  // aim inside the acceptance band
                 double l1 = 0;
                 for (int j = 0; j < NF; j++) l1 += fabs(J[size_t(i) * NF + j]);
@@ -268,7 +288,7 @@ k_solver_step(Batch B, SolverState S, const double* __restrict__ g_all, const do
         if (ku || kl) {
             const int i = w0 + st * 32 + lane;
             double gl, gu, tol;
-            solver_row_bounds(B, p, i, S.torque_tol, S.collision_tol, &gl, &gu, &tol);
+            nlp.row_bounds(B, p, i, S.torque_tol, S.collision_tol, &gl, &gu, &tol);
             tol *= 0.5;
             double a[NF];
             for (int j = 0; j < NF; j++) a[j] = J[size_t(i) * NF + j];
@@ -393,15 +413,17 @@ k_solver_step(Batch B, SolverState S, const double* __restrict__ g_all, const do
 
 // acceptance test of the trial point from g(xt): filter-style — feasible points must lower the cost, infeasible ones
 // must lower the violation
-__global__ void __launch_bounds__(SOLVER_THREADS) k_solver_accept(Batch B, SolverState S, const double* __restrict__ gt_all, int last) {
+template <class Nlp>
+__global__ void __launch_bounds__(SOLVER_THREADS) k_solver_accept(Batch B, Nlp nlp, SolverState S, const double* __restrict__ gt_all,
+                                                                  int last) {
     const int p = B.plist ? B.plist[blockIdx.x] : int(blockIdx.x);
     if (S.status[p] != SOLVER_RUNNING) return;
     __shared__ double s_red[SOLVER_THREADS / 32];
-    const double vt = solver_violation(B, p, gt_all + size_t(p) * B.m(), S.torque_tol, S.collision_tol, s_red);
+    const double vt = solver_violation(B, nlp, p, gt_all + size_t(p) * nlp.m(B), S.torque_tol, S.collision_tol, s_red);
     if (threadIdx.x == 0) {
         double xt[NF];
         for (int j = 0; j < NF; j++) xt[j] = S.xt[size_t(p) * NF + j];
-        const double ft = solver_cost(B, p, S.q_des + size_t(p) * NF, xt, nullptr);
+        const double ft = nlp.cost(B, p, S.q_des + size_t(p) * NF, xt, nullptr);
         S.evals[p] += 1;
         const double f = S.f[p], viol = S.viol[p];
         const bool accept = (vt <= 0 && (viol > 0 || ft < f - 1e-12)) || (vt > 0 && viol > 0 && vt < viol - 1e-12);

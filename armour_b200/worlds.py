@@ -161,6 +161,42 @@ def armtd_offline_jrs(qd0, k_range, T=ARMTD_T):
     return out
 
 
+def armtd_offline_jrs_batch(qd0, k_range, T=ARMTD_T):
+    """armtd_offline_jrs for n problems at once: qd0, k_range [n, 7] -> [n, 6, 7, T], the same arithmetic vectorised over the
+    problems and the intervals."""
+    qd0 = np.asarray(qd0, dtype=np.float64)[:, :, None]          # [n, 7, 1]
+    k_range = np.asarray(k_range, dtype=np.float64)[:, :, None]
+    j = np.arange(T, dtype=np.float64)
+    t0, t1 = j / T, (j + 1) / T                                   # [T]
+
+    def coeffs(t):  # as armtd_offline_jrs: q_des - q0 = A(t) + B(t) * k_a, t [T] -> A [n, 7, T], B [1, 1, T]
+        tau = t - 0.5
+        A = np.where(t <= 0.5, qd0 * t, qd0 * 0.5 + qd0 * tau - qd0 * tau * tau)
+        B = np.where(t <= 0.5, 0.5 * t * t, 0.125 + 0.5 * tau - 0.5 * tau * tau)[None, None, :]
+        return A, B
+
+    A, B = coeffs(0.5 * (t0 + t1))
+    c_cos, c_sin = np.cos(A), np.sin(A)
+    g_cos, g_sin = -np.sin(A) * B * k_range, np.cos(A) * B * k_range
+    r_cos, r_sin = np.zeros_like(A), np.zeros_like(A)
+    for s in np.linspace(0.0, 1.0, 9):
+        At, Bt = coeffs(t0 + s * (t1 - t0))
+        for k in np.linspace(-1.0, 1.0, 33):
+            d = At + Bt * k_range * k
+            r_cos = np.maximum(r_cos, np.abs(np.cos(d) - (c_cos + g_cos * k)))
+            r_sin = np.maximum(r_sin, np.abs(np.sin(d) - (c_sin + g_sin * k)))
+    return np.stack([c_cos, g_cos, 1.1 * r_cos + 1e-6, c_sin, g_sin, 1.1 * r_sin + 1e-6], axis=1)
+
+
+def armtd_random_problems(nprob, nobs, seed=20261017):
+    """A sweep of comparison-planner problems: the start states, waypoints and `nobs` random boxes of random_problems(nprob,
+    nobs, seed) with the synthetic offline JRS of each start velocity.  Returns q0, qd0, q_des, k_range [n, 7], jrs [n, 6, 7, 100]
+    and obstacles [n, nobs, 12]."""
+    q0, qd0, _, q_des, obs = random_problems(nprob, nobs, seed)
+    k_range = armtd_k_range(qd0)
+    return q0, qd0, q_des, k_range, armtd_offline_jrs_batch(qd0, k_range), obs
+
+
 def armtd_problem(path, seed=0):
     """A planning problem of the comparison planner from a saved world: start from the CSV, a random initial velocity,
     straight-line waypoint, the synthetic offline JRS.  Returns q0, qd0, q_des, jrs[6, 7, T], k_range, obstacles."""
