@@ -150,6 +150,32 @@ class SolverOptions(C.Structure):
                 ("qp_sweeps", C.c_int), ("qp_update_budget", C.c_int)]
 
 
+class RolloutOptions(C.Structure):
+    """armour_rollout_options (include/armour_b200.h)."""
+    _fields_ = [("struct_size", C.c_int), ("max_replans", C.c_int), ("lookahead", C.c_double), ("goal_radius", C.c_double),
+                ("audit_samples", C.c_int), ("solver", SolverOptions)]
+
+
+class RolloutOut(C.Structure):
+    """armour_rollout_out (include/armour_b200.h): output arrays, any may be NULL."""
+    _fields_ = [("outcome", ip), ("replans", ip), ("infeasible", ip), ("final_state", dp), ("min_clearance", dp),
+                ("log_state", dp), ("log_q_des", dp), ("log_k", dp), ("log_int", ip), ("log_clearance", dp)]
+
+
+# outcome of a closed-loop episode (ARMOUR_ROLLOUT_*)
+ROLLOUT_BUDGET, ROLLOUT_ARRIVED, ROLLOUT_COLLISION, ROLLOUT_LIMIT = 0, 1, 2, 3
+
+SIGNATURES.update({
+    "armour_rollout_options_default": (None, [C.POINTER(RolloutOptions)]),
+    "armour_batch_rollout_device": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int,
+                                              C.POINTER(RolloutOptions), C.POINTER(RolloutOut)]),
+    "armour_batch_rollout": (C.c_int, [C.c_void_p, C.c_int, dp, dp, dp, C.c_int, C.POINTER(RolloutOptions),
+                                       C.POINTER(RolloutOut)]),
+    "armour_batch_clearance_device": (C.c_int, [C.c_void_p, C.c_int] + [C.c_void_p] * 3 + [C.c_int, C.c_void_p, C.c_void_p]),
+    "armour_batch_clearance": (C.c_int, [C.c_void_p, C.c_int, dp, ip, dp, C.c_int, dp, ip]),
+})
+
+
 _LIB = None
 
 

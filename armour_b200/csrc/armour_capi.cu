@@ -100,6 +100,7 @@ __device__ int g_k1spill[8];  // arena blocks in global memory, all arena blocks
 #include "k3_constraints.cuh"
 #include "k4_solver.cuh"
 #include "armtd.cuh"
+#include "rollout.cuh"
 #include "layout.h"
 
 using namespace armour;
@@ -149,6 +150,12 @@ struct armour_ctx {
     double* d_ja = nullptr;        // [nprob][m_armtd][NF]
     size_t ga_capacity = 0, ja_capacity = 0;
     std::vector<double> h_krange;  // host mirror of d_krange for the cost (empty: fetched after a device build)
+    // closed-loop episodes (armour_batch_rollout*) and clearance queries (allocated on first use, grow only)
+    double* d_roll = nullptr;   // per-world state, current plans and the dense batch of a rollout
+    int* d_roll_i = nullptr;    // outcomes, counters, world lists, verdicts
+    size_t roll_doubles = 0, roll_ints = 0;
+    char* d_stage = nullptr;    // staging of the host-pointer rollout / clearance calls
+    size_t stage_bytes = 0;
 };
 
 namespace {
@@ -437,7 +444,7 @@ int armour_ctx_destroy(armour_ctx* ctx) {
     if (!ctx) return ARMOUR_OK;
     cudaSetDevice(ctx->cfg.device);
     Batch& B = ctx->B;
-    void* ptrs[] = {ctx->d_solver, ctx->d_solver_i, ctx->d_solver_io, ctx->d_unit_flag, ctx->d_jnz, ctx->d_jrs, ctx->d_armtd_in, ctx->d_ga, ctx->d_ja,
+    void* ptrs[] = {ctx->d_roll, ctx->d_roll_i, ctx->d_stage, ctx->d_solver, ctx->d_solver_i, ctx->d_solver_io, ctx->d_unit_flag, ctx->d_jnz, ctx->d_jrs, ctx->d_armtd_in, ctx->d_ga, ctx->d_ja,
                     ctx->d_in, ctx->d_obs, ctx->d_k, ctx->d_g, ctx->d_jac, ctx->d_verdict, B.link_n, B.link_c,
                     B.link_key, B.link_g, B.u_n, B.u_c, B.u_r, B.u_key, B.u_g, B.torque_radius, B.link_gens, B.link_r, B.hp_cand, B.hp_cnt, B.hp_slow,
                     B.link_sliced, B.status};
@@ -977,6 +984,245 @@ int armour_batch_solve(armour_ctx* ctx, int nprob, const double* q_des, const ar
     if (!ctx || !q_des || !k_opt || !feasible) return ARMOUR_ERR_ARG;
     if (nprob < 1 || nprob > ctx->built_nprob) return fail(ctx, ARMOUR_ERR_STATE, "solve before build");
     return solve_from_host(ctx, nprob, q_des, opt, k_opt, feasible, first_violation, iterations, armour_batch_solve_device);
+}
+
+void armour_rollout_options_default(armour_rollout_options* opt) {
+    if (!opt) return;
+    std::memset(opt, 0, sizeof(*opt));
+    opt->struct_size = int(sizeof(armour_rollout_options));
+    opt->max_replans = 100;
+    opt->lookahead = 0.1;
+    opt->goal_radius = 0.05;
+    opt->audit_samples = 16;
+    armour_solver_options_default(&opt->solver);
+}
+
+}  // extern "C"
+
+namespace {
+
+// grow-only device buffer of at least n elements (contents are not kept)
+template <class T>
+int ensure_buffer(armour_ctx* ctx, T** p, size_t* cap, size_t n) {
+    if (*cap >= n) return ARMOUR_OK;
+    if (*p) cudaFree(*p);
+    *p = nullptr;
+    *cap = 0;
+    CU(dalloc(p, n));
+    *cap = n;
+    return ARMOUR_OK;
+}
+
+int check_rollout(armour_ctx* ctx, int nworlds, int nobs, const armour_rollout_options* opt) {
+    if (!ctx) return ARMOUR_ERR_ARG;
+    if (ctx->armtd) return fail(ctx, ARMOUR_ERR_STATE, "closed-loop episodes run the main planner, not the ARMTD comparison planner");
+    if (nworlds < 1) return fail(ctx, ARMOUR_ERR_ARG, "nworlds < 1");
+    if (nworlds > ctx->cfg.max_problems) return fail(ctx, ARMOUR_ERR_STATE, "nworlds larger than max_problems");
+    if (nobs < 0) return fail(ctx, ARMOUR_ERR_ARG, "negative obstacle count");
+    if (nobs > ctx->cfg.max_obstacles) return fail(ctx, ARMOUR_ERR_OBSTACLES, "number of obstacles larger than max_obstacles");
+    if (!opt || opt->struct_size != int(sizeof(armour_rollout_options))) return fail(ctx, ARMOUR_ERR_ARG, "rollout options");
+    if (opt->max_replans < 1 || opt->audit_samples < 2 || !(opt->lookahead > 0) || !(opt->goal_radius >= 0))
+        return fail(ctx, ARMOUR_ERR_ARG, "rollout options");
+    const armour_solver_options& so = opt->solver;
+    if (so.max_iter < 1 || !(so.tol > 0) || so.qp_sweeps < 1 || !(so.collision_tol >= 0))
+        return fail(ctx, ARMOUR_ERR_ARG, "solver options");
+    return ARMOUR_OK;
+}
+
+// The episode loop (include/armour_b200.h, "closed-loop replanning episodes"): per replan k_rollout_plan, the device build and
+// solve of the running worlds, k_rollout_advance, k_clearance over the audit samples, k_rollout_finish; then one copy of the
+// running count to the host and one synchronisation.
+int rollout_run(armour_ctx* ctx, int n, const double* d_start, const double* d_goal, const double* d_obstacles, int nobs,
+                const armour_rollout_options& opt, const armour_rollout_out& out) {
+    CU(cudaSetDevice(ctx->cfg.device));
+    { int rc_c = ensure_constants(ctx); if (rc_c) return rc_c; }
+    const size_t N = size_t(n), S = size_t(opt.audit_samples), no = size_t(nobs) * 12;
+    const size_t need_d = N * (ROLL_STATE + ROLL_PLAN + 1 + 5 * NF + 1) + N * no + N * S * NF;
+    const size_t need_i = 10 * N + 1;
+    { int rc = ensure_buffer(ctx, &ctx->d_roll, &ctx->roll_doubles, need_d); if (rc) return rc; }
+    { int rc = ensure_buffer(ctx, &ctx->d_roll_i, &ctx->roll_ints, need_i); if (rc) return rc; }
+    RolloutDev D;
+    D.n = n;
+    D.R = opt.max_replans;
+    D.nobs = nobs;
+    D.S = opt.audit_samples;
+    D.lookahead = opt.lookahead;
+    D.goal_radius = opt.goal_radius;
+    D.collision_tol = opt.solver.collision_tol;
+    D.start = d_start;
+    D.goal = d_goal;
+    D.obstacles = d_obstacles;
+    double* w = ctx->d_roll;
+    D.state = w; w += N * ROLL_STATE;
+    D.plan = w; w += N * ROLL_PLAN;
+    D.minc = w; w += N;
+    D.dq0 = w; w += N * NF;
+    D.dqd0 = w; w += N * NF;
+    D.dqdd0 = w; w += N * NF;
+    D.dq_des = w; w += N * NF;
+    D.dk = w; w += N * NF;
+    D.dclear = w; w += N;
+    D.dobs = w; w += N * no;
+    D.samp = w;
+    int* wi = ctx->d_roll_i;
+    D.outcome = wi; wi += N;
+    D.replans = wi; wi += N;
+    D.infeasible = wi; wi += N;
+    D.limit = wi; wi += N;
+    D.dfeas = wi; wi += N;
+    D.dfirst = wi; wi += N;
+    D.diters = wi; wi += N;
+    int* list = wi; wi += N;
+    int* next = wi; wi += N;
+    int* d_count = wi;
+    D.log_state = out.log_state;
+    D.log_q_des = out.log_q_des;
+    D.log_k = out.log_k;
+    D.log_int = out.log_int;
+    D.log_clearance = out.log_clearance;
+    cudaStream_t st = ctx->stream;
+    const int ib = std::min<int>(int((N * size_t(opt.max_replans) + ROLL_THREADS - 1) / ROLL_THREADS), 4096);
+    k_rollout_init<<<ib, ROLL_THREADS, 0, st>>>(D, list);
+    CU(cudaGetLastError());
+    ctx->launches += 1;
+    int nrun = n;
+    for (int r = 0; r < opt.max_replans && nrun > 0; r++) {
+        const int gb = (nrun + ROLL_THREADS - 1) / ROLL_THREADS;
+        k_rollout_plan<<<gb, ROLL_THREADS, 0, st>>>(D, r, nrun, list);
+        CU(cudaGetLastError());
+        ctx->launches += 1;
+        { int rc = armour_batch_reachsets_build_device(ctx, nrun, D.dq0, D.dqd0, D.dqdd0, nobs > 0 ? D.dobs : nullptr, nobs); if (rc) return rc; }
+        { int rc = armour_batch_solve_device(ctx, nrun, D.dq_des, &opt.solver, D.dk, D.dfeas, D.dfirst, D.diters); if (rc) return rc; }
+        k_rollout_advance<<<gb, ROLL_THREADS, 0, st>>>(D, r, nrun, list, ctx->B.status, ctx->B.epoch);
+        k_clearance<<<nrun, CLEAR_THREADS, 0, st>>>(D.samp, opt.audit_samples, list, d_obstacles, nobs, D.dclear, nullptr);
+        k_rollout_finish<<<1, FINISH_THREADS, 0, st>>>(D, r, nrun, list, next, d_count);
+        CU(cudaGetLastError());
+        ctx->launches += 3;
+        CU(cudaMemcpyAsync(&nrun, d_count, sizeof(int), cudaMemcpyDeviceToHost, st));
+        CU(cudaStreamSynchronize(st));
+        std::swap(list, next);
+    }
+    if (out.outcome) CU(cudaMemcpyAsync(out.outcome, D.outcome, N * sizeof(int), cudaMemcpyDeviceToDevice, st));
+    if (out.replans) CU(cudaMemcpyAsync(out.replans, D.replans, N * sizeof(int), cudaMemcpyDeviceToDevice, st));
+    if (out.infeasible) CU(cudaMemcpyAsync(out.infeasible, D.infeasible, N * sizeof(int), cudaMemcpyDeviceToDevice, st));
+    if (out.final_state) CU(cudaMemcpyAsync(out.final_state, D.state, N * ROLL_STATE * sizeof(double), cudaMemcpyDeviceToDevice, st));
+    if (out.min_clearance) CU(cudaMemcpyAsync(out.min_clearance, D.minc, N * sizeof(double), cudaMemcpyDeviceToDevice, st));
+    return ARMOUR_OK;
+}
+
+int check_clearance(armour_ctx* ctx, int nconf, int nobs) {
+    if (!ctx) return ARMOUR_ERR_ARG;
+    if (nconf < 1) return fail(ctx, ARMOUR_ERR_ARG, "nconf < 1");
+    if (nobs < 0) return fail(ctx, ARMOUR_ERR_ARG, "negative obstacle count");
+    if (nobs > ctx->cfg.max_obstacles) return fail(ctx, ARMOUR_ERR_OBSTACLES, "number of obstacles larger than max_obstacles");
+    return ARMOUR_OK;
+}
+
+}  // namespace
+
+extern "C" {
+
+int armour_batch_rollout_device(armour_ctx* ctx, int nworlds, const double* d_start, const double* d_goal, const double* d_obstacles,
+                                int nobs, const armour_rollout_options* opt, const armour_rollout_out* d_out) {
+    int rc = check_rollout(ctx, nworlds, nobs, opt);
+    if (rc) return rc;
+    if (!d_start || !d_goal || (nobs > 0 && !d_obstacles) || !d_out) return fail(ctx, ARMOUR_ERR_ARG, "null input");
+    return rollout_run(ctx, nworlds, d_start, d_goal, d_obstacles, nobs, *opt, *d_out);
+}
+
+int armour_batch_rollout(armour_ctx* ctx, int nworlds, const double* start, const double* goal, const double* obstacles, int nobs,
+                         const armour_rollout_options* opt, const armour_rollout_out* out) {
+    int rc = check_rollout(ctx, nworlds, nobs, opt);
+    if (rc) return rc;
+    if (!start || !goal || (nobs > 0 && !obstacles) || !out) return fail(ctx, ARMOUR_ERR_ARG, "null input");
+    CU(cudaSetDevice(ctx->cfg.device));
+    const size_t N = size_t(nworlds), R = size_t(opt->max_replans);
+    // staging: inputs, then one device array per requested output (8-byte aligned pieces)
+    const size_t sz[13] = {N * NF * 8, N * NF * 8, N * size_t(nobs) * 12 * 8,
+                           out->outcome ? N * 4 : 0, out->replans ? N * 4 : 0, out->infeasible ? N * 4 : 0,
+                           out->final_state ? N * ROLL_STATE * 8 : 0, out->min_clearance ? N * 8 : 0,
+                           out->log_state ? R * N * ROLL_STATE * 8 : 0, out->log_q_des ? R * N * NF * 8 : 0,
+                           out->log_k ? R * N * NF * 8 : 0, out->log_int ? R * N * 4 * 4 : 0, out->log_clearance ? R * N * 8 : 0};
+    size_t off[13], total = 0;
+    for (int i = 0; i < 13; i++) {
+        off[i] = total;
+        total += (sz[i] + 255) / 256 * 256;
+    }
+    rc = ensure_buffer(ctx, &ctx->d_stage, &ctx->stage_bytes, total);
+    if (rc) return rc;
+    char* base = ctx->d_stage;
+    auto at = [&](int i) -> void* { return sz[i] ? base + off[i] : nullptr; };
+    cudaStream_t st = ctx->stream;
+    CU(cudaMemcpyAsync(at(0), start, sz[0], cudaMemcpyHostToDevice, st));
+    CU(cudaMemcpyAsync(at(1), goal, sz[1], cudaMemcpyHostToDevice, st));
+    if (nobs > 0) CU(cudaMemcpyAsync(at(2), obstacles, sz[2], cudaMemcpyHostToDevice, st));
+    armour_rollout_out d_out;
+    d_out.outcome = static_cast<int*>(at(3));
+    d_out.replans = static_cast<int*>(at(4));
+    d_out.infeasible = static_cast<int*>(at(5));
+    d_out.final_state = static_cast<double*>(at(6));
+    d_out.min_clearance = static_cast<double*>(at(7));
+    d_out.log_state = static_cast<double*>(at(8));
+    d_out.log_q_des = static_cast<double*>(at(9));
+    d_out.log_k = static_cast<double*>(at(10));
+    d_out.log_int = static_cast<int*>(at(11));
+    d_out.log_clearance = static_cast<double*>(at(12));
+    rc = rollout_run(ctx, nworlds, static_cast<const double*>(at(0)), static_cast<const double*>(at(1)),
+                     nobs > 0 ? static_cast<const double*>(at(2)) : nullptr, nobs, *opt, d_out);
+    if (rc) return rc;
+    void* host[13] = {nullptr, nullptr, nullptr, out->outcome, out->replans, out->infeasible, out->final_state, out->min_clearance,
+                      out->log_state, out->log_q_des, out->log_k, out->log_int, out->log_clearance};
+    for (int i = 3; i < 13; i++)
+        if (sz[i]) CU(cudaMemcpyAsync(host[i], at(i), sz[i], cudaMemcpyDeviceToHost, st));
+    CU(cudaStreamSynchronize(st));
+    return ARMOUR_OK;
+}
+
+int armour_batch_clearance_device(armour_ctx* ctx, int nconf, const double* d_q, const int* d_world, const double* d_obstacles,
+                                  int nobs, double* d_clearance, int* d_which) {
+    int rc = check_clearance(ctx, nconf, nobs);
+    if (rc) return rc;
+    if (!d_q || !d_clearance || (nobs > 0 && !d_obstacles)) return fail(ctx, ARMOUR_ERR_ARG, "null input");
+    CU(cudaSetDevice(ctx->cfg.device));
+    { int rc_c = ensure_constants(ctx); if (rc_c) return rc_c; }
+    k_clearance<<<nconf, CLEAR_THREADS, 0, ctx->stream>>>(d_q, 1, d_world, d_obstacles, nobs, d_clearance, d_which);
+    CU(cudaGetLastError());
+    ctx->launches += 1;
+    return ARMOUR_OK;
+}
+
+int armour_batch_clearance(armour_ctx* ctx, int nconf, const double* q, const int* world, const double* obstacles, int nobs,
+                           double* clearance, int* which) {
+    int rc = check_clearance(ctx, nconf, nobs);
+    if (rc) return rc;
+    if (!q || !clearance || (nobs > 0 && !obstacles)) return fail(ctx, ARMOUR_ERR_ARG, "null input");
+    int nsets = 1;
+    if (world)
+        for (int i = 0; i < nconf; i++) {
+            if (world[i] < 0) return fail(ctx, ARMOUR_ERR_ARG, "negative obstacle-set index");
+            nsets = std::max(nsets, world[i] + 1);
+        }
+    CU(cudaSetDevice(ctx->cfg.device));
+    const size_t nq = size_t(nconf) * NF * 8, nw = world ? size_t(nconf) * 4 : 0, nb = size_t(nsets) * nobs * 12 * 8,
+                 nc = size_t(nconf) * 8, nh = which ? size_t(nconf) * 4 : 0;
+    const size_t oq = 0, ow = oq + (nq + 255) / 256 * 256, ob = ow + (nw + 255) / 256 * 256, oc = ob + (nb + 255) / 256 * 256,
+                 oh = oc + (nc + 255) / 256 * 256;
+    rc = ensure_buffer(ctx, &ctx->d_stage, &ctx->stage_bytes, oh + nh);
+    if (rc) return rc;
+    char* base = ctx->d_stage;
+    cudaStream_t st = ctx->stream;
+    CU(cudaMemcpyAsync(base + oq, q, nq, cudaMemcpyHostToDevice, st));
+    if (world) CU(cudaMemcpyAsync(base + ow, world, nw, cudaMemcpyHostToDevice, st));
+    if (nobs > 0) CU(cudaMemcpyAsync(base + ob, obstacles, nb, cudaMemcpyHostToDevice, st));
+    rc = armour_batch_clearance_device(ctx, nconf, reinterpret_cast<const double*>(base + oq),
+                                       world ? reinterpret_cast<const int*>(base + ow) : nullptr,
+                                       nobs > 0 ? reinterpret_cast<const double*>(base + ob) : nullptr, nobs,
+                                       reinterpret_cast<double*>(base + oc), which ? reinterpret_cast<int*>(base + oh) : nullptr);
+    if (rc) return rc;
+    CU(cudaMemcpyAsync(clearance, base + oc, nc, cudaMemcpyDeviceToHost, st));
+    if (which) CU(cudaMemcpyAsync(which, base + oh, nh, cudaMemcpyDeviceToHost, st));
+    CU(cudaStreamSynchronize(st));
+    return ARMOUR_OK;
 }
 
 // ---- getters ---------------------------------------------------------------------------------------

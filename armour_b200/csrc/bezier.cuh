@@ -45,6 +45,21 @@ ARMOUR_HD double bez_qd(double q0, double Tqd0, double TTqdd0, double k, double 
     const double beta3 = q0 + k;
     return dB0 * q0 + dB1 * beta1 + dB2 * beta2 + dB3 * beta3 + dB4 * beta3 + dB5 * beta3;
 }
+// second derivative w.r.t. normalised time (the reference has none: the closed-loop rollout needs qdd at the end of the
+// executed segment); q''(0) = TTqdd0, q''(1) = 0
+ARMOUR_HD double bez_qdd(double q0, double Tqd0, double TTqdd0, double k, double t) {
+    const double u = 1.0 - t;
+    const double ddB0 = 20.0 * pw3(u);
+    const double ddB1 = -40.0 * pw3(u) + 60.0 * t * pw2(u);
+    const double ddB2 = 20.0 * pw3(u) - 120.0 * t * pw2(u) + 60.0 * pw2(t) * u;
+    const double ddB3 = 60.0 * t * pw2(u) - 120.0 * pw2(t) * u + 20.0 * pw3(t);
+    const double ddB4 = 60.0 * pw2(t) * u - 40.0 * pw3(t);
+    const double ddB5 = 20.0 * pw3(t);
+    const double beta1 = q0 + Tqd0 / 5;
+    const double beta2 = q0 + (2 * Tqd0) / 5 + TTqdd0 / 20;
+    const double beta3 = q0 + k;
+    return ddB0 * q0 + ddB1 * beta1 + ddB2 * beta2 + ddB3 * beta3 + ddB4 * beta3 + ddB5 * beta3;
+}
 // k-independent parts, KPR/Trajectory.cu:812-822
 ARMOUR_HD double bez_q_indep(double q0, double a, double b, double s) {
     return q0 + a * s - 6 * a * pw3(s) + 8 * a * pw4(s) - 3 * a * pw5(s) + (b * pw2(s)) * 0.5 - (3 * b * pw3(s)) * 0.5 +

@@ -150,6 +150,57 @@ class ReachSetEngine:
                                                 iters.ctypes.data_as(_lib.ip)))
         return k, ok.astype(bool), first, iters
 
+    # -- closed-loop episodes (kinova_run_100_worlds.m -> simulator_armtd.run) ------------------------------------------
+    def rollout(self, start, goal, obstacles, max_replans=100, goal_radius=0.05, lookahead=0.1, audit_samples=16,
+                max_iter=None, tol=None, torque_tol=None, collision_tol=None, qp_sweeps=None):
+        """Closed-loop replanning episodes of a batch of worlds on the device (armour_batch_rollout; semantics in
+        include/armour_b200.h).  start, goal: [n, 7]; obstacles: [n, nobs, 12].  Returns a dict of numpy arrays: outcome,
+        replans, infeasible [n], final_state [n, 21], min_clearance [n], log_state [R, n, 21], log_q_des, log_k [R, n, 7],
+        log_int [R, n, 4] (feasible, first violated row, iterations, build status), log_clearance [R, n].  The context's
+        reach sets afterwards are those of the last replan's sub-batch: build again before evaluating."""
+        start, goal = _f64(start).reshape(-1, NF), _f64(goal).reshape(-1, NF)
+        n = start.shape[0]
+        obs = _f64(obstacles)
+        obs = obs.reshape(n, -1, 12) if obs.size else np.zeros((n, 0, 12))
+        opt = _lib.RolloutOptions()
+        self.lib.armour_rollout_options_default(C.byref(opt))
+        opt.max_replans, opt.goal_radius, opt.lookahead = int(max_replans), float(goal_radius), float(lookahead)
+        opt.audit_samples = int(audit_samples)
+        for name, v in (("max_iter", max_iter), ("tol", tol), ("torque_tol", torque_tol), ("collision_tol", collision_tol),
+                        ("qp_sweeps", qp_sweeps)):
+            if v is not None:
+                setattr(opt.solver, name, type(getattr(opt.solver, name))(v))
+        R = opt.max_replans
+        res = dict(outcome=np.zeros(n, np.int32), replans=np.zeros(n, np.int32), infeasible=np.zeros(n, np.int32),
+                   final_state=np.zeros((n, 3 * NF)), min_clearance=np.zeros(n), log_state=np.zeros((max(R, 0), n, 3 * NF)),
+                   log_q_des=np.zeros((max(R, 0), n, NF)), log_k=np.zeros((max(R, 0), n, NF)),
+                   log_int=np.zeros((max(R, 0), n, 4), np.int32), log_clearance=np.zeros((max(R, 0), n)))
+        out = _lib.RolloutOut()
+        for name, a in res.items():
+            setattr(out, name, a.ctypes.data_as(_lib.ip if a.dtype == np.int32 else _lib.dp))
+        self._check(self.lib.armour_batch_rollout(self._h, n, _dp(start), _dp(goal), _dp(obs), obs.shape[1], C.byref(opt),
+                                                  C.byref(out)))
+        self.nprob = 0
+        return res
+
+    def clearance(self, q, obstacles, world=None):
+        """Exact signed clearance of arm configurations q [n, 7] (armour_batch_clearance): link boxes of this context's
+        robot model against obstacle set world[i] of obstacles [nsets, nobs, 12] (or [nobs, 12]; world None: set 0) by the
+        separating-axis test.  Returns (clearance [n], which [n] = l * nobs + o of the closest pair)."""
+        q = _f64(q).reshape(-1, NF)
+        n = q.shape[0]
+        obs = _f64(obstacles)
+        nobs = obs.shape[-2] if obs.size else 0
+        obs = obs.reshape(-1, nobs, 12) if obs.size else np.zeros((1, 0, 12))
+        w = None if world is None else np.ascontiguousarray(np.asarray(world, dtype=np.int32).reshape(n))
+        if w is not None and (w.min() < 0 or w.max() >= obs.shape[0]):
+            raise ValueError("world index outside the obstacle sets")
+        clr = np.empty(n)
+        which = np.empty(n, np.int32)
+        self._check(self.lib.armour_batch_clearance(self._h, n, _dp(q), w.ctypes.data_as(_lib.ip) if w is not None else None,
+                                                    _dp(obs), nobs, _dp(clr), which.ctypes.data_as(_lib.ip)))
+        return clr, which
+
     def measure_fp64_peak(self):
         """Sustained non-tensor FP64 rate of the device in TFLOP/s (FMA probe kernel in the library)."""
         v = C.c_double(0)

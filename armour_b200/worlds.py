@@ -82,6 +82,40 @@ def config1_problem(csv_path):
 
 def random_problems(nprob, nobs, seed=20261017, moving=True):
     """BASELINE config 2 generator: random start / goal / motion state and `nobs` random boxes per problem."""
+    q0, goal, qd0, qdd0, obs = _random_draws(nprob, nobs, seed, moving)
+    q_des = np.stack([straight_line_waypoint(q0[p], goal[p]) for p in range(nprob)])
+    return quantize(q0), quantize(qd0), quantize(qdd0), quantize(q_des), quantize(obs)
+
+
+def random_episodes(nworlds, nobs, seed=20261017):
+    """Closed-loop episodes from the draws of random_problems(nworlds, nobs, seed, moving=False): start, goal [n, 7] and
+    obstacles [n, nobs, 12], %.10f-quantised like random_problems' outputs (start and obstacles equal its q0 and obstacles)."""
+    q0, goal, _, _, obs = _random_draws(nworlds, nobs, seed, False)
+    return quantize(q0), quantize(goal), quantize(obs)
+
+
+PAD_CENTRE = np.array([10.0, 10.0, 10.0])  # m: far beyond the arm's reach (about 1.3 m from the base)
+PAD_HALF_SIZE = 0.005
+
+
+def pad_obstacles(obstacles, n):
+    """Pad every world's obstacle list ([n_i, 12] each) to n obstacles with small boxes (1 cm) far outside the workspace, so
+    that worlds with different counts form one batch.  Returns [len(obstacles), n, 12]; the padding boxes lie along x from
+    PAD_CENTRE, one per slot."""
+    out = np.empty((len(obstacles), n, 12))
+    for w, o in enumerate(obstacles):
+        o = np.asarray(o, dtype=np.float64).reshape(-1, 12)
+        if o.shape[0] > n:
+            raise ValueError(f"world {w} has {o.shape[0]} obstacles, more than {n}")
+        out[w, :o.shape[0]] = o
+        for s in range(o.shape[0], n):
+            out[w, s] = 0.0
+            out[w, s, 0:3] = PAD_CENTRE + np.array([0.1 * s, 0.0, 0.0])
+            out[w, s, 3] = out[w, s, 7] = out[w, s, 11] = PAD_HALF_SIZE
+    return out
+
+
+def _random_draws(nprob, nobs, seed, moving):
     rng = np.random.default_rng(seed)
     q0 = rng.uniform(STATE_LB, STATE_UB, (nprob, NF))
     goal = rng.uniform(STATE_LB, STATE_UB, (nprob, NF))
@@ -98,8 +132,7 @@ def random_problems(nprob, nobs, seed=20261017, moving=True):
             boxes[p, n] = np.concatenate([c, s])
             n += 1
     obs = boxes_to_zonotopes(boxes.reshape(-1, 6)).reshape(nprob, nobs, 12)
-    q_des = np.stack([straight_line_waypoint(q0[p], goal[p]) for p in range(nprob)])
-    return quantize(q0), quantize(qd0), quantize(qdd0), quantize(q_des), quantize(obs)
+    return q0, goal, qd0, qdd0, obs
 
 
 def halton_k(n, dim=NF, skip=1):

@@ -182,6 +182,78 @@ int armour_chunk_intervals(void);
  * sustained non-tensor FP64 rate in TFLOP/s (the FP64 roofline denominator; BASELINE.md section 2). */
 int armour_measure_fp64_peak(armour_ctx* ctx, double* tflops);
 
+/* ---- closed-loop replanning episodes (worlds replanned in sequence) --------------------------------------------------------
+ *
+ * The loop of the reference's system test (kinova_run_100_worlds.m -> simulator_armtd.run): waypoint, plan, execute the plan up
+ * to t_move, replan from where the executed motion ends; run for a batch of worlds on the device, with an exact collision and
+ * joint-limit audit of every executed segment.  A world has a start and a goal configuration and nobs obstacles ([nobs][12]
+ * zonotopes as everywhere else); the arm starts at rest; nworlds <= max_problems.  Replan r of world w:
+ *   1. planning state (q0, qd0, qdd0): (start, 0, 0) at r = 0, afterwards the state step 5 of replan r - 1 produced;
+ *   2. q_des: the straight-line waypoint of armour_b200.worlds.straight_line_waypoint (angdiff on the continuous joints 0, 2,
+ *      4, 6; lookahead rad along d = goal - q), except that when |d| <= lookahead the waypoint is the goal itself (q + d), so
+ *      that an arriving arm is not pulled past it.  The clamp is this library's choice (the reference's high-level planner,
+ *      robot_arm_straight_line_HLP.m, is not part of the reference tree this library restates);
+ *   3. plan: armour_batch_reachsets_build_device + armour_batch_solve_device on the running worlds, from k = 0, with
+ *      opt->solver as given.  A build that overflowed a table evaluates fail-safe: an infeasible replan, logged separately;
+ *   4. executed segment: after a feasible plan the new plan over s in [0, t_move], and it becomes the world's current plan;
+ *      otherwise the current plan's braking half s in [t_move, 1], after which the current plan is the rest plan at its end
+ *      (q = q(1), qd = qdd = 0, k = 0; its Bezier is constant, so repeated failures keep the arm still).  The initial current
+ *      plan is the rest plan at the start.  t_move = t_plan = 0.5 s of the robot model (duration 1 s);
+ *   5. next state: (q, qd, qdd) of the executed plan at the segment's end, time derivatives in real time;
+ *   6. audit: audit_samples evenly spaced samples of the executed segment, both ends included.  At each sample the exact link
+ *      boxes (forward kinematics of all num_joints links) against every obstacle: the signed clearance of two parallelepipeds
+ *      by the separating-axis test (15 axes; > 0 separated, a lower bound on the distance; <= 0 intersecting, -penetration);
+ *      the non-continuous joints against the raw position limits and |qd| against the raw speed limits (without the margins of
+ *      the verdict);
+ *   7. stop: clearance below -opt->solver.collision_tol -> ARMOUR_ROLLOUT_COLLISION, else a limit exceeded -> _LIMIT, else the
+ *      segment's end within goal_radius of the goal (2-norm of the difference, angdiff on the continuous joints) -> _ARRIVED,
+ *      else max_replans used -> _BUDGET.  The loop ends when no world is running.
+ * Stopped worlds leave the later builds and solves: the running worlds are gathered in ascending world index into the dense
+ * batch (the sub-batch of replan r is the worlds with replans > r, in order).  Continuous joints are not wrapped; there is no
+ * %.10f quantisation inside the loop.  Log rows are indexed by world; world w planned at replan r exactly when r < replans[w];
+ * the rows of replans it did not plan are NaN (doubles) and -1 (ints).  The context's reach sets after the call are those of
+ * the last replan's sub-batch.  Not modelled: tracking error and the low-level controller, torque audits, warm starts.
+ * Errors: ARMOUR_ERR_STATE for nworlds > max_problems and for a context of the ARMTD comparison planner, ARMOUR_ERR_OBSTACLES for
+ * nobs > max_obstacles, ARMOUR_ERR_ARG for bad options and null inputs. */
+enum { ARMOUR_ROLLOUT_BUDGET = 0, ARMOUR_ROLLOUT_ARRIVED = 1, ARMOUR_ROLLOUT_COLLISION = 2, ARMOUR_ROLLOUT_LIMIT = 3 };
+typedef struct armour_rollout_options {
+    int struct_size;               /* sizeof(armour_rollout_options) */
+    int max_replans;               /* >= 1, default 100 */
+    double lookahead;              /* > 0, default 0.1 rad (the reference's straight-line waypoint) */
+    double goal_radius;            /* >= 0, default 0.05 rad: this library's choice, the reference's goal test is not in its tree */
+    int audit_samples;             /* >= 2, default 16 */
+    armour_solver_options solver;  /* the solve of every replan; collision_tol is also the audit's tolerance */
+} armour_rollout_options;
+void armour_rollout_options_default(armour_rollout_options* opt);
+/* Outputs; any pointer may be NULL.  [n] = nworlds, [R] = max_replans. */
+typedef struct armour_rollout_out {
+    int* outcome;            /* [n] ARMOUR_ROLLOUT_* */
+    int* replans;            /* [n] replans planned */
+    int* infeasible;         /* [n] replans that executed the braking half */
+    double* final_state;     /* [n][21] q, qd, qdd at the end of the last executed segment */
+    double* min_clearance;   /* [n] smallest audited clearance over the episode, m (+inf without obstacles) */
+    double* log_state;       /* [R][n][21] planning state q0, qd0, qdd0 of replan r */
+    double* log_q_des;       /* [R][n][7] */
+    double* log_k;           /* [R][n][7] k_opt */
+    int* log_int;            /* [R][n][4] feasible, first violated row, solver iterations, build status (0 / ARMOUR_ERR_CAPACITY) */
+    double* log_clearance;   /* [R][n] smallest audited clearance of the segment executed after replan r */
+} armour_rollout_out;
+/* start, goal [nworlds][7], obstacles [nworlds][nobs][12]; DEVICE pointers, in *out too.  One device-to-host copy of the
+ * running count and one synchronisation per replan. */
+int armour_batch_rollout_device(armour_ctx* ctx, int nworlds, const double* d_start, const double* d_goal, const double* d_obstacles,
+                                int nobs, const armour_rollout_options* opt, const armour_rollout_out* d_out);
+/* The same with host pointers (the copies are part of the call). */
+int armour_batch_rollout(armour_ctx* ctx, int nworlds, const double* start, const double* goal, const double* obstacles, int nobs,
+                         const armour_rollout_options* opt, const armour_rollout_out* out);
+/* Exact clearance of nconf arm configurations q [nconf][7]: the link boxes of the context's robot model against obstacle set
+ * world[i] of obstacles [nsets][nobs][12] (world NULL: set 0 for all) by the audit's separating-axis test.  clearance[nconf]
+ * = the smallest over links and obstacles, which[nconf] (may be NULL) = l * nobs + o of the pair attaining it (ties: the lowest),
+ * +inf and -1 without obstacles.  The _device call does not check world[] against the number of sets. */
+int armour_batch_clearance_device(armour_ctx* ctx, int nconf, const double* d_q, const int* d_world, const double* d_obstacles,
+                                  int nobs, double* d_clearance, int* d_which);
+int armour_batch_clearance(armour_ctx* ctx, int nconf, const double* q, const int* world, const double* obstacles, int nobs,
+                           double* clearance, int* which);
+
 /* ---- reach-set tables (k-only monomials after reduce / reduce_link_PZ) -------------------------- */
 
 /* Padded neutral layout shared with the test oracle:
