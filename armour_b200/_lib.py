@@ -82,6 +82,8 @@ SIGNATURES = {
     "armour_batch_get_monomial_counts": (C.c_int, [C.c_void_p, C.c_int, ip, ip]),
     "armour_batch_get_candidate_counts": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p]),
     "armour_chunk_intervals": (C.c_int, []),
+    "armour_eval_image_layout": (C.c_int, [C.c_void_p, C.POINTER(C.c_longlong)]),
+    "armour_batch_get_eval_images": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p]),
     "armour_jacobian_nnz": (C.c_longlong, [C.c_void_p, C.c_int]),
     "armour_jacobian_structure": (C.c_int, [C.c_void_p, C.c_int, ip, ip]),
     "armour_eval_jac_g_structured": (C.c_int, [C.c_void_p, dp, dp]),

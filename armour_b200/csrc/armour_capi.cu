@@ -112,7 +112,8 @@ struct armour_ctx {
     cudaStream_t own_stream = nullptr;
     Batch B;                 // device pointers + dimensions of the current batch
     int built_nprob = 0;     // problems with valid reach sets
-    size_t hp_capacity = 0;  // doubles allocated for B.hp_cand
+    size_t img_capacity = 0; // bytes allocated for B.img
+    size_t cnt_capacity = 0; // bytes allocated for B.hp_cnt
     int hp_nprob = 0;        // problems the candidate buffers were sized for
     int* d_unit_flag = nullptr;  // [max_problems * T] completion stamps of the reach-set units (latency path)
     size_t obs_capacity = 0;
@@ -219,24 +220,27 @@ int ensure_obstacle_buffers(armour_ctx* ctx, int nprob, int nobs) {
     Batch& B = ctx->B;
     B.O = nobs;
     B.nprob = nprob;
-    const size_t need_hp = size_t(nprob) * (B.T / TB) * B.hp_chunk();
-    if (ctx->hp_capacity < need_hp || ctx->hp_nprob < nprob) {
-        // (the candidate lists of the current batch go with the old buffers: whatever was built must be rebuilt)
-        if (B.hp_cand) cudaFree(B.hp_cand);
+    const size_t need_img = size_t(nprob) * (B.T / TB) * B.img_chunk();
+    const size_t need_cnt = size_t(nprob) * B.T * B.NJ * nobs;
+    if (ctx->img_capacity < need_img || ctx->hp_nprob < nprob || ctx->cnt_capacity < need_cnt) {
+        // (the candidate lists and images of the current batch go with the old buffers: whatever was built must be rebuilt)
+        if (B.img) cudaFree(B.img);
         if (B.hp_cnt) cudaFree(B.hp_cnt);
         if (B.hp_slow) cudaFree(B.hp_slow);
-        B.hp_cand = nullptr;
+        B.img = nullptr;
         B.hp_cnt = nullptr;
         B.hp_slow = nullptr;
-        ctx->hp_capacity = 0;
+        ctx->img_capacity = 0;
+        ctx->cnt_capacity = 0;
         ctx->hp_nprob = 0;
         ctx->built_nprob = 0;
         const size_t np = std::max(nprob, ctx->hp_nprob);
-        CU(dalloc(&B.hp_cand, need_hp));
-        CU(dalloc(&B.hp_cnt, need_hp / (HP_CAP * 4)));
+        CU(dalloc(&B.img, need_img));
+        CU(dalloc(&B.hp_cnt, need_cnt));
         CU(dalloc(&B.hp_slow, np));
         CU(cudaMemsetAsync(B.hp_slow, 0, np * sizeof(int), ctx->stream));
-        ctx->hp_capacity = need_hp;
+        ctx->img_capacity = need_img;
+        ctx->cnt_capacity = need_cnt;
         ctx->hp_nprob = nprob;
     }
     B.obstacles = ctx->d_obs;
@@ -429,9 +433,6 @@ int armour_ctx_create(const armour_config* cfg, armour_ctx** out) {
         if ((e = cudaFuncGetAttributes(&fa, k1lat::k_reachsets)) != cudaSuccess) return bail("load k_reachsets", e);
         if ((e = cudaFuncGetAttributes(&fa, k_hyperplanes)) != cudaSuccess) return bail("load k_hyperplanes", e);
         if ((e = cudaFuncGetAttributes(&fa, k_constraints)) != cudaSuccess) return bail("load k_constraints", e);
-        if ((e = cudaFuncSetAttribute(k_constraints, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                      TB * (MAXJ * K3_LTAB_BYTES + NF * K3_UTAB_BYTES) + K3_CAND_ARENA)) != cudaSuccess)
-            return bail("k_constraints shared memory", e);
         if ((e = cudaFuncGetAttributes(&fa, k_constraints_slow)) != cudaSuccess) return bail("load k_constraints_slow", e);
         if ((e = cudaFuncGetAttributes(&fa, k_verdict)) != cudaSuccess) return bail("load k_verdict", e);
     }
@@ -446,7 +447,7 @@ int armour_ctx_destroy(armour_ctx* ctx) {
     Batch& B = ctx->B;
     void* ptrs[] = {ctx->d_roll, ctx->d_roll_i, ctx->d_stage, ctx->d_solver, ctx->d_solver_i, ctx->d_solver_io, ctx->d_unit_flag, ctx->d_jnz, ctx->d_jrs, ctx->d_armtd_in, ctx->d_ga, ctx->d_ja,
                     ctx->d_in, ctx->d_obs, ctx->d_k, ctx->d_g, ctx->d_jac, ctx->d_verdict, B.link_n, B.link_c,
-                    B.link_key, B.link_g, B.u_n, B.u_c, B.u_r, B.u_key, B.u_g, B.torque_radius, B.link_gens, B.link_r, B.hp_cand, B.hp_cnt, B.hp_slow,
+                    B.link_key, B.link_g, B.u_n, B.u_c, B.u_r, B.u_key, B.u_g, B.torque_radius, B.link_gens, B.link_r, B.img, B.hp_cnt, B.hp_slow,
                     B.link_sliced, B.status};
     for (void* p : ptrs)
         if (p) cudaFree(p);
@@ -526,6 +527,8 @@ int armour_batch_reachsets_build_device(armour_ctx* ctx, int nprob, const double
         CU(cudaMemcpyAsync(ctx->d_in + 2 * P * NF, d_qdd0, nb, cudaMemcpyDeviceToDevice, ctx->stream));
         { int rc2 = launch_build(ctx, ctx->B, &nl, &latency); if (rc2) return rc2; }
     }
+    CU(launch_pack_image(ctx->B, ctx->stream));
+    nl++;
     ctx->launches += nl;
     ctx->built_nprob = nprob;
     ctx->h_torque_valid = false;
@@ -557,6 +560,8 @@ int armour_batch_reachsets_build(armour_ctx* ctx, int nprob, const double* q0, c
     ctx->launches += nl;
     CU(launch_hyperplanes(ctx->B, ctx->stream, (latency && nobs > 0) ? ctx->d_unit_flag : nullptr));
     ctx->launches += (nobs > 0);
+    CU(launch_pack_image(ctx->B, ctx->stream));
+    ctx->launches++;
     ctx->built_nprob = nprob;
     ctx->h_torque_valid = false;
     ctx->h_q0.assign(q0, q0 + size_t(nprob) * NF);
@@ -618,6 +623,21 @@ int armour_batch_get_candidate_counts(armour_ctx* ctx, int nprob, unsigned char*
 }
 
 int armour_chunk_intervals(void) { return TB; }
+
+int armour_eval_image_layout(armour_ctx* ctx, long long* layout) {
+    if (!ctx || !layout) return ARMOUR_ERR_ARG;
+    const Batch& B = ctx->B;
+    const size_t v[10] = {B.img_chunk(), 0, B.img_ut(), B.img_lc(), B.img_lr(), B.img_uc(), B.img_ur(), B.img_grp(), B.img_cnt(), B.img_hdr()};
+    for (int i = 0; i < 10; i++) layout[i] = (long long)v[i];
+    return ARMOUR_OK;
+}
+
+int armour_batch_get_eval_images(armour_ctx* ctx, int nprob, void* out) {
+    if (!ctx || !out || nprob < 1 || nprob > ctx->built_nprob) return ARMOUR_ERR_ARG;
+    CU(cudaMemcpyAsync(out, ctx->B.img, size_t(nprob) * (ctx->B.T / TB) * ctx->B.img_chunk(), cudaMemcpyDeviceToHost, ctx->stream));
+    CU(cudaStreamSynchronize(ctx->stream));
+    return ARMOUR_OK;
+}
 
 #ifdef K1_PROFILE
 // developer builds only: per-(interval, operation site) cycle counts of the last single-problem builds
@@ -1450,6 +1470,8 @@ int armour_import_reachsets(armour_ctx* ctx, int prob, int nprob_total, const ar
         if (nobs > 0) CU(cudaMemsetAsync(ctx->B.hp_slow, 0, size_t(nprob_total) * sizeof(int), ctx->stream));
         CU(launch_hyperplanes(ctx->B, ctx->stream));
         ctx->launches += (nobs > 0);
+        CU(launch_pack_image(ctx->B, ctx->stream));
+        ctx->launches++;
         ctx->built_nprob = nprob_total;
         ctx->h_torque_valid = false;
     }

@@ -326,8 +326,9 @@ __global__ void __launch_bounds__(HP_THREADS) k_hyperplanes(Batch B, const int* 
     __syncthreads();
     if (live) {  // step 4: survivors to their scan-order positions (counted over the short list)
         const size_t chunk = size_t(p) * (T / TB) + tb;
-        double* row = B.hp_cand + chunk * B.hp_chunk() + size_t(x) * 4;
-        const size_t cstride = size_t(per_pair) * 4;
+        // the row's fixed run of HP_CAP records in the chunk's evaluation image; k_pack_image compacts the runs
+        double* row = reinterpret_cast<double*>(B.img + chunk * B.img_chunk() + B.img_hdr()) + size_t(x) * HP_CAP * 4;
+        const size_t cstride = 4;
         const int nl = s_nlist[lr];
         if (keep[0] || keep[1] || pi == 0) {
             int count = 0, before[2] = {0, 0};
@@ -357,6 +358,139 @@ __global__ void __launch_bounds__(HP_THREADS) k_hyperplanes(Batch B, const int* 
             if (pi == 0 && count > HP_CAP) atomicAdd(&B.hp_slow[p], 1);  // k_constraints_slow evaluates the row
         }
     }
+}
+
+// ---------------------------------------------------------------------------------------------------
+// Pack the evaluation image of one chunk (layout: Batch::img) at the end of a build.  One CTA per (chunk, problem):
+//   1. the rows are taken in tiles of PK_TILE: exclusive prefix of the tile's stored candidate counts (HP_OVERFLOW rows store
+//      none) in shared memory, continued from the previous tiles;
+//   2. the tile's records move from the rows' fixed runs of HP_CAP (k_hyperplanes) to their CSR positions, in place: the
+//      record with CSR index c comes from run position x * HP_CAP + q >= c, so passes over increasing CSR indices
+//      [c0, c0 + PK_THREADS) that read all their records before they write any never overwrite a record a later pass (of
+//      this tile or a later one) still has to read;
+//   3. header, then the link and torque tables at their exact lengths behind the records.
+// Problems whose build failed are skipped: k_constraints writes their fail-safe rows without reading the image.
+constexpr int PK_THREADS = 256;
+constexpr int PK_TILE = 1024;  // rows per tile (a multiple of 32: the row-group bases are written tile by tile)
+constexpr int PK_ROWS_PER_THREAD = PK_TILE / PK_THREADS;
+__global__ void __launch_bounds__(PK_THREADS) k_pack_image(Batch B) {
+    const int tb = blockIdx.x, p = blockIdx.y, tid = threadIdx.x;
+    if (B.failed(p) != 0) return;
+    const int NJ = B.NJ, T = B.T, rows = B.img_rows();
+    const size_t chunk = size_t(p) * (T / TB) + tb;
+    unsigned char* img = B.img + chunk * B.img_chunk();
+    double* imgd = reinterpret_cast<double*>(img);
+    const unsigned char* cnt = B.hp_cnt + chunk * rows;
+    __shared__ unsigned s_off[PK_TILE + 1];  // first CSR record of each row of the tile, then the tile's end
+    __shared__ unsigned s_part[PK_THREADS];
+    __shared__ unsigned s_carry;             // records of the rows before the tile
+    __shared__ int s_loff[TB * MAXJ + 1], s_uoff[TB * NF + 1];
+    if (tid == 0) {
+        s_carry = 0;
+        // table offsets (counts clamped to the capacities: a valid build never exceeds them)
+        int a = 0;
+        for (int i = 0; i < TB * NJ; i++) {
+            s_loff[i] = a;
+            a += min(B.link_n[(size_t(p) * T + tb * TB) * NJ + i], B.capL);
+        }
+        s_loff[TB * NJ] = a;
+        a = 0;
+        for (int i = 0; i < TB * NF; i++) {
+            s_uoff[i] = a;
+            a += min(B.u_n[(size_t(p) * T + tb * TB) * NF + i], B.capU);
+        }
+        s_uoff[TB * NF] = a;
+    }
+    double4* rec = reinterpret_cast<double4*>(img + B.img_hdr());
+    unsigned* grp = reinterpret_cast<unsigned*>(img + B.img_grp());
+    for (int t0 = 0; t0 < rows; t0 += PK_TILE) {
+        const int n = min(PK_TILE, rows - t0);
+        // 1. prefix of the tile's counts: each thread PK_ROWS_PER_THREAD consecutive rows, then the thread sums
+        const int r0 = min(tid * PK_ROWS_PER_THREAD, n), r1 = min(r0 + PK_ROWS_PER_THREAD, n);
+        unsigned sum = 0;
+        for (int x = r0; x < r1; x++) sum += cnt[t0 + x] == HP_OVERFLOW ? 0u : cnt[t0 + x];
+        s_part[tid] = sum;
+        __syncthreads();  // (also publishes s_carry and the table offsets, or the previous tile's carry)
+        if (tid == 0) {
+            unsigned run = s_carry;
+            for (int i = 0; i < PK_THREADS; i++) {
+                const unsigned v = s_part[i];
+                s_part[i] = run;
+                run += v;
+            }
+            s_off[n] = run;
+        }
+        __syncthreads();
+        sum = s_part[tid];
+        for (int x = r0; x < r1; x++) {
+            s_off[x] = sum;
+            if (((t0 + x) & 31) == 0) grp[(t0 + x) >> 5] = sum;
+            sum += cnt[t0 + x] == HP_OVERFLOW ? 0u : cnt[t0 + x];
+        }
+        __syncthreads();
+        // 2. the tile's records to their CSR positions
+        const unsigned first = s_off[0], end = s_off[n];
+        for (unsigned c0 = first; c0 < end; c0 += PK_THREADS) {
+            const unsigned c = c0 + tid;
+            double4 v;
+            if (c < end) {
+                int lo = 0, hi = n - 1;  // last row of the tile whose first record is <= c (the row that holds c)
+                while (lo < hi) {
+                    const int mid = (lo + hi + 1) >> 1;
+                    if (s_off[mid] <= c) lo = mid; else hi = mid - 1;
+                }
+                v = rec[size_t(t0 + lo) * HP_CAP + (c - s_off[lo])];
+            }
+            __syncthreads();
+            if (c < end) rec[c] = v;
+            __syncthreads();
+        }
+        if (tid == 0) s_carry = end;  // read by thread 0 only, after the next tile's first barrier
+        __syncthreads();
+    }
+    __syncthreads();
+    const unsigned total = s_carry;
+    // 3. header and tables
+    const int nlink = s_loff[TB * NJ], ntorque = s_uoff[TB * NF];
+    const size_t l0 = B.img_hdr() / 8 + size_t(total) * 4;  // first double of the link records
+    const size_t u0 = l0 + size_t(nlink) * 4;                // first torque coefficient
+    const size_t k0 = (u0 + ntorque) * 4;                    // first torque key (uint16 units)
+    const size_t lidx = (size_t(p) * T + tb * TB) * NJ, uidx = (size_t(p) * T + tb * TB) * NF;
+    for (int i = tid; i < TB * NJ; i += PK_THREADS)
+        reinterpret_cast<int2*>(img)[i] = make_int2(int(l0) + 4 * s_loff[i], s_loff[i + 1] - s_loff[i]);
+    for (int i = tid; i < TB * NF; i += PK_THREADS)
+        reinterpret_cast<int4*>(img + B.img_ut())[i] = make_int4(int(u0) + s_uoff[i], int(k0) + s_uoff[i], s_uoff[i + 1] - s_uoff[i], 0);
+    for (int i = tid; i < TB * NJ * 3; i += PK_THREADS) {
+        reinterpret_cast<double*>(img + B.img_lc())[i] = B.link_c[lidx * 3 + i];
+        reinterpret_cast<double*>(img + B.img_lr())[i] = B.link_r[lidx * 3 + i];
+    }
+    for (int i = tid; i < TB * NF; i += PK_THREADS) {
+        reinterpret_cast<double*>(img + B.img_uc())[i] = B.u_c[uidx + i];
+        reinterpret_cast<double*>(img + B.img_ur())[i] = B.u_r[uidx + i];
+    }
+    for (int x = tid; x < rows; x += PK_THREADS) img[B.img_cnt() + x] = cnt[x];
+    for (int q = tid; q < TB * NJ * B.capL; q += PK_THREADS) {
+        const int i = q / B.capL, mI = q - i * B.capL;
+        if (mI >= s_loff[i + 1] - s_loff[i]) continue;
+        const size_t src = (lidx + i) * B.capL + mI;
+        double* dst = imgd + l0 + size_t(s_loff[i] + mI) * 4;
+        dst[0] = B.link_g[src * 3 + 0];
+        dst[1] = B.link_g[src * 3 + 1];
+        dst[2] = B.link_g[src * 3 + 2];
+        dst[3] = __longlong_as_double((long long)B.link_key[src]);  // key in the low half-word (little-endian)
+    }
+    for (int q = tid; q < TB * NF * B.capU; q += PK_THREADS) {
+        const int i = q / B.capU, mI = q - i * B.capU;
+        if (mI >= s_uoff[i + 1] - s_uoff[i]) continue;
+        const size_t src = (uidx + i) * B.capU + mI;
+        imgd[u0 + s_uoff[i] + mI] = B.u_g[src];
+        reinterpret_cast<uint16_t*>(img)[k0 + s_uoff[i] + mI] = B.u_key[src];
+    }
+}
+cudaError_t launch_pack_image(const Batch& B, cudaStream_t st) {
+    if (B.nprob == 0) return cudaSuccess;
+    k_pack_image<<<dim3(B.T / TB, B.nprob), PK_THREADS, 0, st>>>(B);
+    return cudaGetLastError();
 }
 
 // ---------------------------------------------------------------------------------------------------
@@ -440,49 +574,9 @@ __device__ __forceinline__ void slice_component(const uint16_t* __restrict__ key
 // The link warps meet on named barrier 1 and go straight to the collision rows; the torque warps write their
 // rows, then join through barrier 2 (on which the link warps only arrive), so nobody waits for the slowest
 // slice.  Collision rows are handed out in chunks of 32 from a shared counter.
-// ---- TMA bulk copy (cp.async.bulk global -> shared, completion on an mbarrier) --------------------------------------
-__device__ __forceinline__ unsigned smem_u32(const void* p) { return (unsigned)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ void mbar_init(unsigned long long* bar, unsigned count) {
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(bar)), "r"(count) : "memory");
-}
-__device__ __forceinline__ void mbar_arrive_expect_tx(unsigned long long* bar, unsigned bytes) {
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar)), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void bulk_g2s(void* dst, const void* src, unsigned bytes, unsigned long long* bar) {
-    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(smem_u32(dst)),
-                 "l"(src), "r"(bytes), "r"(smem_u32(bar))
-                 : "memory");
-}
-__device__ __forceinline__ void mbar_wait(unsigned long long* bar, unsigned parity) {
-    unsigned ok;
-    do {
-        asm volatile("{\n\t.reg .pred p;\n\tmbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\tselp.u32 %0, 1, 0, p;\n\t}"
-                     : "=r"(ok)
-                     : "r"(smem_u32(bar)), "r"(parity)
-                     : "memory");
-    } while (!ok);
-}
-#ifndef K3_STAGE_CAND
-#define K3_STAGE_CAND 0    // (measured r2t: 577 us against 565 without) 1: the first two candidate records of every row of the chunk (one contiguous run per level) are
-                           // fetched by ONE thread with TMA bulk copies at the start of the CTA and wait in shared memory when
-                           // the scan gets there: the scan's DRAM round trip (the largest stall of the kernel) is gone
-#endif
-constexpr int K3_CAND_ARENA = 36864;  // bytes of staged records: two levels x 576 rows x 32 B
-#ifndef K3_STAGE_TABLES
-#define K3_STAGE_TABLES 0  // 1: the tables of the chunk are fetched with cp.async into fixed shared-memory slots, then walked
-                           // there.  Measured (r2s): 635 us against 560 without — the barrier in front of the walk costs
-                           // more than the serial walk from global memory, whose latency the other 39 warps hide
-#endif
 #ifndef K3_DIRECT_J
 #define K3_DIRECT_J 1      // 1: a lane stores the 7 Jacobian entries of its row itself (56 contiguous bytes); 0: transposition
 #endif
-constexpr int K3_LSLOT = 12;   // monomials of a link table staged in shared memory (longer tables: the rest from global memory)
-constexpr int K3_USLOT = 32;   // same for a torque table
-constexpr int K3_LTAB_BYTES = 32 + K3_LSLOT * 24;  // keys (24 B used), then coefficients [m][3]
-constexpr int K3_UTAB_BYTES = K3_USLOT * 2 + K3_USLOT * 8;
-__device__ __forceinline__ void cp_async16(void* dst, const void* src) {
-    asm volatile("cp.async.ca.shared.global [%0], [%1], 16;" ::"r"((unsigned)__cvta_generic_to_shared(dst)), "l"(src) : "memory");
-}
 #ifndef K3_SKIP_ZERO_DK
 #define K3_SKIP_ZERO_DK 0   // 1: no look-ups / products for d/dk_v with v above the link index (exactly zero); measured: no gain
 #endif
@@ -609,8 +703,6 @@ k_constraints(Batch B, const double* __restrict__ kin, double* __restrict__ g, d
     __shared__ double s_stage[K3_WARPS][32 * NF];  // per-warp transpose buffer: Jacobian rows leave coalesced
 #endif
     __shared__ double s_tj[TB * NF * NF];          // torque rows of the Jacobian: leave as one contiguous run
-    extern __shared__ __align__(16) unsigned char k3_tab[];  // staged tables (K3_STAGE_TABLES), then staged candidate records
-    __shared__ unsigned long long s_bar;                     // completion of the candidate copy
     __shared__ int s_in_domain;
     __shared__ int s_next;  // next chunk of 32 collision rows
 
@@ -639,34 +731,6 @@ k_constraints(Batch B, const double* __restrict__ kin, double* __restrict__ g, d
         }
         return;
     }
-#if K3_STAGE_CAND
-    // rows [0, rows_staged) of candidate levels 0 and 1: [level][row][4] in shared memory
-    const int rows_all = NJ * TB * O;
-    const int rows_staged = rows_all < K3_CAND_ARENA / 64 ? rows_all : K3_CAND_ARENA / 64;
-    double* const s_rec = reinterpret_cast<double*>(k3_tab + (K3_STAGE_TABLES ? TB * (NJ * K3_LTAB_BYTES + NF * K3_UTAB_BYTES) : 0));
-    if (tid == 0) {
-        mbar_init(&s_bar, 1);
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-        const double* src = B.hp_cand + (size_t(p) * (T / TB) + tb) * B.hp_chunk();
-        const unsigned bytes = unsigned(rows_staged) * 32u;
-        mbar_arrive_expect_tx(&s_bar, rows_staged > 0 ? 2 * bytes : 0);
-        if (rows_staged > 0) {
-            bulk_g2s(s_rec, src, bytes, &s_bar);
-            bulk_g2s(s_rec + size_t(rows_staged) * 4, src + size_t(rows_all) * 4, bytes, &s_bar);
-        }
-    }
-#endif
-#ifndef K3_PREFETCH_L2
-#define K3_PREFETCH_L2 0   // measured r2v: 553 us with, 551 without
-#endif
-#if K3_PREFETCH_L2
-    {   // the first two candidate records of every row of the chunk are two contiguous runs: ask L2 for them now, the scan
-        // reads them after the slices (no registers, no shared memory, no wait)
-        const char* c0p = reinterpret_cast<const char*>(B.hp_cand + (size_t(p) * (T / TB) + tb) * B.hp_chunk());
-        const int lines = (NJ * TB * O * 32 * 2 + 127) / 128;
-        for (int i = tid; i < lines; i += K3_THREADS) asm volatile("prefetch.global.L2 [%0];" ::"l"(c0p + size_t(i) * 128));
-    }
-#endif
     if (tid == 32) {
         bool in = true;
         for (int j = 0; j < NF; j++) in = in && (fabs(kin[size_t(p) * NF + j]) <= K_DOMAIN);
@@ -693,6 +757,8 @@ k_constraints(Batch B, const double* __restrict__ kin, double* __restrict__ g, d
 #endif
     const int per_pair = NJ * TB * O;
     const size_t chunk = size_t(p) * (T / TB) + tb;
+    const unsigned char* __restrict__ img = B.img + chunk * B.img_chunk();  // everything this CTA reads of the build
+    const double* __restrict__ imgd = reinterpret_cast<const double*>(img);
     const bool cnt_in_smem = per_pair <= K3_CNT_SMEM;
     __syncthreads();
 
@@ -706,7 +772,7 @@ k_constraints(Batch B, const double* __restrict__ kin, double* __restrict__ g, d
         constexpr int CW = (K3_CNT_SMEM / 4 + K3_LINK_THREADS - 1) / K3_LINK_THREADS;
         unsigned cw[CW];
         if (cnt_in_smem) {
-            const unsigned* src = reinterpret_cast<const unsigned*>(B.hp_cnt + chunk * per_pair);
+            const unsigned* src = reinterpret_cast<const unsigned*>(img + B.img_cnt());
 #pragma unroll
             for (int q = 0; q < CW; q++) cw[q] = (tid + q * K3_LINK_THREADS < per_pair / 4) ? __ldg(src + tid + q * K3_LINK_THREADS) : 0u;
         }
@@ -714,40 +780,15 @@ k_constraints(Batch B, const double* __restrict__ kin, double* __restrict__ g, d
         const int e = tid % 3;
         const int l = (tid / 3) % NJ;
         const int tt = slicer ? tid / (3 * NJ) : 0;
-        const size_t idx = (size_t(p) * T + tb * TB + tt) * NJ + l;
-        const int n = slicer ? B.link_n[idx] : 0;
-#if K3_STAGE_TABLES
-        // the three component threads of a table fetch its first K3_LSLOT monomials in 16-byte pieces (cp.async), all link
-        // warps meet (at a point where every warp is convergent: bar.sync is the aligned form), then each thread walks its
-        // table in shared memory: two DRAM round trips instead of one per pair of monomials
-        unsigned char* slot = k3_tab + (tt * NJ + l) * K3_LTAB_BYTES;
-        const int ns = n < K3_LSLOT ? n : K3_LSLOT;
+        const int li = tt * NJ + l;  // table of the chunk
+        const int2 lt = slicer ? reinterpret_cast<const int2*>(img)[li] : make_int2(0, 0);
         if (slicer) {
-            const char* ksrc = reinterpret_cast<const char*>(B.link_key + idx * B.capL);
-            const char* csrc = reinterpret_cast<const char*>(B.link_g + idx * B.capL * 3);
-            const int kc = (ns * 2 + 15) >> 4, cc = (ns * 24 + 15) >> 4;
-            if (e == 0)
-                for (int c = 0; c < kc; c++) cp_async16(slot + 16 * c, ksrc + 16 * c);
-            for (int c = e; c < cc; c += 3) cp_async16(slot + 32 + 16 * c, csrc + 16 * c);
-        }
-        asm volatile("cp.async.commit_group;" ::: "memory");
-        asm volatile("cp.async.wait_group 0;" ::: "memory");
-        __syncwarp();
-        asm volatile("bar.sync 4, %0;" ::"n"(K3_LINK_THREADS) : "memory");
-#endif
-        if (slicer) {
-            double value = B.link_c[idx * 3 + e];
+            double value = reinterpret_cast<const double*>(img + B.img_lc())[li * 3 + e];
             double grad[NF] = {0, 0, 0, 0, 0, 0, 0};
-#if K3_STAGE_TABLES
-            K3_SLICE(reinterpret_cast<const uint16_t*>(slot), reinterpret_cast<const double*>(slot + 32) + e, ns, 1, 3, K3_SLICE_TABLES,
-                            value, grad);
-            if (n > ns)
-                K3_SLICE(B.link_key + idx * B.capL + ns, B.link_g + (idx * B.capL + ns) * 3 + e, n - ns, 1, 3, K3_SLICE_TABLES, value, grad);
-#else
-            K3_SLICE(B.link_key + idx * B.capL, B.link_g + idx * B.capL * 3 + e, n, 1, 3, K3_SLICE_TABLES, value, grad);
-#endif
+            // 32-byte records: coefficient e at double e, the key in the low half-word of double 3 (half-word 12)
+            K3_SLICE(reinterpret_cast<const uint16_t*>(imgd + lt.x) + 12, imgd + lt.x + e, lt.y, 16, 4, K3_SLICE_TABLES, value, grad);
             // centre of Interval(c - r, c + r), as getCenter(slice()) does (KPR/NLPclass.cu:313)
-            const double r = B.link_r[idx * 3 + e];
+            const double r = reinterpret_cast<const double*>(img + B.img_lr())[li * 3 + e];
             const double c = ((value - r) + (value + r)) * 0.5;
             s_lc[tt][l][e] = c;
             if (p == 0) B.link_sliced[((size_t(tb) * TB + tt) * NJ + l) * 3 + e] = c;  // armtd_NLP::link_sliced_center
@@ -767,43 +808,14 @@ k_constraints(Batch B, const double* __restrict__ kin, double* __restrict__ g, d
         double value = 0.0;
         double grad[NF] = {0, 0, 0, 0, 0, 0, 0};
         const bool on = i < TB * NF;
-        const size_t idx = (size_t(p) * T + tb * TB) * NF + (on ? i : 0);
+        const int4 ut = on ? reinterpret_cast<const int4*>(img + B.img_ut())[i] : make_int4(0, 0, 0, 0);
         if (on) {
             // lane `part` takes the monomials part, part + 2, ...; the two partial sums are added below
             // (the oracle adds the monomials one after the other: a difference of a few ulp)
-            const int n = B.u_n[idx];
-#if K3_STAGE_TABLES
-            unsigned char* slot = k3_tab + TB * NJ * K3_LTAB_BYTES + i * K3_UTAB_BYTES;
-            const int ns = n < K3_USLOT ? n : K3_USLOT;
-            {
-                const char* ksrc = reinterpret_cast<const char*>(B.u_key + idx * B.capU);
-                const char* csrc = reinterpret_cast<const char*>(B.u_g + idx * B.capU);
-                const int kc = (ns * 2 + 15) >> 4, cc = (ns * 8 + 15) >> 4;
-                for (int c = part; c < kc; c += K3_TORQUE_LANES) cp_async16(slot + 16 * c, ksrc + 16 * c);
-                for (int c = part; c < cc; c += K3_TORQUE_LANES) cp_async16(slot + K3_USLOT * 2 + 16 * c, csrc + 16 * c);
-            }
-        }
-        asm volatile("cp.async.commit_group;" ::: "memory");
-        asm volatile("cp.async.wait_group 0;" ::: "memory");
-        __syncwarp();
-        asm volatile("bar.sync 5, %0;" ::"n"(K3_THREADS - K3_LINK_THREADS) : "memory");
-        if (on) {
-            const int n = B.u_n[idx];
-            unsigned char* slot = k3_tab + TB * NJ * K3_LTAB_BYTES + i * K3_UTAB_BYTES;
-            const int ns = n < K3_USLOT ? n : K3_USLOT;
-            const int mine_s = (ns - part + K3_TORQUE_LANES - 1) / K3_TORQUE_LANES;
-            K3_SLICE(reinterpret_cast<const uint16_t*>(slot) + part, reinterpret_cast<const double*>(slot + K3_USLOT * 2) + part,
-                            mine_s > 0 ? mine_s : 0, K3_TORQUE_LANES, K3_TORQUE_LANES, K3_SLICE_TABLES, value, grad);
-            if (n > ns) {  // K3_USLOT is even: lane `part` continues at monomial K3_USLOT + part
-                const int rest = (n - ns - part + K3_TORQUE_LANES - 1) / K3_TORQUE_LANES;
-                K3_SLICE(B.u_key + idx * B.capU + ns + part, B.u_g + idx * B.capU + ns + part, rest > 0 ? rest : 0,
-                                K3_TORQUE_LANES, K3_TORQUE_LANES, K3_SLICE_TABLES, value, grad);
-            }
-#else
+            const int n = ut.z;
             const int mine = (n - part + K3_TORQUE_LANES - 1) / K3_TORQUE_LANES;
-            K3_SLICE(B.u_key + idx * B.capU + part, B.u_g + idx * B.capU + part, mine > 0 ? mine : 0,
+            K3_SLICE(reinterpret_cast<const uint16_t*>(img) + ut.y + part, imgd + ut.x + part, mine > 0 ? mine : 0,
                             K3_TORQUE_LANES, K3_TORQUE_LANES, K3_SLICE_TABLES, value, grad);
-#endif
         }
 #pragma unroll
         for (int d = 1; d < K3_TORQUE_LANES; d <<= 1) {
@@ -813,8 +825,8 @@ k_constraints(Batch B, const double* __restrict__ kin, double* __restrict__ g, d
         }
         double* st = s_tj;
         if (on && part == 0) {
-            value = B.u_c[idx] + value;
-            const double r = B.u_r[idx];
+            value = reinterpret_cast<const double*>(img + B.img_uc())[i] + value;
+            const double r = reinterpret_cast<const double*>(img + B.img_ur())[i];
             if (gp) gp[tb * TB * NF + i] = ((value - r) + (value + r)) * 0.5;
 #pragma unroll
             for (int v = 0; v < NF; v++) st[i * NF + v] = grad[v];
@@ -829,16 +841,14 @@ k_constraints(Batch B, const double* __restrict__ kin, double* __restrict__ g, d
     }
 
     // ---- phase 2: collision rows.  x = (l*TB + tt)*O + o; 32 consecutive rows per warp pass
-    const double* cand = B.hp_cand + chunk * B.hp_chunk();
-    const unsigned char* cnt = B.hp_cnt + chunk * per_pair;
-    const size_t cstride2 = size_t(per_pair) * 2;  // candidate stride in double2 units
+    // the stored records of the chunk, row after row; grp[g] = records of the rows before row 32 g
+    const double2* __restrict__ cand = reinterpret_cast<const double2*>(img + B.img_hdr());
+    const unsigned* __restrict__ grp = reinterpret_cast<const unsigned*>(img + B.img_grp());
+    const unsigned char* cnt = img + B.img_cnt();
     const bool in_domain = s_in_domain != 0;
     const float inv_O = O > 0 ? 1.0f / float(O) : 0.0f;
 #if !K3_DIRECT_J
     double* stage = &s_stage[warp][0];
-#endif
-#if K3_STAGE_CAND
-    mbar_wait(&s_bar, 0);  // issued before the slices: complete long ago (and nothing may be in flight when the CTA exits)
 #endif
     for (;;) {
         int x0 = 0;
@@ -847,33 +857,31 @@ k_constraints(Batch B, const double* __restrict__ kin, double* __restrict__ g, d
         if (x0 >= per_pair) break;
         const int x = x0 + lane;
         bool active = x < per_pair;
+        const unsigned base = grp[x0 >> 5];
         double max_elt = -100000000;
         double A0 = 0, A1 = 0, A2 = 0;  // minus the winning signed normal
         int l = 0, tt = 0, o = 0;
+        const int n = active ? (cnt_in_smem ? s_cnt[x] : cnt[x]) : 0;
+        // first record of the row: base + the records of the warp's earlier rows (inclusive scan over the lanes)
+        const int stored = n == HP_OVERFLOW ? 0 : n;
+        int before = stored;
+#pragma unroll
+        for (int d = 1; d < 32; d <<= 1) {
+            const int t = __shfl_up_sync(0xffffffffu, before, d);
+            if (lane >= d) before += t;
+        }
+        before -= stored;
         if (active) {
             const int ltt = __float2int_rz((float(x) + 0.5f) * inv_O);  // x / O, exact for x < 2^22
             o = x - ltt * O;
             tt = ltt % TB;
             l = ltt / TB;
             const double c0 = s_lc[tt][l][0], c1 = s_lc[tt][l][1], c2 = s_lc[tt][l][2];
-            const int n = cnt_in_smem ? s_cnt[x] : cnt[x];
             if (n != HP_OVERFLOW && in_domain) {
-                const double2* row = reinterpret_cast<const double2*>(cand) + size_t(x) * 2;
+                const double2* row = cand + size_t(base + unsigned(before)) * 2;
                 // K3_CQ candidate records in flight per thread (the scan itself stays in order)
                 for (int q0 = 0; q0 < n; q0 += K3_CQ) {
                     double2 u[K3_CQ], w[K3_CQ];
-#if K3_STAGE_CAND
-                    static_assert(K3_CQ == 2, "the staged levels are the first pass of the scan");
-                    if (q0 == 0 && x < rows_staged) {
-                        const double2* sr = reinterpret_cast<const double2*>(s_rec) + size_t(x) * 2;
-                        u[0] = sr[0];
-                        w[0] = sr[1];
-                        if (n > 1) {
-                            u[1] = sr[size_t(rows_staged) * 2];
-                            w[1] = sr[size_t(rows_staged) * 2 + 1];
-                        }
-                    } else
-#endif
 #pragma unroll
                     for (int i = 0; i < K3_CQ; i++) {
                         if (q0 + i < n) {
@@ -885,10 +893,10 @@ k_constraints(Batch B, const double* __restrict__ kin, double* __restrict__ g, d
                             asm volatile("ld.global.nc.v4.f64 {%0, %1, %2, %3}, [%4];"
 #endif
                                          : "=d"(u[i].x), "=d"(u[i].y), "=d"(w[i].x), "=d"(w[i].y)
-                                         : "l"(row + (q0 + i) * cstride2));
+                                         : "l"(row + (q0 + i) * 2));
 #else
-                            u[i] = __ldg(row + (q0 + i) * cstride2);
-                            w[i] = __ldg(row + (q0 + i) * cstride2 + 1);
+                            u[i] = __ldg(row + (q0 + i) * 2);
+                            w[i] = __ldg(row + (q0 + i) * 2 + 1);
 #endif
                         }
                     }
@@ -1215,11 +1223,8 @@ cudaError_t launch_constraints(const Batch& B, const double* d_k, double* d_g, d
     }
 #endif
     dim3 grid(B.T / TB, B.nprob);
-    const int rows_all = B.NJ * TB * B.O;
-    const size_t dyn = (K3_STAGE_TABLES ? size_t(TB) * (B.NJ * K3_LTAB_BYTES + NF * K3_UTAB_BYTES) : 0) +
-                       (K3_STAGE_CAND ? size_t(rows_all < K3_CAND_ARENA / 64 ? rows_all : K3_CAND_ARENA / 64) * 64 : 0);
     if (B.O == 0) {
-        k_constraints<<<grid, K3_THREADS, dyn, st>>>(B, d_k, d_g, d_jac);
+        k_constraints<<<grid, K3_THREADS, 0, st>>>(B, d_k, d_g, d_jac);
         return cudaGetLastError();
     }
     // slow path first (a normal launch: it waits for whatever precedes it on the stream), the main kernel behind it as a
@@ -1230,7 +1235,7 @@ cudaError_t launch_constraints(const Batch& B, const double* d_k, double* d_g, d
     cudaLaunchConfig_t cfg = {};
     cfg.gridDim = grid;
     cfg.blockDim = dim3(K3_THREADS);
-    cfg.dynamicSmemBytes = dyn;
+    cfg.dynamicSmemBytes = 0;
     cfg.stream = st;
     cudaLaunchAttribute attr[1];
     attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;

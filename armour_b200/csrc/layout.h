@@ -48,12 +48,22 @@ struct Batch {
     double* torque_radius;    // [p][j*T + t]
     double* link_gens;        // [p][t][NJ][18]     column-major 3x6
     double* link_r;           // [p][t][NJ][3]      diag of the radius block of link_gens (all an evaluation needs)
-    // collision half-space candidates: records [p][t/TB][candidate][l][t%TB][o][4] = (s*Cx, s*Cy, s*Cz, b): candidate-
-    // major inside a chunk, so that the q-th records of 32 consecutive rows are one contiguous KB; the number of candidates
-    // per row [p][t/TB][l][t%TB][o] (HP_OVERFLOW: no list); and per problem the number of rows without a list
-    double* hp_cand;
+    // collision half-space candidates: the number of candidates per row [p][t/TB][l][t%TB][o] (HP_OVERFLOW: no list), and per
+    // problem the number of rows without a list.  The records themselves live in the evaluation image (img below).
     unsigned char* hp_cnt;
     int* hp_slow;
+    // evaluation images, one fixed slot of img_chunk() bytes per chunk [p][t/TB]: everything k_constraints reads for one
+    // (problem, TB intervals), packed at the end of every build so that the kernel reads only the bytes it uses.
+    //   header   int2 [TB][NJ] link tables (first double of the table in the image, monomials)
+    //            int4 [TB][NF] torque tables (first coefficient in doubles, first key in uint16 units, monomials, 0)
+    //            double [TB][NJ][3] link centres, [TB][NJ][3] link radii, [TB][NF] torque centres, [TB][NF] torque radii
+    //            uint32 [ngrp] stored candidates of the rows before row 32 g; uint8 [rows] candidate counts (hp_cnt)
+    //   img_hdr()  candidate records (s*Cx, s*Cy, s*Cz, b) row after row in scan order (CSR: rows in the chunk's x order)
+    //   then     link tables back to back, one 32-byte record (3 coefficients, key in the low 16 bits of the fourth double)
+    //            per monomial; torque coefficients of all tables back to back, then their keys
+    // During the build k_hyperplanes writes each row's candidates into a fixed run of HP_CAP records at img_hdr(); the pack
+    // kernel compacts them in place (a record never moves up) and appends the tables.
+    unsigned char* img;
     // outputs of the last evaluation
     double* link_sliced;      // [t][NJ][3] of problem 0 (armtd_NLP::link_sliced_center)
     int* status;              // [p] epoch * 8 + failure code of a build that overflowed a table (see failed()): evaluations
@@ -62,7 +72,20 @@ struct Batch {
     // CTA row y works on problem plist[y]; nullptr = identity
     const int* plist;
 
-    __host__ __device__ size_t hp_chunk() const { return size_t(HP_CAP) * 4 * NJ * TB * O; }
+    // byte offsets inside one evaluation image (see img)
+    __host__ __device__ int img_rows() const { return NJ * TB * O; }
+    __host__ __device__ size_t img_ut() const { return size_t(TB) * NJ * 8; }
+    __host__ __device__ size_t img_lc() const { return img_ut() + size_t(TB) * NF * 16; }
+    __host__ __device__ size_t img_lr() const { return img_lc() + size_t(TB) * NJ * 24; }
+    __host__ __device__ size_t img_uc() const { return img_lr() + size_t(TB) * NJ * 24; }
+    __host__ __device__ size_t img_ur() const { return img_uc() + size_t(TB) * NF * 8; }
+    __host__ __device__ size_t img_grp() const { return img_ur() + size_t(TB) * NF * 8; }
+    __host__ __device__ size_t img_cnt() const { return img_grp() + size_t(img_rows() + 31) / 32 * 4; }
+    __host__ __device__ size_t img_hdr() const { return (img_cnt() + img_rows() + 127) / 128 * 128; }
+    __host__ __device__ size_t img_chunk() const {
+        const size_t tables = size_t(TB) * NJ * capL * 32 + size_t(TB) * NF * capU * 10;
+        return (img_hdr() + size_t(img_rows()) * HP_CAP * 32 + tables + 127) / 128 * 128;
+    }
     __host__ __device__ int m() const { return NF * T + NJ * T * O + 4 * NF; }
     // failure code of problem p in the CURRENT build (0: none); stamps of older builds do not count
     __device__ int failed(int p) const { return (status[p] >> 3) == epoch ? (status[p] & 7) : 0; }

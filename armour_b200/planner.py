@@ -126,6 +126,23 @@ class ReachSetEngine:
             self._check(self.lib.armour_batch_get_candidate_counts(self._h, self.nprob, out.ctypes.data_as(C.c_void_p)))
         return out
 
+    def eval_image_layout(self):
+        """Byte offsets inside one chunk's evaluation image at the current obstacle count, and its size ("chunk").
+        Layout in DESIGN.md."""
+        lay = (C.c_longlong * 10)()
+        self._check(self.lib.armour_eval_image_layout(self._h, lay))
+        names = ("chunk", "link_tables", "torque_tables", "link_c", "link_r", "u_c", "u_r", "groups", "counts", "records")
+        return dict(zip(names, (int(v) for v in lay)))
+
+    def eval_images(self):
+        """Evaluation images of the built problems: (uint8 [nprob, T/C, bytes per chunk], eval_image_layout()).  An
+        inspection aid for tests and tools."""
+        layout = self.eval_image_layout()
+        C_ = self.lib.armour_chunk_intervals()
+        out = np.zeros((self.nprob, self.T // C_, layout["chunk"]), np.uint8)
+        self._check(self.lib.armour_batch_get_eval_images(self._h, self.nprob, out.ctypes.data_as(C.c_void_p)))
+        return out, layout
+
     def solve(self, q_des, max_iter=None, tol=None, qp_sweeps=None, qp_update_budget=None):
         """Batched planning on the device (armour_batch_solve): the trust-region SQP of the C++ host solver run on the
         GPU for every built problem, from k = 0.  Returns (k_opt [nprob, 7], feasible [nprob] bool, first violated row

@@ -178,6 +178,14 @@ int armour_batch_get_monomial_counts(armour_ctx* ctx, int nprob, int* link_n, in
  * half-spaces per row (KPR/CollisionChecking.cu:169-228). */
 int armour_batch_get_candidate_counts(armour_ctx* ctx, int nprob, unsigned char* out);
 int armour_chunk_intervals(void);
+/* Evaluation images (inspection aid): at the end of every build the reach-set tables and candidate lists of each chunk of
+ * C intervals are packed into one contiguous image, which is all the evaluation kernel reads.  layout receives 10 byte
+ * counts: image bytes per chunk, then the offsets of the link-table entries, torque-table entries, link centres, link
+ * radii, torque centres, torque radii, row-group bases, candidate counts and candidate records (see DESIGN.md).
+ * armour_batch_get_eval_images copies the images of problems 0..nprob-1 ([p][T/C] chunks of that size) into out.
+ * Images of problems whose build failed are not written. */
+int armour_eval_image_layout(armour_ctx* ctx, long long* layout);
+int armour_batch_get_eval_images(armour_ctx* ctx, int nprob, void* out);
 /* Measurement aid: runs a dependent-chain-free FP64 FMA kernel on the context's device and returns the
  * sustained non-tensor FP64 rate in TFLOP/s (the FP64 roofline denominator; BASELINE.md section 2). */
 int armour_measure_fp64_peak(armour_ctx* ctx, double* tflops);
