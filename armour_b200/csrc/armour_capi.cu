@@ -102,9 +102,11 @@ __device__ int g_k1spill[8];  // arena blocks in global memory, all arena blocks
 #include "armtd.cuh"
 #include "rollout.cuh"
 #include "layout.h"
+#include "device_buffer.h"
 
 using namespace armour;
 
+// Every device allocation of a context is one of its DeviceBuffer members (or K1Scratch's); the pointers of B are views of them.
 struct armour_ctx {
     armour_config cfg;
     RobotConstants rc;
@@ -112,25 +114,23 @@ struct armour_ctx {
     cudaStream_t own_stream = nullptr;
     Batch B;                 // device pointers + dimensions of the current batch
     int built_nprob = 0;     // problems with valid reach sets
-    size_t img_capacity = 0; // bytes allocated for B.img
-    size_t cnt_capacity = 0; // bytes allocated for B.hp_cnt
-    int hp_nprob = 0;        // problems the candidate buffers were sized for
-    int* d_unit_flag = nullptr;  // [max_problems * T] completion stamps of the reach-set units (latency path)
-    size_t obs_capacity = 0;
-    double* d_in = nullptr;  // [3][max_problems][NF] q0, qd0, qdd0
-    double* d_obs = nullptr;
-    double* d_k = nullptr;   // staging for the host-pointer evaluation calls
-    double* d_g = nullptr;
-    double* d_jac = nullptr;
-    size_t g_capacity = 0, jac_capacity = 0;
-    double* d_jnz = nullptr;  // packed non-zeros of the Jacobian (structured evaluation)
-    size_t jnz_capacity = 0;
-    int* d_verdict = nullptr;  // [2][max_problems]
+    // reach-set tables of max_problems problems, allocated at creation (B.link_n ... B.status)
+    DeviceBuffer<int> link_n, u_n, status;
+    DeviceBuffer<double> link_c, link_g, u_c, u_r, u_g, torque_radius, link_gens, link_r, link_sliced;
+    DeviceBuffer<uint16_t> link_key, u_key;
+    // sized for the batch by ensure_obstacle_buffers (B.obstacles, B.img, B.hp_cnt, B.hp_slow)
+    DeviceBuffer<double> d_obs;
+    DeviceBuffer<unsigned char> img, hp_cnt;
+    DeviceBuffer<int> hp_slow;
+    DeviceBuffer<int> d_unit_flag;  // [max_problems * T] completion stamps of the reach-set units (latency path)
+    DeviceBuffer<double> d_in;      // [3][max_problems][NF] q0, qd0, qdd0
+    DeviceBuffer<double> d_k;       // staging for the host-pointer evaluation calls
+    DeviceBuffer<double> d_g, d_jac;
+    DeviceBuffer<double> d_jnz;     // packed non-zeros of the Jacobian (structured evaluation)
+    DeviceBuffer<int> d_verdict;    // [2][max_problems]
     // batched device solver (allocated on first use)
-    double* d_solver = nullptr;   // state arrays + second g buffer + linearised rows
-    int* d_solver_i = nullptr;    // have_best, status, iters, evals, running counter
-    double* d_solver_io = nullptr;  // q_des, k_opt staging of the host-pointer call
-    size_t solver_doubles = 0, solver_ints = 0;  // elements allocated for d_solver / d_solver_i
+    DeviceBuffer<double> d_solver;  // state arrays + second g buffer + linearised rows
+    DeviceBuffer<int> d_solver_i;   // have_best, status, iters, evals, running counter
     k1lat::K1Scratch k1_lat;  // scratch of the latency configuration of k_reachsets
     k1thr::K1Scratch k1_thr;  // scratch of the throughput configuration (allocated on first use)
     bool k1_thr_ready = false;
@@ -141,22 +141,19 @@ struct armour_ctx {
     std::vector<double> h_q0, h_qd0, h_qdd0;
     // ARMTD comparison planner (armour_armtd_*): imported joint reachable set, KPA-layout outputs, trajectory parameters
     bool armtd = false;
-    double* d_jrs = nullptr;       // [max_problems][ARMTD_T_PADDED][NF][6] the offline table rotated by q0 (B.jrs_ext)
-    double* d_armtd_in = nullptr;  // one allocation for the four arrays below
+    DeviceBuffer<double> d_jrs;       // [max_problems][ARMTD_T_PADDED][NF][6] the offline table rotated by q0 (B.jrs_ext)
+    DeviceBuffer<double> d_armtd_in;  // one allocation for the four arrays below
     double* d_krange = nullptr;    // [max_problems][NF] k_range of each problem
     double* d_zero = nullptr;      // [max_problems][NF] zeros: qdd0 of the build (unused by the forward kinematics)
     double* d_cs = nullptr;        // [max_problems][NF][2] cos q0, sin q0 staged by the host-pointer build
     double* d_jrs_raw = nullptr;   // [max_problems][6][NF][ARMTD_T] offline tables staged by the host-pointer build
-    double* d_ga = nullptr;        // [nprob][m_armtd] KPA-layout g of the host-pointer calls and of the solver
-    double* d_ja = nullptr;        // [nprob][m_armtd][NF]
-    size_t ga_capacity = 0, ja_capacity = 0;
+    DeviceBuffer<double> d_ga;     // [nprob][m_armtd] KPA-layout g of the host-pointer calls and of the solver
+    DeviceBuffer<double> d_ja;     // [nprob][m_armtd][NF]
     std::vector<double> h_krange;  // host mirror of d_krange for the cost (empty: fetched after a device build)
-    // closed-loop episodes (armour_batch_rollout*) and clearance queries (allocated on first use, grow only)
-    double* d_roll = nullptr;   // per-world state, current plans and the dense batch of a rollout
-    int* d_roll_i = nullptr;    // outcomes, counters, world lists, verdicts
-    size_t roll_doubles = 0, roll_ints = 0;
-    char* d_stage = nullptr;    // staging of the host-pointer rollout / clearance calls
-    size_t stage_bytes = 0;
+    // closed-loop episodes (armour_batch_rollout*), allocated on first use
+    DeviceBuffer<double> d_roll;  // per-world state, current plans and the dense batch of a rollout
+    DeviceBuffer<int> d_roll_i;   // outcomes, counters, world lists, verdicts
+    DeviceBuffer<char> d_stage;   // inputs and outputs of the host-pointer calls that stage (see stage())
 };
 
 namespace {
@@ -187,63 +184,39 @@ int fail(armour_ctx* c, int code, const std::string& msg) {
             return fail(ctx, ARMOUR_ERR_CUDA, std::string(#expr) + ": " + cudaGetErrorString(e__)); \
     } while (0)
 
-template <class T>
-cudaError_t dalloc(T** p, size_t n) {
-    return cudaMalloc(reinterpret_cast<void**>(p), std::max<size_t>(n, 1) * sizeof(T));
-}
-
-int ensure_eval_buffers(armour_ctx* ctx, int nprob, bool need_g, bool need_jac) {
-    const size_t m = size_t(ctx->B.m());
-    if (need_g && ctx->g_capacity < nprob * m) {
-        if (ctx->d_g) cudaFree(ctx->d_g);
-        ctx->d_g = nullptr;
-        CU(dalloc(&ctx->d_g, nprob * m));
-        ctx->g_capacity = nprob * m;
-    }
-    if (need_jac && ctx->jac_capacity < nprob * m * NF) {
-        if (ctx->d_jac) cudaFree(ctx->d_jac);
-        ctx->d_jac = nullptr;
-        CU(dalloc(&ctx->d_jac, nprob * m * NF));
-        ctx->jac_capacity = nprob * m * NF;
-    }
+// d_g / d_jac for `rows` constraint rows (of all problems together)
+int ensure_eval_buffers(armour_ctx* ctx, size_t rows, bool need_g, bool need_jac) {
+    if (need_g) CU(ctx->d_g.reserve(rows));
+    if (need_jac) CU(ctx->d_jac.reserve(rows * NF));
     return ARMOUR_OK;
 }
 
+// The obstacle, image and candidate-count buffers of a batch of nprob problems with nobs obstacles each.  The current batch
+// (B.O, B.nprob) is the caller's to set.
 int ensure_obstacle_buffers(armour_ctx* ctx, int nprob, int nobs) {
-    const size_t need_obs = size_t(nprob) * nobs * 12;
-    if (ctx->obs_capacity < need_obs) {
-        if (ctx->d_obs) cudaFree(ctx->d_obs);
-        ctx->d_obs = nullptr;
-        CU(dalloc(&ctx->d_obs, need_obs));
-        ctx->obs_capacity = need_obs;
-    }
     Batch& B = ctx->B;
-    B.O = nobs;
-    B.nprob = nprob;
-    const size_t need_img = size_t(nprob) * (B.T / TB) * B.img_chunk();
+    Batch next = B;
+    next.O = nobs;
+    const size_t need_img = size_t(nprob) * (B.T / TB) * next.img_chunk();
     const size_t need_cnt = size_t(nprob) * B.T * B.NJ * nobs;
-    if (ctx->img_capacity < need_img || ctx->hp_nprob < nprob || ctx->cnt_capacity < need_cnt) {
-        // (the candidate lists and images of the current batch go with the old buffers: whatever was built must be rebuilt)
-        if (B.img) cudaFree(B.img);
-        if (B.hp_cnt) cudaFree(B.hp_cnt);
-        if (B.hp_slow) cudaFree(B.hp_slow);
-        B.img = nullptr;
-        B.hp_cnt = nullptr;
-        B.hp_slow = nullptr;
-        ctx->img_capacity = 0;
-        ctx->cnt_capacity = 0;
-        ctx->hp_nprob = 0;
-        ctx->built_nprob = 0;
-        const size_t np = std::max(nprob, ctx->hp_nprob);
-        CU(dalloc(&B.img, need_img));
-        CU(dalloc(&B.hp_cnt, need_cnt));
-        CU(dalloc(&B.hp_slow, np));
-        CU(cudaMemsetAsync(B.hp_slow, 0, np * sizeof(int), ctx->stream));
-        ctx->img_capacity = need_img;
-        ctx->cnt_capacity = need_cnt;
-        ctx->hp_nprob = nprob;
+    const bool regrow = ctx->img.capacity() < need_img || ctx->hp_cnt.capacity() < need_cnt || ctx->hp_slow.capacity() < size_t(nprob);
+    // growing drops the built batch: its candidate lists and images go with the old buffers.  (The obstacle buffer grows only
+    // when hp_cnt does, so a batch whose obstacles were freed is never left built either.)
+    if (regrow) ctx->built_nprob = 0;
+    CU(ctx->d_obs.reserve(size_t(nprob) * nobs * 12));
+    B.obstacles = ctx->d_obs.get();
+    if (regrow) {
+        ctx->img = {};
+        ctx->hp_cnt = {};
+        ctx->hp_slow = {};
+        CU(ctx->img.reserve(need_img));
+        CU(ctx->hp_cnt.reserve(std::max<size_t>(need_cnt, 1)));  // (one byte without obstacles: B.hp_cnt is never null)
+        CU(ctx->hp_slow.reserve(nprob));
+        CU(cudaMemsetAsync(ctx->hp_slow.get(), 0, nprob * sizeof(int), ctx->stream));
+        B.img = ctx->img.get();
+        B.hp_cnt = ctx->hp_cnt.get();
+        B.hp_slow = ctx->hp_slow.get();
     }
-    B.obstacles = ctx->d_obs;
     return ARMOUR_OK;
 }
 
@@ -260,7 +233,7 @@ int launch_build(armour_ctx* ctx, const Batch& B, int* nl, bool* latency) {
         }
         CU(k1thr::launch_reachsets(B, ctx->k1_thr, ctx->stream, nl));
     } else {
-        CU(k1lat::launch_reachsets(B, ctx->k1_lat, ctx->stream, nl, ctx->d_unit_flag));
+        CU(k1lat::launch_reachsets(B, ctx->k1_lat, ctx->stream, nl, ctx->d_unit_flag.get()));
     }
     return ARMOUR_OK;
 }
@@ -287,6 +260,28 @@ int ensure_constants(armour_ctx* ctx) {
     CU(upload_constants(ctx->rc, ctx->stream));
     o.rc = ctx->rc;
     o.valid = true;
+    return ARMOUR_OK;
+}
+
+// First step of an entry point that launches: this context's device, and its constants on that device.
+int enter(armour_ctx* ctx) {
+    CU(cudaSetDevice(ctx->cfg.device));
+    return ensure_constants(ctx);
+}
+
+// The host-pointer calls that stage their inputs and outputs cut the context's one staging buffer into pieces of the given
+// sizes in bytes, 256-byte aligned (nullptr for a size of 0).  A call that stages may call only *_device entry points: any
+// other host-pointer call could stage over its pieces.
+template <size_t N>
+int stage(armour_ctx* ctx, const size_t (&bytes)[N], void* (&piece)[N]) {
+    size_t total = 0;
+    for (size_t b : bytes) total += (b + 255) / 256 * 256;
+    CU(ctx->d_stage.reserve(total));
+    char* p = ctx->d_stage.get();
+    for (size_t i = 0; i < N; i++) {
+        piece[i] = bytes[i] ? p : nullptr;
+        p += (bytes[i] + 255) / 256 * 256;
+    }
     return ARMOUR_OK;
 }
 
@@ -392,32 +387,36 @@ int armour_ctx_create(const armour_config* cfg, armour_ctx** out) {
     B.capL = cfg->cap_link_monomials;
     B.capU = cfg->cap_torque_monomials;
     const size_t P = size_t(cfg->max_problems), T = size_t(B.T), NJ = size_t(B.NJ);
-#define ALLOC(ptr, n) \
-    if ((e = dalloc(&ptr, (n))) != cudaSuccess) return bail(#ptr, e)
-    ALLOC(ctx->d_in, 3 * P * NF);
-    ALLOC(B.link_n, P * T * NJ);
-    ALLOC(B.link_c, P * T * NJ * 3);
-    ALLOC(B.link_key, P * T * NJ * B.capL);
-    ALLOC(B.link_g, P * T * NJ * B.capL * 3);
-    ALLOC(B.u_n, P * T * NF);
-    ALLOC(B.u_c, P * T * NF);
-    ALLOC(B.u_r, P * T * NF);
-    ALLOC(B.u_key, P * T * NF * B.capU);
-    ALLOC(B.u_g, P * T * NF * B.capU);
-    ALLOC(B.torque_radius, P * NF * T);
-    ALLOC(B.link_gens, P * T * NJ * 18);
-    ALLOC(B.link_r, P * T * NJ * 3);
-    ALLOC(B.link_sliced, P * T * NJ * 3);
-    ALLOC(B.status, P);
-    ALLOC(ctx->d_unit_flag, P * T);
-    ALLOC(ctx->d_k, P * NF);
-    ALLOC(ctx->d_verdict, 2 * P);
+#define ALLOC(buf, n) \
+    if ((e = ctx->buf.reserve(n)) != cudaSuccess) return bail(#buf, e)
+#define TABLE(field, n) \
+    ALLOC(field, n);    \
+    B.field = ctx->field.get()
+    ALLOC(d_in, 3 * P * NF);
+    TABLE(link_n, P * T * NJ);
+    TABLE(link_c, P * T * NJ * 3);
+    TABLE(link_key, P * T * NJ * B.capL);
+    TABLE(link_g, P * T * NJ * B.capL * 3);
+    TABLE(u_n, P * T * NF);
+    TABLE(u_c, P * T * NF);
+    TABLE(u_r, P * T * NF);
+    TABLE(u_key, P * T * NF * B.capU);
+    TABLE(u_g, P * T * NF * B.capU);
+    TABLE(torque_radius, P * NF * T);
+    TABLE(link_gens, P * T * NJ * 18);
+    TABLE(link_r, P * T * NJ * 3);
+    TABLE(link_sliced, P * T * NJ * 3);
+    TABLE(status, P);
+    ALLOC(d_unit_flag, P * T);
+    ALLOC(d_k, P * NF);
+    ALLOC(d_verdict, 2 * P);
+#undef TABLE
 #undef ALLOC
-    B.q0 = ctx->d_in;
-    B.qd0 = ctx->d_in + P * NF;
-    B.qdd0 = ctx->d_in + 2 * P * NF;
+    B.q0 = ctx->d_in.get();
+    B.qd0 = ctx->d_in.get() + P * NF;
+    B.qdd0 = ctx->d_in.get() + 2 * P * NF;
     if ((e = cudaMemsetAsync(B.status, 0, P * sizeof(int), ctx->stream)) != cudaSuccess) return bail("memset", e);
-    if ((e = cudaMemsetAsync(ctx->d_unit_flag, 0, P * T * sizeof(int), ctx->stream)) != cudaSuccess) return bail("memset", e);
+    if ((e = cudaMemsetAsync(ctx->d_unit_flag.get(), 0, P * T * sizeof(int), ctx->stream)) != cudaSuccess) return bail("memset", e);
     // no table may ever be read with an uninitialised count (a failed build leaves its tables untouched)
     if ((e = cudaMemsetAsync(B.link_n, 0, P * T * NJ * sizeof(int), ctx->stream)) != cudaSuccess) return bail("memset", e);
     if ((e = cudaMemsetAsync(B.u_n, 0, P * T * NF * sizeof(int), ctx->stream)) != cudaSuccess) return bail("memset", e);
@@ -444,17 +443,10 @@ int armour_ctx_create(const armour_config* cfg, armour_ctx** out) {
 int armour_ctx_destroy(armour_ctx* ctx) {
     if (!ctx) return ARMOUR_OK;
     cudaSetDevice(ctx->cfg.device);
-    Batch& B = ctx->B;
-    void* ptrs[] = {ctx->d_roll, ctx->d_roll_i, ctx->d_stage, ctx->d_solver, ctx->d_solver_i, ctx->d_solver_io, ctx->d_unit_flag, ctx->d_jnz, ctx->d_jrs, ctx->d_armtd_in, ctx->d_ga, ctx->d_ja,
-                    ctx->d_in, ctx->d_obs, ctx->d_k, ctx->d_g, ctx->d_jac, ctx->d_verdict, B.link_n, B.link_c,
-                    B.link_key, B.link_g, B.u_n, B.u_c, B.u_r, B.u_key, B.u_g, B.torque_radius, B.link_gens, B.link_r, B.img, B.hp_cnt, B.hp_slow,
-                    B.link_sliced, B.status};
-    for (void* p : ptrs)
-        if (p) cudaFree(p);
     k1lat::k1_scratch_destroy(&ctx->k1_lat);
     k1thr::k1_scratch_destroy(&ctx->k1_thr);
     if (ctx->own_stream) cudaStreamDestroy(ctx->own_stream);
-    delete ctx;
+    delete ctx;  // frees the buffers
     return ARMOUR_OK;
 }
 
@@ -480,17 +472,10 @@ int armour_num_constraints(const armour_ctx* ctx, int nobs) {
 int armour_ctx_reserve(armour_ctx* ctx, int nprob, int nobs) {
     int rc = check_batch(ctx, nprob, nobs);
     if (rc) return rc;
-    CU(cudaSetDevice(ctx->cfg.device));
-    { int rc_c = ensure_constants(ctx); if (rc_c) return rc_c; }
-    const int O = ctx->B.O, np = ctx->B.nprob;
-    rc = ensure_obstacle_buffers(ctx, nprob, nobs);
-    ctx->B.O = O;  // reserving does not change the current batch
-    ctx->B.nprob = np;
+    { int rc_e = enter(ctx); if (rc_e) return rc_e; }
+    rc = ensure_obstacle_buffers(ctx, nprob, nobs);  // (reserving does not change the current batch)
     if (rc) return rc;
-    ctx->B.O = nobs;
-    rc = ensure_eval_buffers(ctx, nprob, true, true);
-    ctx->B.O = O;
-    return rc;
+    return ensure_eval_buffers(ctx, size_t(nprob) * armour_num_constraints(ctx, nobs), true, true);
 }
 
 // ---- build -----------------------------------------------------------------------------------------
@@ -499,10 +484,12 @@ int armour_batch_reachsets_build_device(armour_ctx* ctx, int nprob, const double
     int rc = check_batch(ctx, nprob, nobs);
     if (rc) return rc;
     if (!d_q0 || !d_qd0 || !d_qdd0 || (nobs > 0 && !d_obstacles)) return fail(ctx, ARMOUR_ERR_ARG, "null input");
-    CU(cudaSetDevice(ctx->cfg.device));
-    { int rc_c = ensure_constants(ctx); if (rc_c) return rc_c; }
+    { int rc_e = enter(ctx); if (rc_e) return rc_e; }
     rc = ensure_obstacle_buffers(ctx, nprob, nobs);
     if (rc) return rc;
+    ctx->B.O = nobs;
+    ctx->B.nprob = nprob;
+    double* d_in = ctx->d_in.get();
     const size_t P = size_t(ctx->cfg.max_problems);
     ctx->B.epoch++;
     int nl = 0;
@@ -517,14 +504,14 @@ int armour_batch_reachsets_build_device(armour_ctx* ctx, int nprob, const double
         Bb.qdd0 = d_qdd0;
         Bb.obstacles = d_obstacles;
         { int rc2 = launch_build(ctx, Bb, &nl, &latency); if (rc2) return rc2; }
-        HpStage stage{ctx->d_in, ctx->d_in + P * NF, ctx->d_in + 2 * P * NF, ctx->d_obs};
-        CU(launch_hyperplanes(Bb, ctx->stream, latency ? ctx->d_unit_flag : nullptr, stage));
+        HpStage stage{d_in, d_in + P * NF, d_in + 2 * P * NF, ctx->d_obs.get()};
+        CU(launch_hyperplanes(Bb, ctx->stream, latency ? ctx->d_unit_flag.get() : nullptr, stage));
         nl++;
     } else {
         const size_t nb = size_t(nprob) * NF * sizeof(double);
-        CU(cudaMemcpyAsync(ctx->d_in, d_q0, nb, cudaMemcpyDeviceToDevice, ctx->stream));
-        CU(cudaMemcpyAsync(ctx->d_in + P * NF, d_qd0, nb, cudaMemcpyDeviceToDevice, ctx->stream));
-        CU(cudaMemcpyAsync(ctx->d_in + 2 * P * NF, d_qdd0, nb, cudaMemcpyDeviceToDevice, ctx->stream));
+        CU(cudaMemcpyAsync(d_in, d_q0, nb, cudaMemcpyDeviceToDevice, ctx->stream));
+        CU(cudaMemcpyAsync(d_in + P * NF, d_qd0, nb, cudaMemcpyDeviceToDevice, ctx->stream));
+        CU(cudaMemcpyAsync(d_in + 2 * P * NF, d_qdd0, nb, cudaMemcpyDeviceToDevice, ctx->stream));
         { int rc2 = launch_build(ctx, ctx->B, &nl, &latency); if (rc2) return rc2; }
     }
     CU(launch_pack_image(ctx->B, ctx->stream));
@@ -541,24 +528,26 @@ int armour_batch_reachsets_build(armour_ctx* ctx, int nprob, const double* q0, c
     int rc = check_batch(ctx, nprob, nobs);
     if (rc) return rc;
     if (!q0 || !qd0 || !qdd0 || (nobs > 0 && !obstacles)) return fail(ctx, ARMOUR_ERR_ARG, "null input");
-    CU(cudaSetDevice(ctx->cfg.device));
-    { int rc_c = ensure_constants(ctx); if (rc_c) return rc_c; }
+    { int rc_e = enter(ctx); if (rc_e) return rc_e; }
     rc = ensure_obstacle_buffers(ctx, nprob, nobs);
     if (rc) return rc;
+    ctx->B.O = nobs;
+    ctx->B.nprob = nprob;
+    double* d_in = ctx->d_in.get();
     const size_t P = size_t(ctx->cfg.max_problems);
     const size_t nb = size_t(nprob) * NF * sizeof(double);
-    CU(cudaMemcpyAsync(ctx->d_in, q0, nb, cudaMemcpyHostToDevice, ctx->stream));
-    CU(cudaMemcpyAsync(ctx->d_in + P * NF, qd0, nb, cudaMemcpyHostToDevice, ctx->stream));
-    CU(cudaMemcpyAsync(ctx->d_in + 2 * P * NF, qdd0, nb, cudaMemcpyHostToDevice, ctx->stream));
+    CU(cudaMemcpyAsync(d_in, q0, nb, cudaMemcpyHostToDevice, ctx->stream));
+    CU(cudaMemcpyAsync(d_in + P * NF, qd0, nb, cudaMemcpyHostToDevice, ctx->stream));
+    CU(cudaMemcpyAsync(d_in + 2 * P * NF, qdd0, nb, cudaMemcpyHostToDevice, ctx->stream));
     if (nobs > 0)
-        CU(cudaMemcpyAsync(ctx->d_obs, obstacles, size_t(nprob) * nobs * 12 * sizeof(double), cudaMemcpyHostToDevice,
+        CU(cudaMemcpyAsync(ctx->d_obs.get(), obstacles, size_t(nprob) * nobs * 12 * sizeof(double), cudaMemcpyHostToDevice,
                            ctx->stream));
     ctx->B.epoch++;
     int nl = 0;
     bool latency = false;
     { int rc2 = launch_build(ctx, ctx->B, &nl, &latency); if (rc2) return rc2; }
     ctx->launches += nl;
-    CU(launch_hyperplanes(ctx->B, ctx->stream, (latency && nobs > 0) ? ctx->d_unit_flag : nullptr));
+    CU(launch_hyperplanes(ctx->B, ctx->stream, (latency && nobs > 0) ? ctx->d_unit_flag.get() : nullptr));
     ctx->launches += (nobs > 0);
     CU(launch_pack_image(ctx->B, ctx->stream));
     ctx->launches++;
@@ -661,41 +650,42 @@ extern "C" int armour_debug_k1_profile(long long* out, int reset) {
 
 int armour_measure_fp64_peak(armour_ctx* ctx, double* tflops) {
     if (!ctx || !tflops) return ARMOUR_ERR_ARG;
-    CU(cudaSetDevice(ctx->cfg.device));
-    { int rc_c = ensure_constants(ctx); if (rc_c) return rc_c; }
+    { int rc_e = enter(ctx); if (rc_e) return rc_e; }
     int sms = 0;
     CU(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, ctx->cfg.device));
-    double* d_out = nullptr;
-    CU(dalloc(&d_out, 1));
-    cudaEvent_t e0, e1;
-    CU(cudaEventCreate(&e0));
-    CU(cudaEventCreate(&e1));
+    DeviceBuffer<double> d_out;
+    CU(d_out.reserve(1));
+    cudaEvent_t e0 = nullptr, e1 = nullptr;
     const int iters = 4096, grid = sms * 8, block = 256;
     double best = 0.0;
-    for (int rep = 0; rep < 4; rep++) {
-        CU(cudaEventRecord(e0, ctx->stream));
-        k_fp64_peak<<<grid, block, 0, ctx->stream>>>(d_out, iters, 1.0000001);
-        CU(cudaEventRecord(e1, ctx->stream));
-        CU(cudaEventSynchronize(e1));
-        float ms = 0;
-        CU(cudaEventElapsedTime(&ms, e0, e1));
-        const double fl = 2.0 * 8 * double(iters) * double(grid) * block;
-        if (rep > 0) best = std::max(best, fl / (ms * 1e-3) / 1e12);
-    }
-    ctx->launches += 4;
-    cudaEventDestroy(e0);
-    cudaEventDestroy(e1);
-    cudaFree(d_out);
-    *tflops = best;
-    return ARMOUR_OK;
+    auto run = [&]() -> int {
+        CU(cudaEventCreate(&e0));
+        CU(cudaEventCreate(&e1));
+        for (int rep = 0; rep < 4; rep++) {
+            CU(cudaEventRecord(e0, ctx->stream));
+            k_fp64_peak<<<grid, block, 0, ctx->stream>>>(d_out.get(), iters, 1.0000001);
+            CU(cudaEventRecord(e1, ctx->stream));
+            CU(cudaEventSynchronize(e1));
+            float ms = 0;
+            CU(cudaEventElapsedTime(&ms, e0, e1));
+            const double fl = 2.0 * 8 * double(iters) * double(grid) * block;
+            if (rep > 0) best = std::max(best, fl / (ms * 1e-3) / 1e12);
+        }
+        ctx->launches += 4;
+        return ARMOUR_OK;
+    };
+    const int rc = run();
+    if (e0) cudaEventDestroy(e0);
+    if (e1) cudaEventDestroy(e1);
+    if (rc == ARMOUR_OK) *tflops = best;
+    return rc;
 }
 
 // ---- evaluate --------------------------------------------------------------------------------------
 int armour_batch_eval_device(armour_ctx* ctx, int nprob, const double* d_k, double* d_g, double* d_values) {
     if (!ctx || !d_k) return ARMOUR_ERR_ARG;
     if (nprob < 1 || nprob > ctx->built_nprob) return fail(ctx, ARMOUR_ERR_STATE, "evaluate before build");
-    CU(cudaSetDevice(ctx->cfg.device));
-    { int rc_c = ensure_constants(ctx); if (rc_c) return rc_c; }
+    { int rc_e = enter(ctx); if (rc_e) return rc_e; }
     Batch B = ctx->B;
     B.nprob = nprob;
     CU(launch_constraints(B, d_k, d_g, d_values, ctx->stream));
@@ -706,17 +696,16 @@ int armour_batch_eval_device(armour_ctx* ctx, int nprob, const double* d_k, doub
 int armour_batch_eval(armour_ctx* ctx, int nprob, const double* k, double* g, double* values) {
     if (!ctx || !k) return ARMOUR_ERR_ARG;
     if (nprob < 1 || nprob > ctx->built_nprob) return fail(ctx, ARMOUR_ERR_STATE, "evaluate before build");
-    CU(cudaSetDevice(ctx->cfg.device));
-    { int rc_c = ensure_constants(ctx); if (rc_c) return rc_c; }
-    int rc = ensure_eval_buffers(ctx, nprob, g != nullptr, values != nullptr);
-    if (rc) return rc;
+    { int rc_e = enter(ctx); if (rc_e) return rc_e; }
     const size_t m = size_t(ctx->B.m());
-    CU(cudaMemcpyAsync(ctx->d_k, k, size_t(nprob) * NF * sizeof(double), cudaMemcpyHostToDevice, ctx->stream));
-    rc = armour_batch_eval_device(ctx, nprob, ctx->d_k, g ? ctx->d_g : nullptr, values ? ctx->d_jac : nullptr);
+    int rc = ensure_eval_buffers(ctx, nprob * m, g != nullptr, values != nullptr);
     if (rc) return rc;
-    if (g) CU(cudaMemcpyAsync(g, ctx->d_g, nprob * m * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
+    CU(cudaMemcpyAsync(ctx->d_k.get(), k, size_t(nprob) * NF * sizeof(double), cudaMemcpyHostToDevice, ctx->stream));
+    rc = armour_batch_eval_device(ctx, nprob, ctx->d_k.get(), g ? ctx->d_g.get() : nullptr, values ? ctx->d_jac.get() : nullptr);
+    if (rc) return rc;
+    if (g) CU(cudaMemcpyAsync(g, ctx->d_g.get(), nprob * m * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
     if (values)
-        CU(cudaMemcpyAsync(values, ctx->d_jac, nprob * m * NF * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
+        CU(cudaMemcpyAsync(values, ctx->d_jac.get(), nprob * m * NF * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
     CU(cudaStreamSynchronize(ctx->stream));
     return ARMOUR_OK;
 }
@@ -753,13 +742,13 @@ int armour_batch_eval_structured_device(armour_ctx* ctx, int nprob, const double
     if (!ctx || !d_k || !d_values_nnz) return ARMOUR_ERR_ARG;
     if (nprob < 1 || nprob > ctx->built_nprob) return fail(ctx, ARMOUR_ERR_STATE, "evaluate before build");
     CU(cudaSetDevice(ctx->cfg.device));
-    int rc = ensure_eval_buffers(ctx, nprob, false, true);
+    int rc = ensure_eval_buffers(ctx, size_t(nprob) * ctx->B.m(), false, true);
     if (rc) return rc;
-    rc = armour_batch_eval_device(ctx, nprob, d_k, d_g, ctx->d_jac);
+    rc = armour_batch_eval_device(ctx, nprob, d_k, d_g, ctx->d_jac.get());
     if (rc) return rc;
     Batch B = ctx->B;
     B.nprob = nprob;
-    CU(launch_pack_jacobian(B, ctx->d_jac, d_values_nnz, ctx->stream));
+    CU(launch_pack_jacobian(B, ctx->d_jac.get(), d_values_nnz, ctx->stream));
     ctx->launches += 1;
     return ARMOUR_OK;
 }
@@ -768,22 +757,16 @@ int armour_batch_eval_structured(armour_ctx* ctx, int nprob, const double* k, do
     if (!ctx || !k || !values_nnz) return ARMOUR_ERR_ARG;
     if (nprob < 1 || nprob > ctx->built_nprob) return fail(ctx, ARMOUR_ERR_STATE, "evaluate before build");
     CU(cudaSetDevice(ctx->cfg.device));
-    int rc = ensure_eval_buffers(ctx, nprob, g != nullptr, true);
-    if (rc) return rc;
     const size_t m = size_t(ctx->B.m());
-    const size_t nnz = size_t(jac_nnz(ctx->B.T, ctx->B.NJ, ctx->B.O));
-    if (ctx->jnz_capacity < nprob * nnz) {
-        if (ctx->d_jnz) cudaFree(ctx->d_jnz);
-        ctx->d_jnz = nullptr;
-        ctx->jnz_capacity = 0;
-        CU(dalloc(&ctx->d_jnz, nprob * nnz));
-        ctx->jnz_capacity = nprob * nnz;
-    }
-    CU(cudaMemcpyAsync(ctx->d_k, k, size_t(nprob) * NF * sizeof(double), cudaMemcpyHostToDevice, ctx->stream));
-    rc = armour_batch_eval_structured_device(ctx, nprob, ctx->d_k, g ? ctx->d_g : nullptr, ctx->d_jnz);
+    int rc = ensure_eval_buffers(ctx, nprob * m, g != nullptr, true);
     if (rc) return rc;
-    if (g) CU(cudaMemcpyAsync(g, ctx->d_g, nprob * m * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
-    CU(cudaMemcpyAsync(values_nnz, ctx->d_jnz, nprob * nnz * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
+    const size_t nnz = size_t(jac_nnz(ctx->B.T, ctx->B.NJ, ctx->B.O));
+    CU(ctx->d_jnz.reserve(nprob * nnz));
+    CU(cudaMemcpyAsync(ctx->d_k.get(), k, size_t(nprob) * NF * sizeof(double), cudaMemcpyHostToDevice, ctx->stream));
+    rc = armour_batch_eval_structured_device(ctx, nprob, ctx->d_k.get(), g ? ctx->d_g.get() : nullptr, ctx->d_jnz.get());
+    if (rc) return rc;
+    if (g) CU(cudaMemcpyAsync(g, ctx->d_g.get(), nprob * m * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
+    CU(cudaMemcpyAsync(values_nnz, ctx->d_jnz.get(), nprob * nnz * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
     CU(cudaStreamSynchronize(ctx->stream));
     return ARMOUR_OK;
 }
@@ -803,8 +786,7 @@ int armour_eval_g_jac(armour_ctx* ctx, const double* k, double* g, double* value
 int armour_batch_verdict_device(armour_ctx* ctx, int nprob, const double* d_g, int* d_feasible, int* d_first) {
     if (!ctx || !d_g || !d_feasible || !d_first) return ARMOUR_ERR_ARG;
     if (nprob < 1 || nprob > ctx->built_nprob) return fail(ctx, ARMOUR_ERR_STATE, "verdict before build");
-    CU(cudaSetDevice(ctx->cfg.device));
-    { int rc_c = ensure_constants(ctx); if (rc_c) return rc_c; }
+    { int rc_e = enter(ctx); if (rc_e) return rc_e; }
     Batch B = ctx->B;
     B.nprob = nprob;
     CU(launch_verdict(B, d_g, d_feasible, d_first, ctx->stream));
@@ -841,24 +823,10 @@ int run_solver(armour_ctx* ctx, int nprob, const double* d_q_des, const armour_s
     // scratch: state arrays + second g buffer + linearised rows.  Its size depends on nprob AND on m (obstacle count of
     // the current batch): capacity is tracked in elements and the layout below always uses this call's nprob.
     const size_t P = size_t(nprob);
-    const size_t need_d = P * (3 * NF + 4) + P * m + P * SOLVER_ROWCAP * SOLVER_ROWW;
-    const size_t need_i = 8 * P + 1;
-    if (ctx->solver_doubles < need_d) {
-        if (ctx->d_solver) cudaFree(ctx->d_solver);
-        ctx->d_solver = nullptr;
-        ctx->solver_doubles = 0;
-        CU(dalloc(&ctx->d_solver, need_d));
-        ctx->solver_doubles = need_d;
-    }
-    if (ctx->solver_ints < need_i) {
-        if (ctx->d_solver_i) cudaFree(ctx->d_solver_i);
-        ctx->d_solver_i = nullptr;
-        ctx->solver_ints = 0;
-        CU(dalloc(&ctx->d_solver_i, need_i));
-        ctx->solver_ints = need_i;
-    }
+    CU(ctx->d_solver.reserve(P * (3 * NF + 4) + P * m + P * SOLVER_ROWCAP * SOLVER_ROWW));
+    CU(ctx->d_solver_i.reserve(8 * P + 1));
     SolverState S;
-    double* w = ctx->d_solver;
+    double* w = ctx->d_solver.get();
     S.x = w; w += P * NF;
     S.xt = w; w += P * NF;
     S.best = w; w += P * NF;
@@ -868,7 +836,7 @@ int run_solver(armour_ctx* ctx, int nprob, const double* d_q_des, const armour_s
     S.delta = w; w += P;
     double* d_gt = w; w += P * m;
     S.rows = w;
-    S.have_best = ctx->d_solver_i;
+    S.have_best = ctx->d_solver_i.get();
     S.status = S.have_best + P;
     S.iters = S.status + P;
     S.evals = S.iters + P;
@@ -949,21 +917,20 @@ int run_solver(armour_ctx* ctx, int nprob, const double* d_q_des, const armour_s
 using SolveDeviceFn = int (*)(armour_ctx*, int, const double*, const armour_solver_options*, double*, int*, int*, int*);
 int solve_from_host(armour_ctx* ctx, int nprob, const double* q_des, const armour_solver_options* opt, double* k_opt, int* feasible,
                     int* first_violation, int* iterations, SolveDeviceFn solve_device) {
-    CU(cudaSetDevice(ctx->cfg.device));
-    { int rc_c = ensure_constants(ctx); if (rc_c) return rc_c; }
-    if (!ctx->d_solver_io) CU(dalloc(&ctx->d_solver_io, size_t(ctx->cfg.max_problems) * (2 * NF + 2)));
-    const size_t P = size_t(ctx->cfg.max_problems);
-    double* d_q = ctx->d_solver_io;
-    double* d_ko = d_q + P * NF;
-    int* d_i = reinterpret_cast<int*>(d_ko + P * NF);  // feasible, first, iterations: 3 * P ints in 2 * P doubles
-    cudaStream_t st = ctx->stream;
-    CU(cudaMemcpyAsync(d_q, q_des, size_t(nprob) * NF * sizeof(double), cudaMemcpyHostToDevice, st));
-    int rc = solve_device(ctx, nprob, d_q, opt, d_ko, d_i, d_i + P, d_i + 2 * P);
+    { int rc_e = enter(ctx); if (rc_e) return rc_e; }
+    const size_t nk = size_t(nprob) * NF * sizeof(double), ni = size_t(nprob) * sizeof(int);
+    void* d[5];  // q_des, k_opt, feasible, first violation, iterations
+    int rc = stage(ctx, {nk, nk, ni, ni, ni}, d);
     if (rc) return rc;
-    CU(cudaMemcpyAsync(k_opt, d_ko, size_t(nprob) * NF * sizeof(double), cudaMemcpyDeviceToHost, st));
-    CU(cudaMemcpyAsync(feasible, d_i, size_t(nprob) * sizeof(int), cudaMemcpyDeviceToHost, st));
-    if (first_violation) CU(cudaMemcpyAsync(first_violation, d_i + P, size_t(nprob) * sizeof(int), cudaMemcpyDeviceToHost, st));
-    if (iterations) CU(cudaMemcpyAsync(iterations, d_i + 2 * P, size_t(nprob) * sizeof(int), cudaMemcpyDeviceToHost, st));
+    cudaStream_t st = ctx->stream;
+    CU(cudaMemcpyAsync(d[0], q_des, nk, cudaMemcpyHostToDevice, st));
+    rc = solve_device(ctx, nprob, static_cast<double*>(d[0]), opt, static_cast<double*>(d[1]), static_cast<int*>(d[2]),
+                      static_cast<int*>(d[3]), static_cast<int*>(d[4]));
+    if (rc) return rc;
+    CU(cudaMemcpyAsync(k_opt, d[1], nk, cudaMemcpyDeviceToHost, st));
+    CU(cudaMemcpyAsync(feasible, d[2], ni, cudaMemcpyDeviceToHost, st));
+    if (first_violation) CU(cudaMemcpyAsync(first_violation, d[3], ni, cudaMemcpyDeviceToHost, st));
+    if (iterations) CU(cudaMemcpyAsync(iterations, d[4], ni, cudaMemcpyDeviceToHost, st));
     CU(cudaStreamSynchronize(st));
     return ARMOUR_OK;
 }
@@ -980,9 +947,8 @@ int armour_batch_solve_device(armour_ctx* ctx, int nprob, const double* d_q_des,
     armour_solver_options_default(&opt);
     if (opt_in) opt = *opt_in;
     if (opt.max_iter < 1 || !(opt.tol > 0) || opt.qp_sweeps < 1) return fail(ctx, ARMOUR_ERR_ARG, "solver options");
-    CU(cudaSetDevice(ctx->cfg.device));
-    { int rc_c = ensure_constants(ctx); if (rc_c) return rc_c; }
-    int rc = ensure_eval_buffers(ctx, nprob, true, true);
+    { int rc_e = enter(ctx); if (rc_e) return rc_e; }
+    int rc = ensure_eval_buffers(ctx, size_t(nprob) * ctx->B.m(), true, true);
     if (rc) return rc;
     cudaStream_t st = ctx->stream;
     auto eval = [ctx, st](const Batch& Bb, const double* x, double* g, double* jac) {
@@ -995,8 +961,8 @@ int armour_batch_solve_device(armour_ctx* ctx, int nprob, const double* d_q_des,
         CU(launch_verdict(B, g, feasible, first, st));
         return int(ARMOUR_OK);
     };
-    return run_solver(ctx, nprob, d_q_des, opt, ArmourNlp{}, ctx->B.m(), ctx->d_g, ctx->d_jac, eval, 1 + (ctx->B.O > 0), verdict,
-                      d_k_opt, d_feasible, d_first, d_iters);
+    return run_solver(ctx, nprob, d_q_des, opt, ArmourNlp{}, ctx->B.m(), ctx->d_g.get(), ctx->d_jac.get(), eval, 1 + (ctx->B.O > 0),
+                      verdict, d_k_opt, d_feasible, d_first, d_iters);
 }
 
 int armour_batch_solve(armour_ctx* ctx, int nprob, const double* q_des, const armour_solver_options* opt, double* k_opt,
@@ -1021,18 +987,6 @@ void armour_rollout_options_default(armour_rollout_options* opt) {
 
 namespace {
 
-// grow-only device buffer of at least n elements (contents are not kept)
-template <class T>
-int ensure_buffer(armour_ctx* ctx, T** p, size_t* cap, size_t n) {
-    if (*cap >= n) return ARMOUR_OK;
-    if (*p) cudaFree(*p);
-    *p = nullptr;
-    *cap = 0;
-    CU(dalloc(p, n));
-    *cap = n;
-    return ARMOUR_OK;
-}
-
 int check_rollout(armour_ctx* ctx, int nworlds, int nobs, const armour_rollout_options* opt) {
     if (!ctx) return ARMOUR_ERR_ARG;
     if (ctx->armtd) return fail(ctx, ARMOUR_ERR_STATE, "closed-loop episodes run the main planner, not the ARMTD comparison planner");
@@ -1054,13 +1008,10 @@ int check_rollout(armour_ctx* ctx, int nworlds, int nobs, const armour_rollout_o
 // running count to the host and one synchronisation.
 int rollout_run(armour_ctx* ctx, int n, const double* d_start, const double* d_goal, const double* d_obstacles, int nobs,
                 const armour_rollout_options& opt, const armour_rollout_out& out) {
-    CU(cudaSetDevice(ctx->cfg.device));
-    { int rc_c = ensure_constants(ctx); if (rc_c) return rc_c; }
+    { int rc_e = enter(ctx); if (rc_e) return rc_e; }
     const size_t N = size_t(n), S = size_t(opt.audit_samples), no = size_t(nobs) * 12;
-    const size_t need_d = N * (ROLL_STATE + ROLL_PLAN + 1 + 5 * NF + 1) + N * no + N * S * NF;
-    const size_t need_i = 10 * N + 1;
-    { int rc = ensure_buffer(ctx, &ctx->d_roll, &ctx->roll_doubles, need_d); if (rc) return rc; }
-    { int rc = ensure_buffer(ctx, &ctx->d_roll_i, &ctx->roll_ints, need_i); if (rc) return rc; }
+    CU(ctx->d_roll.reserve(N * (ROLL_STATE + ROLL_PLAN + 1 + 5 * NF + 1) + N * no + N * S * NF));
+    CU(ctx->d_roll_i.reserve(10 * N + 1));
     RolloutDev D;
     D.n = n;
     D.R = opt.max_replans;
@@ -1072,7 +1023,7 @@ int rollout_run(armour_ctx* ctx, int n, const double* d_start, const double* d_g
     D.start = d_start;
     D.goal = d_goal;
     D.obstacles = d_obstacles;
-    double* w = ctx->d_roll;
+    double* w = ctx->d_roll.get();
     D.state = w; w += N * ROLL_STATE;
     D.plan = w; w += N * ROLL_PLAN;
     D.minc = w; w += N;
@@ -1084,7 +1035,7 @@ int rollout_run(armour_ctx* ctx, int n, const double* d_start, const double* d_g
     D.dclear = w; w += N;
     D.dobs = w; w += N * no;
     D.samp = w;
-    int* wi = ctx->d_roll_i;
+    int* wi = ctx->d_roll_i.get();
     D.outcome = wi; wi += N;
     D.replans = wi; wi += N;
     D.infeasible = wi; wi += N;
@@ -1157,43 +1108,37 @@ int armour_batch_rollout(armour_ctx* ctx, int nworlds, const double* start, cons
     if (!start || !goal || (nobs > 0 && !obstacles) || !out) return fail(ctx, ARMOUR_ERR_ARG, "null input");
     CU(cudaSetDevice(ctx->cfg.device));
     const size_t N = size_t(nworlds), R = size_t(opt->max_replans);
-    // staging: inputs, then one device array per requested output (8-byte aligned pieces)
+    // inputs, then one device array per requested output
     const size_t sz[13] = {N * NF * 8, N * NF * 8, N * size_t(nobs) * 12 * 8,
                            out->outcome ? N * 4 : 0, out->replans ? N * 4 : 0, out->infeasible ? N * 4 : 0,
                            out->final_state ? N * ROLL_STATE * 8 : 0, out->min_clearance ? N * 8 : 0,
                            out->log_state ? R * N * ROLL_STATE * 8 : 0, out->log_q_des ? R * N * NF * 8 : 0,
                            out->log_k ? R * N * NF * 8 : 0, out->log_int ? R * N * 4 * 4 : 0, out->log_clearance ? R * N * 8 : 0};
-    size_t off[13], total = 0;
-    for (int i = 0; i < 13; i++) {
-        off[i] = total;
-        total += (sz[i] + 255) / 256 * 256;
-    }
-    rc = ensure_buffer(ctx, &ctx->d_stage, &ctx->stage_bytes, total);
+    void* d[13];
+    rc = stage(ctx, sz, d);
     if (rc) return rc;
-    char* base = ctx->d_stage;
-    auto at = [&](int i) -> void* { return sz[i] ? base + off[i] : nullptr; };
     cudaStream_t st = ctx->stream;
-    CU(cudaMemcpyAsync(at(0), start, sz[0], cudaMemcpyHostToDevice, st));
-    CU(cudaMemcpyAsync(at(1), goal, sz[1], cudaMemcpyHostToDevice, st));
-    if (nobs > 0) CU(cudaMemcpyAsync(at(2), obstacles, sz[2], cudaMemcpyHostToDevice, st));
+    CU(cudaMemcpyAsync(d[0], start, sz[0], cudaMemcpyHostToDevice, st));
+    CU(cudaMemcpyAsync(d[1], goal, sz[1], cudaMemcpyHostToDevice, st));
+    if (nobs > 0) CU(cudaMemcpyAsync(d[2], obstacles, sz[2], cudaMemcpyHostToDevice, st));
     armour_rollout_out d_out;
-    d_out.outcome = static_cast<int*>(at(3));
-    d_out.replans = static_cast<int*>(at(4));
-    d_out.infeasible = static_cast<int*>(at(5));
-    d_out.final_state = static_cast<double*>(at(6));
-    d_out.min_clearance = static_cast<double*>(at(7));
-    d_out.log_state = static_cast<double*>(at(8));
-    d_out.log_q_des = static_cast<double*>(at(9));
-    d_out.log_k = static_cast<double*>(at(10));
-    d_out.log_int = static_cast<int*>(at(11));
-    d_out.log_clearance = static_cast<double*>(at(12));
-    rc = rollout_run(ctx, nworlds, static_cast<const double*>(at(0)), static_cast<const double*>(at(1)),
-                     nobs > 0 ? static_cast<const double*>(at(2)) : nullptr, nobs, *opt, d_out);
+    d_out.outcome = static_cast<int*>(d[3]);
+    d_out.replans = static_cast<int*>(d[4]);
+    d_out.infeasible = static_cast<int*>(d[5]);
+    d_out.final_state = static_cast<double*>(d[6]);
+    d_out.min_clearance = static_cast<double*>(d[7]);
+    d_out.log_state = static_cast<double*>(d[8]);
+    d_out.log_q_des = static_cast<double*>(d[9]);
+    d_out.log_k = static_cast<double*>(d[10]);
+    d_out.log_int = static_cast<int*>(d[11]);
+    d_out.log_clearance = static_cast<double*>(d[12]);
+    rc = rollout_run(ctx, nworlds, static_cast<double*>(d[0]), static_cast<double*>(d[1]), static_cast<double*>(d[2]), nobs, *opt,
+                     d_out);
     if (rc) return rc;
     void* host[13] = {nullptr, nullptr, nullptr, out->outcome, out->replans, out->infeasible, out->final_state, out->min_clearance,
                       out->log_state, out->log_q_des, out->log_k, out->log_int, out->log_clearance};
     for (int i = 3; i < 13; i++)
-        if (sz[i]) CU(cudaMemcpyAsync(host[i], at(i), sz[i], cudaMemcpyDeviceToHost, st));
+        if (sz[i]) CU(cudaMemcpyAsync(host[i], d[i], sz[i], cudaMemcpyDeviceToHost, st));
     CU(cudaStreamSynchronize(st));
     return ARMOUR_OK;
 }
@@ -1203,8 +1148,7 @@ int armour_batch_clearance_device(armour_ctx* ctx, int nconf, const double* d_q,
     int rc = check_clearance(ctx, nconf, nobs);
     if (rc) return rc;
     if (!d_q || !d_clearance || (nobs > 0 && !d_obstacles)) return fail(ctx, ARMOUR_ERR_ARG, "null input");
-    CU(cudaSetDevice(ctx->cfg.device));
-    { int rc_c = ensure_constants(ctx); if (rc_c) return rc_c; }
+    { int rc_e = enter(ctx); if (rc_e) return rc_e; }
     k_clearance<<<nconf, CLEAR_THREADS, 0, ctx->stream>>>(d_q, 1, d_world, d_obstacles, nobs, d_clearance, d_which);
     CU(cudaGetLastError());
     ctx->launches += 1;
@@ -1225,22 +1169,18 @@ int armour_batch_clearance(armour_ctx* ctx, int nconf, const double* q, const in
     CU(cudaSetDevice(ctx->cfg.device));
     const size_t nq = size_t(nconf) * NF * 8, nw = world ? size_t(nconf) * 4 : 0, nb = size_t(nsets) * nobs * 12 * 8,
                  nc = size_t(nconf) * 8, nh = which ? size_t(nconf) * 4 : 0;
-    const size_t oq = 0, ow = oq + (nq + 255) / 256 * 256, ob = ow + (nw + 255) / 256 * 256, oc = ob + (nb + 255) / 256 * 256,
-                 oh = oc + (nc + 255) / 256 * 256;
-    rc = ensure_buffer(ctx, &ctx->d_stage, &ctx->stage_bytes, oh + nh);
+    void* d[5];  // q, world, obstacles, clearance, which
+    rc = stage(ctx, {nq, nw, nb, nc, nh}, d);
     if (rc) return rc;
-    char* base = ctx->d_stage;
     cudaStream_t st = ctx->stream;
-    CU(cudaMemcpyAsync(base + oq, q, nq, cudaMemcpyHostToDevice, st));
-    if (world) CU(cudaMemcpyAsync(base + ow, world, nw, cudaMemcpyHostToDevice, st));
-    if (nobs > 0) CU(cudaMemcpyAsync(base + ob, obstacles, nb, cudaMemcpyHostToDevice, st));
-    rc = armour_batch_clearance_device(ctx, nconf, reinterpret_cast<const double*>(base + oq),
-                                       world ? reinterpret_cast<const int*>(base + ow) : nullptr,
-                                       nobs > 0 ? reinterpret_cast<const double*>(base + ob) : nullptr, nobs,
-                                       reinterpret_cast<double*>(base + oc), which ? reinterpret_cast<int*>(base + oh) : nullptr);
+    CU(cudaMemcpyAsync(d[0], q, nq, cudaMemcpyHostToDevice, st));
+    if (world) CU(cudaMemcpyAsync(d[1], world, nw, cudaMemcpyHostToDevice, st));
+    if (nobs > 0) CU(cudaMemcpyAsync(d[2], obstacles, nb, cudaMemcpyHostToDevice, st));
+    rc = armour_batch_clearance_device(ctx, nconf, static_cast<double*>(d[0]), static_cast<int*>(d[1]), static_cast<double*>(d[2]), nobs,
+                                       static_cast<double*>(d[3]), static_cast<int*>(d[4]));
     if (rc) return rc;
-    CU(cudaMemcpyAsync(clearance, base + oc, nc, cudaMemcpyDeviceToHost, st));
-    if (which) CU(cudaMemcpyAsync(which, base + oh, nh, cudaMemcpyDeviceToHost, st));
+    CU(cudaMemcpyAsync(clearance, d[3], nc, cudaMemcpyDeviceToHost, st));
+    if (which) CU(cudaMemcpyAsync(which, d[4], nh, cudaMemcpyDeviceToHost, st));
     CU(cudaStreamSynchronize(st));
     return ARMOUR_OK;
 }
@@ -1418,11 +1358,12 @@ int armour_import_reachsets(armour_ctx* ctx, int prob, int nprob_total, const ar
     if (!in || !in->u_radius || !in->torque_radius || !in->link_gens || !q0 || !qd0 || !qdd0 || prob < 0 ||
         prob >= nprob_total)
         return ARMOUR_ERR_ARG;
-    CU(cudaSetDevice(ctx->cfg.device));
-    { int rc_c = ensure_constants(ctx); if (rc_c) return rc_c; }
+    { int rc_e = enter(ctx); if (rc_e) return rc_e; }
     if (prob == 0 || ctx->B.O != nobs || ctx->B.nprob != nprob_total) {
         rc = ensure_obstacle_buffers(ctx, nprob_total, nobs);
         if (rc) return rc;
+        ctx->B.O = nobs;
+        ctx->B.nprob = nprob_total;
     }
     if (prob == 0) ctx->B.epoch++;  // imported tables: no build failure can be pending
     const Batch& B = ctx->B;
@@ -1460,10 +1401,10 @@ int armour_import_reachsets(armour_ctx* ctx, int prob, int nprob_total, const ar
         for (int e = 0; e < 3; e++) lr[i * 3 + e] = in->link_gens[i * 18 + e + (3 + e) * 3];
     H2D(B.link_r + prob * T * NJ * 3, lr.data(), lr.size() * sizeof(double));
     H2D(B.u_r + prob * T * NF, in->u_radius, T * NF * sizeof(double));
-    H2D(ctx->d_in + prob * NF, q0, NF * sizeof(double));
-    H2D(ctx->d_in + P * NF + prob * NF, qd0, NF * sizeof(double));
-    H2D(ctx->d_in + 2 * P * NF + prob * NF, qdd0, NF * sizeof(double));
-    if (nobs > 0) H2D(ctx->d_obs + size_t(prob) * nobs * 12, obstacles, size_t(nobs) * 12 * sizeof(double));
+    H2D(ctx->d_in.get() + prob * NF, q0, NF * sizeof(double));
+    H2D(ctx->d_in.get() + P * NF + prob * NF, qd0, NF * sizeof(double));
+    H2D(ctx->d_in.get() + 2 * P * NF + prob * NF, qdd0, NF * sizeof(double));
+    if (nobs > 0) H2D(ctx->d_obs.get() + size_t(prob) * nobs * 12, obstacles, size_t(nobs) * 12 * sizeof(double));
 #undef H2D
     CU(cudaStreamSynchronize(st));  // the staging vectors die at return
     if (prob == nprob_total - 1) {
@@ -1506,19 +1447,19 @@ int armtd_ctx_create(const armour_config* cfg_in, bool batch, armour_ctx** out) 
     int rc = armour_ctx_create(&cfg, &ctx);
     if (rc) return rc;
     const size_t P = size_t(ctx->cfg.max_problems);
-    if (dalloc(&ctx->d_jrs, P * ARMTD_T_PADDED * NF * 6) != cudaSuccess ||
-        dalloc(&ctx->d_armtd_in, P * NF * 4 + P * 6 * NF * ARMTD_T) != cudaSuccess ||
-        cudaMemsetAsync(ctx->d_armtd_in, 0, P * NF * 2 * sizeof(double), ctx->stream) != cudaSuccess ||
+    if (ctx->d_jrs.reserve(P * ARMTD_T_PADDED * NF * 6) != cudaSuccess ||
+        ctx->d_armtd_in.reserve(P * NF * 4 + P * 6 * NF * ARMTD_T) != cudaSuccess ||
+        cudaMemsetAsync(ctx->d_armtd_in.get(), 0, P * NF * 2 * sizeof(double), ctx->stream) != cudaSuccess ||
         cudaStreamSynchronize(ctx->stream) != cudaSuccess) {
         armour_ctx_destroy(ctx);
         return ARMOUR_ERR_NOMEM;
     }
-    ctx->d_krange = ctx->d_armtd_in;
+    ctx->d_krange = ctx->d_armtd_in.get();
     ctx->d_zero = ctx->d_krange + P * NF;
     ctx->d_cs = ctx->d_zero + P * NF;
     ctx->d_jrs_raw = ctx->d_cs + P * NF * 2;
     ctx->armtd = true;
-    ctx->B.jrs_ext = ctx->d_jrs;
+    ctx->B.jrs_ext = ctx->d_jrs.get();
     *out = ctx;
     return ARMOUR_OK;
 }
@@ -1538,20 +1479,8 @@ int check_armtd_built(armour_ctx* ctx, int nprob, const char* what) {
 
 int ensure_armtd_buffers(armour_ctx* ctx, int nprob, bool need_jac) {
     const size_t ma = size_t(nprob) * armtd_m(ctx->B.NJ, ctx->B.O);
-    if (ctx->ga_capacity < ma) {
-        if (ctx->d_ga) cudaFree(ctx->d_ga);
-        ctx->d_ga = nullptr;
-        ctx->ga_capacity = 0;
-        CU(dalloc(&ctx->d_ga, ma));
-        ctx->ga_capacity = ma;
-    }
-    if (need_jac && ctx->ja_capacity < ma * NF) {
-        if (ctx->d_ja) cudaFree(ctx->d_ja);
-        ctx->d_ja = nullptr;
-        ctx->ja_capacity = 0;
-        CU(dalloc(&ctx->d_ja, ma * NF));
-        ctx->ja_capacity = ma * NF;
-    }
+    CU(ctx->d_ga.reserve(ma));
+    if (need_jac) CU(ctx->d_ja.reserve(ma * NF));
     return ARMOUR_OK;
 }
 
@@ -1559,8 +1488,8 @@ int ensure_armtd_buffers(armour_ctx* ctx, int nprob, bool need_jac) {
 // the caller), then k_armtd_assemble (d_g / d_jac may be nullptr; with d_jac == nullptr no Jacobian is computed).  Launches
 // 2 + (O > 0) kernels.
 int armtd_eval_launch(armour_ctx* ctx, const Batch& Bb, const double* d_k, double* d_g, double* d_jac) {
-    CU(launch_constraints(Bb, d_k, ctx->d_g, d_jac ? ctx->d_jac : nullptr, ctx->stream));
-    CU(launch_armtd_assemble(Bb, ctx->d_krange, d_k, ctx->d_g, ctx->d_jac, d_g, d_jac, ctx->stream));
+    CU(launch_constraints(Bb, d_k, ctx->d_g.get(), d_jac ? ctx->d_jac.get() : nullptr, ctx->stream));
+    CU(launch_armtd_assemble(Bb, ctx->d_krange, d_k, ctx->d_g.get(), ctx->d_jac.get(), d_g, d_jac, ctx->stream));
     return ARMOUR_OK;
 }
 
@@ -1572,8 +1501,8 @@ int fetch_armtd_inputs(armour_ctx* ctx) {
     ctx->h_qd0.resize(n);
     ctx->h_qdd0.assign(n, 0.0);
     ctx->h_krange.resize(n);
-    CU(cudaMemcpyAsync(ctx->h_q0.data(), ctx->d_in, n * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
-    CU(cudaMemcpyAsync(ctx->h_qd0.data(), ctx->d_in + P * NF, n * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
+    CU(cudaMemcpyAsync(ctx->h_q0.data(), ctx->d_in.get(), n * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
+    CU(cudaMemcpyAsync(ctx->h_qd0.data(), ctx->d_in.get() + P * NF, n * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
     CU(cudaMemcpyAsync(ctx->h_krange.data(), ctx->d_krange, n * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
     CU(cudaStreamSynchronize(ctx->stream));
     return ARMOUR_OK;
@@ -1596,10 +1525,9 @@ int armour_armtd_batch_build_device(armour_ctx* ctx, int nprob, const double* d_
     int rc = check_armtd_batch(ctx, nprob, nobs);
     if (rc) return rc;
     if (!d_q0 || !d_qd0 || !d_jrs || !d_k_range || (nobs > 0 && !d_obstacles)) return fail(ctx, ARMOUR_ERR_ARG, "null input");
-    CU(cudaSetDevice(ctx->cfg.device));
-    { int rc_c = ensure_constants(ctx); if (rc_c) return rc_c; }
+    { int rc_e = enter(ctx); if (rc_e) return rc_e; }
     const int n = nprob * ARMTD_T_PADDED * NF;
-    k_armtd_jrs<<<(n + 255) / 256, 256, 0, ctx->stream>>>(nprob, d_q0, d_sincos, d_jrs, ctx->d_jrs);
+    k_armtd_jrs<<<(n + 255) / 256, 256, 0, ctx->stream>>>(nprob, d_q0, d_sincos, d_jrs, ctx->d_jrs.get());
     CU(cudaGetLastError());
     ctx->launches++;
     CU(cudaMemcpyAsync(ctx->d_krange, d_k_range, size_t(nprob) * NF * sizeof(double), cudaMemcpyDeviceToDevice, ctx->stream));
@@ -1612,8 +1540,7 @@ int armour_armtd_batch_build(armour_ctx* ctx, int nprob, const double* q0, const
     int rc = check_armtd_batch(ctx, nprob, nobs);
     if (rc) return rc;
     if (!q0 || !qd0 || !jrs || !k_range || (nobs > 0 && !obstacles)) return fail(ctx, ARMOUR_ERR_ARG, "null input");
-    CU(cudaSetDevice(ctx->cfg.device));
-    { int rc_c = ensure_constants(ctx); if (rc_c) return rc_c; }
+    { int rc_e = enter(ctx); if (rc_e) return rc_e; }
     // cos q0 / sin q0 with the host's libm, as the reference's ConstantAccelerationCurve constructor (KPA/Trajectory.cu:29-62)
     const size_t n = size_t(nprob) * NF;
     std::vector<double> cs(2 * n);
@@ -1626,7 +1553,7 @@ int armour_armtd_batch_build(armour_ctx* ctx, int nprob, const double* q0, const
     CU(cudaMemcpyAsync(ctx->d_jrs_raw, jrs, n * 6 * ARMTD_T * sizeof(double), cudaMemcpyHostToDevice, st));
     CU(cudaMemcpyAsync(ctx->d_krange, k_range, n * sizeof(double), cudaMemcpyHostToDevice, st));
     const int nt = nprob * ARMTD_T_PADDED * NF;
-    k_armtd_jrs<<<(nt + 255) / 256, 256, 0, st>>>(nprob, nullptr, ctx->d_cs, ctx->d_jrs_raw, ctx->d_jrs);
+    k_armtd_jrs<<<(nt + 255) / 256, 256, 0, st>>>(nprob, nullptr, ctx->d_cs, ctx->d_jrs_raw, ctx->d_jrs.get());
     CU(cudaGetLastError());
     ctx->launches++;
     ctx->h_krange.assign(k_range, k_range + n);
@@ -1646,9 +1573,8 @@ int armour_armtd_batch_eval_device(armour_ctx* ctx, int nprob, const double* d_k
     if (!ctx || !d_k || (!d_g && !d_values)) return ARMOUR_ERR_ARG;
     int rc = check_armtd_built(ctx, nprob, "evaluate");
     if (rc) return rc;
-    CU(cudaSetDevice(ctx->cfg.device));
-    { int rc_c = ensure_constants(ctx); if (rc_c) return rc_c; }
-    rc = ensure_eval_buffers(ctx, nprob, true, d_values != nullptr);
+    { int rc_e = enter(ctx); if (rc_e) return rc_e; }
+    rc = ensure_eval_buffers(ctx, size_t(nprob) * ctx->B.m(), true, d_values != nullptr);
     if (rc) return rc;
     Batch B = ctx->B;
     B.nprob = nprob;
@@ -1666,11 +1592,11 @@ int armour_armtd_batch_eval(armour_ctx* ctx, int nprob, const double* k, double*
     if (rc) return rc;
     const size_t ma = size_t(nprob) * armtd_m(ctx->B.NJ, ctx->B.O);
     cudaStream_t st = ctx->stream;
-    CU(cudaMemcpyAsync(ctx->d_k, k, size_t(nprob) * NF * sizeof(double), cudaMemcpyHostToDevice, st));
-    rc = armour_armtd_batch_eval_device(ctx, nprob, ctx->d_k, g ? ctx->d_ga : nullptr, values ? ctx->d_ja : nullptr);
+    CU(cudaMemcpyAsync(ctx->d_k.get(), k, size_t(nprob) * NF * sizeof(double), cudaMemcpyHostToDevice, st));
+    rc = armour_armtd_batch_eval_device(ctx, nprob, ctx->d_k.get(), g ? ctx->d_ga.get() : nullptr, values ? ctx->d_ja.get() : nullptr);
     if (rc) return rc;
-    if (g) CU(cudaMemcpyAsync(g, ctx->d_ga, ma * sizeof(double), cudaMemcpyDeviceToHost, st));
-    if (values) CU(cudaMemcpyAsync(values, ctx->d_ja, ma * NF * sizeof(double), cudaMemcpyDeviceToHost, st));
+    if (g) CU(cudaMemcpyAsync(g, ctx->d_ga.get(), ma * sizeof(double), cudaMemcpyDeviceToHost, st));
+    if (values) CU(cudaMemcpyAsync(values, ctx->d_ja.get(), ma * NF * sizeof(double), cudaMemcpyDeviceToHost, st));
     CU(cudaStreamSynchronize(st));
     return ARMOUR_OK;
 }
@@ -1704,8 +1630,7 @@ int armour_armtd_batch_verdict_device(armour_ctx* ctx, int nprob, const double* 
     if (!ctx || !d_g || !d_feasible || !d_first) return ARMOUR_ERR_ARG;
     int rc = check_armtd_built(ctx, nprob, "verdict");
     if (rc) return rc;
-    CU(cudaSetDevice(ctx->cfg.device));
-    { int rc_c = ensure_constants(ctx); if (rc_c) return rc_c; }
+    { int rc_e = enter(ctx); if (rc_e) return rc_e; }
     k_armtd_verdict<<<nprob, 256, 0, ctx->stream>>>(ctx->B.NJ, ctx->B.O, d_g, d_feasible, d_first);
     CU(cudaGetLastError());
     ctx->launches++;
@@ -1718,11 +1643,11 @@ int armour_armtd_verdict(armour_ctx* ctx, const double* g, int* feasible, int* f
     int rc = ensure_armtd_buffers(ctx, 1, false);
     if (rc) return rc;
     cudaStream_t st = ctx->stream;
-    CU(cudaMemcpyAsync(ctx->d_ga, g, size_t(armtd_m(ctx->B.NJ, ctx->B.O)) * sizeof(double), cudaMemcpyHostToDevice, st));
-    rc = armour_armtd_batch_verdict_device(ctx, 1, ctx->d_ga, ctx->d_verdict, ctx->d_verdict + 1);
+    CU(cudaMemcpyAsync(ctx->d_ga.get(), g, size_t(armtd_m(ctx->B.NJ, ctx->B.O)) * sizeof(double), cudaMemcpyHostToDevice, st));
+    rc = armour_armtd_batch_verdict_device(ctx, 1, ctx->d_ga.get(), ctx->d_verdict.get(), ctx->d_verdict.get() + 1);
     if (rc) return rc;
     int v[2];
-    CU(cudaMemcpyAsync(v, ctx->d_verdict, sizeof(v), cudaMemcpyDeviceToHost, st));
+    CU(cudaMemcpyAsync(v, ctx->d_verdict.get(), sizeof(v), cudaMemcpyDeviceToHost, st));
     CU(cudaStreamSynchronize(st));
     *feasible = v[0];
     if (first_violation) *first_violation = v[1];
@@ -1756,9 +1681,8 @@ int armour_armtd_batch_solve_device(armour_ctx* ctx, int nprob, const double* d_
     opt.tol = 1e-7;  // IPOPT_OPTIMIZATION_TOLERANCE of KPA (KPA/Parameters.h:43), as armtd_main sets it
     if (opt_in) opt = *opt_in;
     if (opt.max_iter < 1 || !(opt.tol > 0) || opt.qp_sweeps < 1) return fail(ctx, ARMOUR_ERR_ARG, "solver options");
-    CU(cudaSetDevice(ctx->cfg.device));
-    { int rc_c = ensure_constants(ctx); if (rc_c) return rc_c; }
-    rc = ensure_eval_buffers(ctx, nprob, true, true);
+    { int rc_e = enter(ctx); if (rc_e) return rc_e; }
+    rc = ensure_eval_buffers(ctx, size_t(nprob) * ctx->B.m(), true, true);
     if (rc) return rc;
     rc = ensure_armtd_buffers(ctx, nprob, true);
     if (rc) return rc;
@@ -1768,8 +1692,8 @@ int armour_armtd_batch_solve_device(armour_ctx* ctx, int nprob, const double* d_
         CU(cudaGetLastError());
         return int(ARMOUR_OK);
     };
-    return run_solver(ctx, nprob, d_q_des, opt, ArmtdNlp{ctx->d_krange}, armtd_m(ctx->B.NJ, ctx->B.O), ctx->d_ga, ctx->d_ja, eval,
-                      2 + (ctx->B.O > 0), verdict, d_k_opt, d_feasible, d_first, d_iters);
+    return run_solver(ctx, nprob, d_q_des, opt, ArmtdNlp{ctx->d_krange}, armtd_m(ctx->B.NJ, ctx->B.O), ctx->d_ga.get(),
+                      ctx->d_ja.get(), eval, 2 + (ctx->B.O > 0), verdict, d_k_opt, d_feasible, d_first, d_iters);
 }
 
 int armour_armtd_batch_solve(armour_ctx* ctx, int nprob, const double* q_des, const armour_solver_options* opt, double* k_opt,

@@ -18,17 +18,18 @@
 
 #include "../../include/armour_b200.h"
 #include "controller.cuh"
+#include "device_buffer.h"
 
+using armour::DeviceBuffer;
 using namespace armour::ctl;
 
 struct armour_controller {
     int device = 0;
-    Model host;               // the model as uploaded (derived blocks filled on the device)
-    Model* d_model = nullptr;
+    Model host;                 // the model as uploaded (derived blocks filled on the device)
+    DeviceBuffer<Model> d_model;
     cudaStream_t stream = nullptr;
     bool own_stream = true;
-    double* d_buf = nullptr;  // staging of the host-pointer entry points
-    size_t buf_doubles = 0;
+    DeviceBuffer<double> d_buf;  // staging of the host-pointer entry points
     std::vector<double> h_trig;
     std::string last_error;
     long long launches = 0;
@@ -298,15 +299,6 @@ void convert_model(const FileModel& F, double eps, Model& M) {
     }
 }
 
-int ensure_buf(armour_controller* ctl, size_t doubles) {
-    if (ctl->buf_doubles >= doubles) return ARMOUR_OK;
-    if (ctl->d_buf) cudaFree(ctl->d_buf);
-    ctl->d_buf = nullptr;
-    ctl->buf_doubles = 0;
-    CCU(cudaMalloc(&ctl->d_buf, doubles * sizeof(double)));
-    ctl->buf_doubles = doubles;
-    return ARMOUR_OK;
-}
 // sin(-q), cos(-q) with the host's libm, as the reference computes them (spatial_interval.cpp:150-151 with theta = -q);
 // large batches are split over the host's threads (each value depends on its own angle only)
 void host_trig(const double* q, size_t count, std::vector<double>& out) {
@@ -356,7 +348,6 @@ int armour_controller_create(const char* model_file, double model_uncertainty, i
     convert_model(F, model_uncertainty, c->host);
     auto bail = [&](cudaError_t e, const char* what) {
         const std::string msg = std::string(what) + ": " + cudaGetErrorString(e);
-        if (c->d_model) cudaFree(c->d_model);
         if (c->stream) cudaStreamDestroy(c->stream);
         delete c;
         return cfail(nullptr, ARMOUR_ERR_CUDA, msg);
@@ -364,11 +355,11 @@ int armour_controller_create(const char* model_file, double model_uncertainty, i
     cudaError_t e;
     if ((e = cudaSetDevice(device)) != cudaSuccess) return bail(e, "cudaSetDevice");
     if ((e = cudaStreamCreateWithFlags(&c->stream, cudaStreamNonBlocking)) != cudaSuccess) return bail(e, "cudaStreamCreate");
-    if ((e = cudaMalloc(&c->d_model, sizeof(Model))) != cudaSuccess) return bail(e, "cudaMalloc(model)");
-    if ((e = cudaMemcpyAsync(c->d_model, &c->host, sizeof(Model), cudaMemcpyHostToDevice, c->stream)) != cudaSuccess) return bail(e, "upload");
-    k_model_setup<<<1, 32, 0, c->stream>>>(c->d_model);
+    if ((e = c->d_model.reserve(1)) != cudaSuccess) return bail(e, "cudaMalloc(model)");
+    if ((e = cudaMemcpyAsync(c->d_model.get(), &c->host, sizeof(Model), cudaMemcpyHostToDevice, c->stream)) != cudaSuccess) return bail(e, "upload");
+    k_model_setup<<<1, 32, 0, c->stream>>>(c->d_model.get());
     if ((e = cudaGetLastError()) != cudaSuccess) return bail(e, "k_model_setup");
-    if ((e = cudaMemcpyAsync(&c->host, c->d_model, sizeof(Model), cudaMemcpyDeviceToHost, c->stream)) != cudaSuccess) return bail(e, "download");
+    if ((e = cudaMemcpyAsync(&c->host, c->d_model.get(), sizeof(Model), cudaMemcpyDeviceToHost, c->stream)) != cudaSuccess) return bail(e, "download");
     if ((e = cudaStreamSynchronize(c->stream)) != cudaSuccess) return bail(e, "k_model_setup");
     c->launches = 1;
     (void)ctl;
@@ -379,10 +370,8 @@ int armour_controller_create(const char* model_file, double model_uncertainty, i
 void armour_controller_destroy(armour_controller* ctl) {
     if (!ctl) return;
     cudaSetDevice(ctl->device);
-    if (ctl->d_buf) cudaFree(ctl->d_buf);
-    if (ctl->d_model) cudaFree(ctl->d_model);
     if (ctl->stream && ctl->own_stream) cudaStreamDestroy(ctl->stream);
-    delete ctl;
+    delete ctl;  // frees the buffers
 }
 
 int armour_controller_num_joints(const armour_controller* ctl) { return ctl ? ctl->host.nj : ARMOUR_ERR_ARG; }
@@ -434,7 +423,7 @@ int armour_controller_rnea_device(armour_controller* ctl, int n, const double* d
     if ((d_tau_lo == nullptr) != (d_tau_hi == nullptr)) return cfail(ctl, ARMOUR_ERR_ARG, "tau_lo and tau_hi go together");
     CCU(cudaSetDevice(ctl->device));
     TrigSrc trig{d_sincos};
-    k_rnea<<<grid(n), CTL_THREADS, 0, ctl->stream>>>(ctl->d_model, n, d_q, d_qd, d_qda, d_qdd, trig, apply_friction, apply_gravity,
+    k_rnea<<<grid(n), CTL_THREADS, 0, ctl->stream>>>(ctl->d_model.get(), n, d_q, d_qd, d_qda, d_qdd, trig, apply_friction, apply_gravity,
                                                       d_tau, d_tau_lo, d_tau_hi);
     CCU(cudaGetLastError());
     ctl->launches++;
@@ -447,9 +436,8 @@ int armour_controller_rnea(armour_controller* ctl, int n, const double* q, const
     if (n < 1) return cfail(ctl, ARMOUR_ERR_ARG, "n must be positive");
     CCU(cudaSetDevice(ctl->device));
     const size_t N = size_t(n) * ctl->host.nj;
-    int rc = ensure_buf(ctl, N * 9);
-    if (rc) return rc;
-    double* d = ctl->d_buf;  // q qd qda qdd | sincos (2N) | tau lo hi
+    CCU(ctl->d_buf.reserve(N * 9));
+    double* d = ctl->d_buf.get();  // q qd qda qdd | sincos (2N) | tau lo hi
     host_trig(q, N, ctl->h_trig);
     cudaStream_t st = ctl->stream;
     CCU(cudaMemcpyAsync(d, q, N * sizeof(double), cudaMemcpyHostToDevice, st));
@@ -458,8 +446,8 @@ int armour_controller_rnea(armour_controller* ctl, int n, const double* q, const
     CCU(cudaMemcpyAsync(d + 3 * N, qdd, N * sizeof(double), cudaMemcpyHostToDevice, st));
     CCU(cudaMemcpyAsync(d + 4 * N, ctl->h_trig.data(), 2 * N * sizeof(double), cudaMemcpyHostToDevice, st));
     const bool want_iv = tau_lo && tau_hi;
-    rc = armour_controller_rnea_device(ctl, n, d, d + N, d + 2 * N, d + 3 * N, d + 4 * N, apply_friction, apply_gravity,
-                                       tau ? d + 6 * N : nullptr, want_iv ? d + 7 * N : nullptr, want_iv ? d + 8 * N : nullptr);
+    int rc = armour_controller_rnea_device(ctl, n, d, d + N, d + 2 * N, d + 3 * N, d + 4 * N, apply_friction, apply_gravity,
+                                           tau ? d + 6 * N : nullptr, want_iv ? d + 7 * N : nullptr, want_iv ? d + 8 * N : nullptr);
     if (rc) return rc;
     if (tau) CCU(cudaMemcpyAsync(tau, d + 6 * N, N * sizeof(double), cudaMemcpyDeviceToHost, st));
     if (want_iv) {
@@ -490,7 +478,7 @@ int armour_controller_update_device(armour_controller* ctl, int n, const armour_
     if (rc) return rc;
     CCU(cudaSetDevice(ctl->device));
     TrigSrc trig{d_sincos};
-    k_controller_update<<<grid(n), CTL_THREADS, 0, ctl->stream>>>(ctl->d_model, n, G, d_q, d_qd, d_q_des, d_qd_des, d_qdd_des, trig, d_u,
+    k_controller_update<<<grid(n), CTL_THREADS, 0, ctl->stream>>>(ctl->d_model.get(), n, G, d_q, d_qd, d_q_des, d_qd_des, d_qdd_des, trig, d_u,
                                                                    d_u_nominal, d_v, d_status);
     CCU(cudaGetLastError());
     ctl->launches++;
@@ -504,17 +492,16 @@ int armour_controller_update(armour_controller* ctl, int n, const armour_control
     if (n < 1) return cfail(ctl, ARMOUR_ERR_ARG, "n must be positive");
     CCU(cudaSetDevice(ctl->device));
     const size_t N = size_t(n) * ctl->host.nj;
-    int rc = ensure_buf(ctl, N * 10 + size_t(n));
-    if (rc) return rc;
-    double* d = ctl->d_buf;  // q qd q_des qd_des qdd_des | sincos (2N) | u u_nominal v | status (ints in n doubles)
+    CCU(ctl->d_buf.reserve(N * 10 + size_t(n)));
+    double* d = ctl->d_buf.get();  // q qd q_des qd_des qdd_des | sincos (2N) | u u_nominal v | status (ints in n doubles)
     host_trig(q, N, ctl->h_trig);
     cudaStream_t st = ctl->stream;
     const double* src[5] = {q, qd, q_des, qd_des, qdd_des};
     for (int k = 0; k < 5; k++) CCU(cudaMemcpyAsync(d + k * N, src[k], N * sizeof(double), cudaMemcpyHostToDevice, st));
     CCU(cudaMemcpyAsync(d + 5 * N, ctl->h_trig.data(), 2 * N * sizeof(double), cudaMemcpyHostToDevice, st));
     int* d_status = reinterpret_cast<int*>(d + 10 * N);
-    rc = armour_controller_update_device(ctl, n, gains, d, d + N, d + 2 * N, d + 3 * N, d + 4 * N, d + 5 * N, d + 7 * N, d + 8 * N,
-                                         d + 9 * N, d_status);
+    int rc = armour_controller_update_device(ctl, n, gains, d, d + N, d + 2 * N, d + 3 * N, d + 4 * N, d + 5 * N, d + 7 * N,
+                                             d + 8 * N, d + 9 * N, d_status);
     if (rc) return rc;
     CCU(cudaMemcpyAsync(u, d + 7 * N, N * sizeof(double), cudaMemcpyDeviceToHost, st));
     if (u_nominal) CCU(cudaMemcpyAsync(u_nominal, d + 8 * N, N * sizeof(double), cudaMemcpyDeviceToHost, st));
