@@ -8,39 +8,11 @@ import numpy as np
 import pytest
 
 from conftest import WORLDS
+from halfspace_ref import chunk_candidates, chunk_rows, half_spaces, row_generators
 
 pytestmark = pytest.mark.gpu
 NF = 7
 K_TEST = np.array([0.5, 0.6, 0.7, 0.0, -0.5, -0.6, -0.7])
-
-
-PAIRS = [(a, b) for a in range(8) for b in range(a + 1, 9)]  # generator pairs in the reference's scan order
-
-
-def _half_spaces(G, oc):
-    """All 72 signed half-spaces (s*C, b) of rows with generators G [rows, 9, 3] and obstacle centres oc [rows, 3], in scan
-    order pos_0, neg_0, pos_1, ..., computed with the expressions of k_hyperplanes (no contraction): [rows, 72, 4] and the
-    mask of non-degenerate normals [rows, 72]."""
-    rows = G.shape[0]
-    out = np.zeros((rows, 72, 4))
-    nzs = np.zeros((rows, 72), bool)
-    for i, (a, b) in enumerate(PAIRS):
-        ga, gb = G[:, a], G[:, b]
-        cx = ga[:, 1] * gb[:, 2] - ga[:, 2] * gb[:, 1]
-        cy = ga[:, 2] * gb[:, 0] - ga[:, 0] * gb[:, 2]
-        cz = ga[:, 0] * gb[:, 1] - ga[:, 1] * gb[:, 0]
-        nrm = np.sqrt(cx * cx + cy * cy + cz * cz)
-        safe = np.where(nrm > 0, nrm, 1.0)
-        C0, C1, C2 = (np.where(nrm > 0, c / safe, 0.0) for c in (cx, cy, cz))
-        d = C0 * oc[:, 0] + C1 * oc[:, 1] + C2 * oc[:, 2]
-        delta = np.zeros(rows)
-        for g in range(9):
-            delta = delta + np.abs(C0 * G[:, g, 0] + C1 * G[:, g, 1] + C2 * G[:, g, 2])
-        nz = np.sqrt(C0 * C0 + C1 * C1 + C2 * C2) > 0
-        out[:, 2 * i] = np.stack([C0, C1, C2, d + delta], axis=1)
-        out[:, 2 * i + 1] = np.stack([-C0, -C1, -C2, -d + delta], axis=1)
-        nzs[:, 2 * i] = nzs[:, 2 * i + 1] = nz
-    return out, nzs
 
 
 def _check_images(eng, failed=(), obs=None, g0=None):
@@ -88,12 +60,10 @@ def _check_images(eng, failed=(), obs=None, g0=None):
                     assert uc[i] == ex["cu"][src] and ur[i] == ex["ru"][src]
             if rows == 0:
                 continue
-            cnt = b[lay["counts"]:lay["counts"] + rows]
+            cnt, grp, recs, first = chunk_candidates(b, lay, rows)
             assert np.array_equal(cnt, cnt_all[p, tb].reshape(-1))
             stored = np.where(cnt == 255, 0, cnt).astype(np.int64)
-            grp = b[lay["groups"]:lay["groups"] + 4 * ((rows + 31) // 32)].view(np.uint32)
-            assert np.array_equal(grp, np.concatenate([[0], np.cumsum(stored)])[0:rows:32])
-            recs = d[lay["records"] // 8:lay["records"] // 8 + 4 * stored.sum()].reshape(-1, 4)
+            assert np.array_equal(grp, first[0:rows:32])
             if obs is not None:
                 _check_records(eng, ex, obs[p], tb, C_, cnt, recs, g0 if p == 0 else None)
             # the link tables follow the records directly
@@ -102,12 +72,9 @@ def _check_images(eng, failed=(), obs=None, g0=None):
 
 def _check_records(eng, ex, ob, tb, C_, cnt, recs, g0):
     NJ, O, T = eng.NJ, ob.shape[0], eng.T
+    t, l, o = chunk_rows(NJ, C_, O, tb)
     x = np.arange(NJ * C_ * O)
-    o, tt, l = x % O, (x // O) % C_, x // (O * C_)
-    t = tb * C_ + tt
-    LG = ex["link_gens"][t, l]                    # [rows, 18], column-major 3 x 6
-    G = np.concatenate([ob[o, 3:12].reshape(-1, 3, 3), LG.reshape(-1, 6, 3)], axis=1)
-    hs, nz = _half_spaces(G, ob[o, 0:3])
+    hs, nz = half_spaces(*row_generators(ob, ex["link_gens"], t, l, o))
     if g0 is not None:
         centres = eng.link_sliced_center()[t, l]  # [rows, 3] of problem 0
     first = 0
