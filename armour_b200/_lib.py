@@ -175,6 +175,12 @@ SIGNATURES.update({
                                        C.POINTER(RolloutOut)]),
     "armour_batch_clearance_device": (C.c_int, [C.c_void_p, C.c_int] + [C.c_void_p] * 3 + [C.c_int, C.c_void_p, C.c_void_p]),
     "armour_batch_clearance": (C.c_int, [C.c_void_p, C.c_int, dp, ip, dp, C.c_int, dp, ip]),
+    "armour_armtd_batch_rollout_device": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int,
+                                                    C.POINTER(RolloutOptions), C.POINTER(RolloutOut)]),
+    "armour_armtd_batch_rollout": (C.c_int, [C.c_void_p, C.c_int, dp, dp, dp, C.c_int, C.POINTER(RolloutOptions),
+                                             C.POINTER(RolloutOut)]),
+    "armour_armtd_offline_jrs": (C.c_int, [C.c_void_p, C.c_int, dp, dp, dp]),
+    "armour_armtd_offline_jrs_device": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p]),
 })
 
 

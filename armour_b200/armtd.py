@@ -178,6 +178,21 @@ class ArmtdBatch:
         self._check(rc)
         return self
 
+    def offline_jrs(self, qd0, k_range):
+        """The offline table the episodes build from (armour_armtd_offline_jrs): this repository's synthetic stand-in for the
+        reference's CORA tables, computed on the device; worlds.armtd_offline_jrs_batch restated to a few ulp.  qd0, k_range
+        [n, 7] -> [n, 6, 7, 100]."""
+        qd0, k_range = _f64(qd0).reshape(-1, NF), _f64(k_range).reshape(-1, NF)
+        if qd0.shape != k_range.shape:
+            raise ValueError("qd0 and k_range must have one row per problem")
+        out = np.empty((qd0.shape[0], 6, NF, T))
+        self._check(self.lib.armour_armtd_offline_jrs(self._h, qd0.shape[0], _dp(qd0), _dp(k_range), _dp(out)))
+        return out
+
+    def offline_jrs_device(self, n, d_qd0, d_k_range, d_jrs):
+        """Asynchronous armour_armtd_offline_jrs_device on device pointers (ints)."""
+        self._check(self.lib.armour_armtd_offline_jrs_device(self._h, n, d_qd0, d_k_range, d_jrs))
+
     def build_device(self, nprob, nobs, d_q0, d_qd0, d_jrs, d_k_range, d_obstacles, d_sincos=None):
         """Asynchronous build from device pointers (ints, e.g. torch.Tensor.data_ptr()); d_sincos [n, 7, 2] = cos q0, sin q0,
         or None for the device's sincos."""
@@ -261,3 +276,14 @@ class ArmtdBatch:
         self._check(self.lib.armour_armtd_batch_solve(self._h, self.nprob, _dp(q_des), C.byref(opt), _dp(k), _ip(ok), _ip(first),
                                                       _ip(iters)))
         return k, ok.astype(bool), first, iters
+
+    def rollout(self, start, goal, obstacles, max_replans=100, goal_radius=0.05, lookahead=0.1, audit_samples=16, max_iter=None,
+                tol=1e-7, collision_tol=None, qp_sweeps=None):
+        """Closed-loop episodes of this planner for a batch of worlds on the device (armour_armtd_batch_rollout; semantics in
+        include/armour_b200.h): the same worlds, options, audit and returned dict as ReachSetEngine.rollout, KPA's tolerance by
+        default.  The context's reach sets afterwards are those of the last replan's sub-batch: build again before evaluating."""
+        from .planner import run_rollout
+        res = run_rollout(self, self.lib.armour_armtd_batch_rollout, start, goal, obstacles, max_replans, goal_radius, lookahead,
+                          audit_samples, dict(max_iter=max_iter, tol=tol, collision_tol=collision_tol, qp_sweeps=qp_sweeps))
+        self.nprob, self.nobs, self.m = 0, 0, 0
+        return res

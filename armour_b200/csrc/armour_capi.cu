@@ -987,9 +987,13 @@ void armour_rollout_options_default(armour_rollout_options* opt) {
 
 namespace {
 
-int check_rollout(armour_ctx* ctx, int nworlds, int nobs, const armour_rollout_options* opt) {
+// armtd: the call runs episodes of the ARMTD comparison planner (armour_armtd_batch_rollout*), which need a context of that planner
+int check_rollout(armour_ctx* ctx, int nworlds, int nobs, const armour_rollout_options* opt, bool armtd) {
     if (!ctx) return ARMOUR_ERR_ARG;
-    if (ctx->armtd) return fail(ctx, ARMOUR_ERR_STATE, "closed-loop episodes run the main planner, not the ARMTD comparison planner");
+    if (ctx->armtd && !armtd)
+        return fail(ctx, ARMOUR_ERR_STATE, "armour_batch_rollout runs the main planner: use armour_armtd_batch_rollout on an ARMTD context");
+    if (!ctx->armtd && armtd)
+        return fail(ctx, ARMOUR_ERR_STATE, "not an ARMTD context (armour_armtd_ctx_create / armour_armtd_batch_ctx_create)");
     if (nworlds < 1) return fail(ctx, ARMOUR_ERR_ARG, "nworlds < 1");
     if (nworlds > ctx->cfg.max_problems) return fail(ctx, ARMOUR_ERR_STATE, "nworlds larger than max_problems");
     if (nobs < 0) return fail(ctx, ARMOUR_ERR_ARG, "negative obstacle count");
@@ -1003,14 +1007,51 @@ int check_rollout(armour_ctx* ctx, int nworlds, int nobs, const armour_rollout_o
     return ARMOUR_OK;
 }
 
-// The episode loop (include/armour_b200.h, "closed-loop replanning episodes"): per replan k_rollout_plan, the device build and
-// solve of the running worlds, k_rollout_advance, k_clearance over the audit samples, k_rollout_finish; then one copy of the
-// running count to the host and one synchronisation.
+// The planner policies of the episode loop.  extra: doubles of rollout scratch per world beyond the common arrays, bound by
+// bind(w, N); plan(): the build and solve of the dense batch of nrun running worlds into D.dk / dfeas / dfirst / diters;
+// traj(): the trajectory class of k_rollout_advance.
+// The main planner: armour_batch_reachsets_build_device + armour_batch_solve_device, the Bezier of its plans.
+struct ArmourEpisodes {
+    static constexpr size_t extra = 0;
+    void bind(double*, size_t) {}
+    int plan(armour_ctx* ctx, const RolloutDev& D, int nrun, int nobs, const armour_solver_options& so) const {
+        int rc = armour_batch_reachsets_build_device(ctx, nrun, D.dq0, D.dqd0, D.dqdd0, nobs > 0 ? D.dobs : nullptr, nobs);
+        if (rc) return rc;
+        return armour_batch_solve_device(ctx, nrun, D.dq_des, &so, D.dk, D.dfeas, D.dfirst, D.diters);
+    }
+    RollBezier traj() const { return {}; }
+};
+// The ARMTD comparison planner: a prepare step (k_armtd_offline_jrs deriving k_range from qd0 and the stand-in table of every
+// running world), armour_armtd_batch_build_device with the device's sincos + armour_armtd_batch_solve_device, the
+// constant-acceleration curve.  Scratch: k_range [N][NF] and the table [N][6][NF][100] of the dense batch.
+struct ArmtdEpisodes {
+    static constexpr size_t extra = NF + 6 * NF * ARMTD_T;
+    double* k_range = nullptr;
+    double* jrs = nullptr;
+    void bind(double* w, size_t N) {
+        k_range = w;
+        jrs = w + N * NF;
+    }
+    int plan(armour_ctx* ctx, const RolloutDev& D, int nrun, int nobs, const armour_solver_options& so) const {
+        CU(launch_armtd_offline_jrs(nrun, D.dqd0, nullptr, k_range, jrs, ctx->stream));
+        ctx->launches += 1;
+        int rc = armour_armtd_batch_build_device(ctx, nrun, D.dq0, D.dqd0, jrs, k_range, nobs > 0 ? D.dobs : nullptr, nobs, nullptr);
+        if (rc) return rc;
+        return armour_armtd_batch_solve_device(ctx, nrun, D.dq_des, &so, D.dk, D.dfeas, D.dfirst, D.diters);
+    }
+    RollConstAcc traj() const { return {k_range}; }
+};
+
+// The episode loop (include/armour_b200.h, "closed-loop replanning episodes"): per replan k_rollout_plan, the planner's device
+// build and solve of the running worlds, k_rollout_advance, k_clearance over the audit samples, k_rollout_finish; then one copy
+// of the running count to the host and one synchronisation.
+template <class Episodes>
 int rollout_run(armour_ctx* ctx, int n, const double* d_start, const double* d_goal, const double* d_obstacles, int nobs,
                 const armour_rollout_options& opt, const armour_rollout_out& out) {
     { int rc_e = enter(ctx); if (rc_e) return rc_e; }
     const size_t N = size_t(n), S = size_t(opt.audit_samples), no = size_t(nobs) * 12;
-    CU(ctx->d_roll.reserve(N * (ROLL_STATE + ROLL_PLAN + 1 + 5 * NF + 1) + N * no + N * S * NF));
+    CU(ctx->d_roll.reserve(N * (ROLL_STATE + ROLL_PLAN + 1 + 5 * NF + 1) + N * no + N * S * NF + N * Episodes::extra));
+    Episodes ep;
     CU(ctx->d_roll_i.reserve(10 * N + 1));
     RolloutDev D;
     D.n = n;
@@ -1034,7 +1075,8 @@ int rollout_run(armour_ctx* ctx, int n, const double* d_start, const double* d_g
     D.dk = w; w += N * NF;
     D.dclear = w; w += N;
     D.dobs = w; w += N * no;
-    D.samp = w;
+    D.samp = w; w += N * S * NF;
+    ep.bind(w, N);
     int* wi = ctx->d_roll_i.get();
     D.outcome = wi; wi += N;
     D.replans = wi; wi += N;
@@ -1062,9 +1104,8 @@ int rollout_run(armour_ctx* ctx, int n, const double* d_start, const double* d_g
         k_rollout_plan<<<gb, ROLL_THREADS, 0, st>>>(D, r, nrun, list);
         CU(cudaGetLastError());
         ctx->launches += 1;
-        { int rc = armour_batch_reachsets_build_device(ctx, nrun, D.dq0, D.dqd0, D.dqdd0, nobs > 0 ? D.dobs : nullptr, nobs); if (rc) return rc; }
-        { int rc = armour_batch_solve_device(ctx, nrun, D.dq_des, &opt.solver, D.dk, D.dfeas, D.dfirst, D.diters); if (rc) return rc; }
-        k_rollout_advance<<<gb, ROLL_THREADS, 0, st>>>(D, r, nrun, list, ctx->B.status, ctx->B.epoch);
+        { int rc = ep.plan(ctx, D, nrun, nobs, opt.solver); if (rc) return rc; }
+        k_rollout_advance<<<gb, ROLL_THREADS, 0, st>>>(D, r, nrun, list, ctx->B.status, ctx->B.epoch, ep.traj());
         k_clearance<<<nrun, CLEAR_THREADS, 0, st>>>(D.samp, opt.audit_samples, list, d_obstacles, nobs, D.dclear, nullptr);
         k_rollout_finish<<<1, FINISH_THREADS, 0, st>>>(D, r, nrun, list, next, d_count);
         CU(cudaGetLastError());
@@ -1081,29 +1122,24 @@ int rollout_run(armour_ctx* ctx, int n, const double* d_start, const double* d_g
     return ARMOUR_OK;
 }
 
-int check_clearance(armour_ctx* ctx, int nconf, int nobs) {
-    if (!ctx) return ARMOUR_ERR_ARG;
-    if (nconf < 1) return fail(ctx, ARMOUR_ERR_ARG, "nconf < 1");
-    if (nobs < 0) return fail(ctx, ARMOUR_ERR_ARG, "negative obstacle count");
-    if (nobs > ctx->cfg.max_obstacles) return fail(ctx, ARMOUR_ERR_OBSTACLES, "number of obstacles larger than max_obstacles");
-    return ARMOUR_OK;
+int run_episodes(armour_ctx* ctx, bool armtd, int n, const double* d_start, const double* d_goal, const double* d_obstacles, int nobs,
+                 const armour_rollout_options& opt, const armour_rollout_out& out) {
+    if (armtd) return rollout_run<ArmtdEpisodes>(ctx, n, d_start, d_goal, d_obstacles, nobs, opt, out);
+    return rollout_run<ArmourEpisodes>(ctx, n, d_start, d_goal, d_obstacles, nobs, opt, out);
 }
 
-}  // namespace
-
-extern "C" {
-
-int armour_batch_rollout_device(armour_ctx* ctx, int nworlds, const double* d_start, const double* d_goal, const double* d_obstacles,
-                                int nobs, const armour_rollout_options* opt, const armour_rollout_out* d_out) {
-    int rc = check_rollout(ctx, nworlds, nobs, opt);
+int rollout_device(armour_ctx* ctx, int nworlds, const double* d_start, const double* d_goal, const double* d_obstacles, int nobs,
+                   const armour_rollout_options* opt, const armour_rollout_out* d_out, bool armtd) {
+    int rc = check_rollout(ctx, nworlds, nobs, opt, armtd);
     if (rc) return rc;
     if (!d_start || !d_goal || (nobs > 0 && !d_obstacles) || !d_out) return fail(ctx, ARMOUR_ERR_ARG, "null input");
-    return rollout_run(ctx, nworlds, d_start, d_goal, d_obstacles, nobs, *opt, *d_out);
+    return run_episodes(ctx, armtd, nworlds, d_start, d_goal, d_obstacles, nobs, *opt, *d_out);
 }
 
-int armour_batch_rollout(armour_ctx* ctx, int nworlds, const double* start, const double* goal, const double* obstacles, int nobs,
-                         const armour_rollout_options* opt, const armour_rollout_out* out) {
-    int rc = check_rollout(ctx, nworlds, nobs, opt);
+// host-pointer front of the episodes: stages the inputs in and the requested outputs out
+int rollout_host(armour_ctx* ctx, int nworlds, const double* start, const double* goal, const double* obstacles, int nobs,
+                 const armour_rollout_options* opt, const armour_rollout_out* out, bool armtd) {
+    int rc = check_rollout(ctx, nworlds, nobs, opt, armtd);
     if (rc) return rc;
     if (!start || !goal || (nobs > 0 && !obstacles) || !out) return fail(ctx, ARMOUR_ERR_ARG, "null input");
     CU(cudaSetDevice(ctx->cfg.device));
@@ -1132,8 +1168,8 @@ int armour_batch_rollout(armour_ctx* ctx, int nworlds, const double* start, cons
     d_out.log_k = static_cast<double*>(d[10]);
     d_out.log_int = static_cast<int*>(d[11]);
     d_out.log_clearance = static_cast<double*>(d[12]);
-    rc = rollout_run(ctx, nworlds, static_cast<double*>(d[0]), static_cast<double*>(d[1]), static_cast<double*>(d[2]), nobs, *opt,
-                     d_out);
+    rc = run_episodes(ctx, armtd, nworlds, static_cast<double*>(d[0]), static_cast<double*>(d[1]), static_cast<double*>(d[2]), nobs,
+                      *opt, d_out);
     if (rc) return rc;
     void* host[13] = {nullptr, nullptr, nullptr, out->outcome, out->replans, out->infeasible, out->final_state, out->min_clearance,
                       out->log_state, out->log_q_des, out->log_k, out->log_int, out->log_clearance};
@@ -1143,6 +1179,39 @@ int armour_batch_rollout(armour_ctx* ctx, int nworlds, const double* start, cons
     return ARMOUR_OK;
 }
 
+
+int check_clearance(armour_ctx* ctx, int nconf, int nobs) {
+    if (!ctx) return ARMOUR_ERR_ARG;
+    if (nconf < 1) return fail(ctx, ARMOUR_ERR_ARG, "nconf < 1");
+    if (nobs < 0) return fail(ctx, ARMOUR_ERR_ARG, "negative obstacle count");
+    if (nobs > ctx->cfg.max_obstacles) return fail(ctx, ARMOUR_ERR_OBSTACLES, "number of obstacles larger than max_obstacles");
+    return ARMOUR_OK;
+}
+
+}  // namespace
+
+extern "C" {
+
+int armour_batch_rollout_device(armour_ctx* ctx, int nworlds, const double* d_start, const double* d_goal, const double* d_obstacles,
+                                int nobs, const armour_rollout_options* opt, const armour_rollout_out* d_out) {
+    return rollout_device(ctx, nworlds, d_start, d_goal, d_obstacles, nobs, opt, d_out, false);
+}
+
+int armour_batch_rollout(armour_ctx* ctx, int nworlds, const double* start, const double* goal, const double* obstacles, int nobs,
+                         const armour_rollout_options* opt, const armour_rollout_out* out) {
+    return rollout_host(ctx, nworlds, start, goal, obstacles, nobs, opt, out, false);
+}
+
+int armour_armtd_batch_rollout_device(armour_ctx* ctx, int nworlds, const double* d_start, const double* d_goal,
+                                      const double* d_obstacles, int nobs, const armour_rollout_options* opt,
+                                      const armour_rollout_out* d_out) {
+    return rollout_device(ctx, nworlds, d_start, d_goal, d_obstacles, nobs, opt, d_out, true);
+}
+
+int armour_armtd_batch_rollout(armour_ctx* ctx, int nworlds, const double* start, const double* goal, const double* obstacles,
+                               int nobs, const armour_rollout_options* opt, const armour_rollout_out* out) {
+    return rollout_host(ctx, nworlds, start, goal, obstacles, nobs, opt, out, true);
+}
 int armour_batch_clearance_device(armour_ctx* ctx, int nconf, const double* d_q, const int* d_world, const double* d_obstacles,
                                   int nobs, double* d_clearance, int* d_which) {
     int rc = check_clearance(ctx, nconf, nobs);
@@ -1533,6 +1602,37 @@ int armour_armtd_batch_build_device(armour_ctx* ctx, int nprob, const double* d_
     CU(cudaMemcpyAsync(ctx->d_krange, d_k_range, size_t(nprob) * NF * sizeof(double), cudaMemcpyDeviceToDevice, ctx->stream));
     ctx->h_krange.clear();
     return armour_batch_reachsets_build_device(ctx, nprob, d_q0, d_qd0, ctx->d_zero, d_obstacles, nobs);
+}
+
+int armour_armtd_offline_jrs_device(armour_ctx* ctx, int n, const double* d_qd0, const double* d_k_range, double* d_jrs) {
+    if (!ctx) return ARMOUR_ERR_ARG;
+    if (!ctx->armtd) return fail(ctx, ARMOUR_ERR_STATE, "not an ARMTD context (armour_armtd_ctx_create / armour_armtd_batch_ctx_create)");
+    if (n < 1) return fail(ctx, ARMOUR_ERR_ARG, "n < 1");
+    if (!d_qd0 || !d_k_range || !d_jrs) return fail(ctx, ARMOUR_ERR_ARG, "null input");
+    { int rc_e = enter(ctx); if (rc_e) return rc_e; }
+    CU(launch_armtd_offline_jrs(n, d_qd0, d_k_range, nullptr, d_jrs, ctx->stream));
+    ctx->launches++;
+    return ARMOUR_OK;
+}
+
+int armour_armtd_offline_jrs(armour_ctx* ctx, int n, const double* qd0, const double* k_range, double* jrs) {
+    if (!ctx) return ARMOUR_ERR_ARG;
+    if (!ctx->armtd) return fail(ctx, ARMOUR_ERR_STATE, "not an ARMTD context (armour_armtd_ctx_create / armour_armtd_batch_ctx_create)");
+    if (n < 1) return fail(ctx, ARMOUR_ERR_ARG, "n < 1");
+    if (!qd0 || !k_range || !jrs) return fail(ctx, ARMOUR_ERR_ARG, "null input");
+    CU(cudaSetDevice(ctx->cfg.device));
+    const size_t nk = size_t(n) * NF * sizeof(double), nj = size_t(n) * 6 * NF * ARMTD_T * sizeof(double);
+    void* d[3];  // qd0, k_range, jrs
+    int rc = stage(ctx, {nk, nk, nj}, d);
+    if (rc) return rc;
+    cudaStream_t st = ctx->stream;
+    CU(cudaMemcpyAsync(d[0], qd0, nk, cudaMemcpyHostToDevice, st));
+    CU(cudaMemcpyAsync(d[1], k_range, nk, cudaMemcpyHostToDevice, st));
+    rc = armour_armtd_offline_jrs_device(ctx, n, static_cast<double*>(d[0]), static_cast<double*>(d[1]), static_cast<double*>(d[2]));
+    if (rc) return rc;
+    CU(cudaMemcpyAsync(jrs, d[2], nj, cudaMemcpyDeviceToHost, st));
+    CU(cudaStreamSynchronize(st));
+    return ARMOUR_OK;
 }
 
 int armour_armtd_batch_build(armour_ctx* ctx, int nprob, const double* q0, const double* qd0, const double* jrs,

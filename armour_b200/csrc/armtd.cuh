@@ -114,6 +114,94 @@ __host__ __device__ inline void armtd_joint_extremum(double q0, double qd0, doub
     grad[3] = d ? gv_max_p : gv_max_s;
 }
 
+// The executed motion of an ARMTD plan, the constant-acceleration curve of armtd_joint_extremum for one joint at time t in
+// [0, 1] (k_actual = k_range * k): q0 + qd0 t + k_actual t^2 / 2 up to t_move, then braking to rest at t_total.  Both phases are
+// written with armtd_joint_extremum's expressions (q_peak, q_dot_peak, q_ddot_to_stop, q_stop with tau in place of t_to_stop),
+// so the end points at t = 0.5 and t = 1 are exactly the values its joint-limit rows bounded.
+__host__ __device__ inline void armtd_curve(double q0, double qd0, double k_actual, double t, double* q, double* qd) {
+    const double t_move = 0.5, t_total = 1.0, t_to_stop = t_total - t_move;
+    if (t <= t_move) {
+        *q = q0 + qd0 * t + k_actual * t * t * 0.5;
+        *qd = qd0 + k_actual * t;
+        return;
+    }
+    const double q_peak = q0 + qd0 * t_move + k_actual * t_move * t_move * 0.5;
+    const double q_dot_peak = qd0 + k_actual * t_move;
+    const double q_ddot_to_stop = -q_dot_peak / t_to_stop;
+    const double tau = t - t_move;
+    *q = q_peak + q_dot_peak * tau + 0.5 * q_ddot_to_stop * tau * tau;
+    *qd = q_dot_peak + q_ddot_to_stop * tau;
+}
+
+// This repository's SYNTHETIC STAND-IN for the reference's offline joint-reachable-set table, not the reference's CORA table
+// (that one is MATLAB output the reference tree does not contain): worlds.armtd_offline_jrs_batch restated operation for
+// operation, one thread per (problem, joint, interval).  For interval j of [0, 1] in 100 steps, the displacement
+// d(t, k) = q(t) - q0 = A(t) + B(t) * k_range * k of the curve above gets the centre and slope of cos d / sin d at the interval's
+// mid-time and the radius 1.1 * (largest residual over 9 times x 33 values of k, in numpy's order) + 1e-6.  Output jrs
+// [n][6][NF][100] (c_cos, g_cos, r_cos, c_sin, g_sin, r_sin), the layout of armour_armtd_batch_build_device.  k_range [n][NF]
+// is read when given; with k_range == nullptr it is derived from qd0 as worlds.armtd_k_range does, max(pi / 24, |qd0| / 3),
+// and written to k_range_out (the episodes' prepare step).  The library is compiled with -fmad=false, like numpy's unfused
+// arithmetic; the device's sincos stands in for numpy's cos / sin (a few ulp).
+__device__ __forceinline__ void armtd_offline_coeffs(double qd0, double t, double* A, double* B) {
+    const double tau = t - 0.5;
+    if (t <= 0.5) {
+        *A = qd0 * t;
+        *B = 0.5 * t * t;
+    } else {
+        *A = qd0 * 0.5 + qd0 * tau - qd0 * tau * tau;
+        *B = 0.125 + 0.5 * tau - 0.5 * tau * tau;
+    }
+}
+__global__ void __launch_bounds__(256)
+k_armtd_offline_jrs(int n, const double* __restrict__ qd0, const double* __restrict__ k_range, double* __restrict__ k_range_out,
+                    double* __restrict__ jrs) {
+    const int x = blockIdx.x * blockDim.x + threadIdx.x;
+    if (x >= n * NF * ARMTD_T) return;
+    const int j = x % ARMTD_T, i = (x / ARMTD_T) % NF, p = x / (ARMTD_T * NF);
+    const double v = qd0[size_t(p) * NF + i];
+    double kr;
+    if (k_range) {
+        kr = k_range[size_t(p) * NF + i];
+    } else {
+        kr = fmax(M_PI / 24, fabs(v) / 3);
+        if (j == 0) k_range_out[size_t(p) * NF + i] = kr;
+    }
+    const double t0 = double(j) / ARMTD_T, t1 = double(j + 1) / ARMTD_T;
+    double A, B;
+    armtd_offline_coeffs(v, 0.5 * (t0 + t1), &A, &B);
+    double sA, cA;
+    sincos(A, &sA, &cA);
+    const double g_cos = -sA * B * kr, g_sin = cA * B * kr;
+    double r_cos = 0.0, r_sin = 0.0;
+    for (int a = 0; a < 9; a++) {
+        const double s = double(a) * 0.125;  // np.linspace(0, 1, 9), exact
+        double At, Bt;
+        armtd_offline_coeffs(v, t0 + s * (t1 - t0), &At, &Bt);
+        for (int b = 0; b < 33; b++) {
+            const double k = double(b) * 0.0625 + -1.0;  // np.linspace(-1, 1, 33), exact
+            const double d = At + Bt * kr * k;
+            double sd, cd;
+            sincos(d, &sd, &cd);
+            r_cos = fmax(r_cos, fabs(cd - (cA + g_cos * k)));
+            r_sin = fmax(r_sin, fabs(sd - (sA + g_sin * k)));
+        }
+    }
+    double* o = jrs + size_t(p) * 6 * NF * ARMTD_T + size_t(i) * ARMTD_T + j;  // o[c * NF * 100]: array c
+    const size_t S = size_t(NF) * ARMTD_T;
+    o[0 * S] = cA;
+    o[1 * S] = g_cos;
+    o[2 * S] = 1.1 * r_cos + 1e-6;
+    o[3 * S] = sA;
+    o[4 * S] = g_sin;
+    o[5 * S] = 1.1 * r_sin + 1e-6;
+}
+inline cudaError_t launch_armtd_offline_jrs(int n, const double* qd0, const double* k_range, double* k_range_out, double* jrs,
+                                            cudaStream_t st) {
+    const int nt = n * NF * ARMTD_T;
+    k_armtd_offline_jrs<<<(nt + 255) / 256, 256, 0, st>>>(n, qd0, k_range, k_range_out, jrs);
+    return cudaGetLastError();
+}
+
 // g_full / j_full: the main planner's layout with Tp = 104 intervals (torque rows, collision rows (l * Tp + t) * O + o, Bezier
 // rows), B.m() rows per problem; g / jac: KPA's layout, armtd_m() rows per problem, collision rows (l * 100 + t) * O + o then
 // 4 * NF joint-limit rows (KPA/NLPclass.cu:43-44, 248-336).  The joint-limit rows of the Jacobian are diagonal: the reference

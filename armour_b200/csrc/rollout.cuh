@@ -1,23 +1,26 @@
-// Closed-loop replanning episodes on the device (armour_batch_rollout*) and the exact clearance of arm configurations
-// (armour_batch_clearance*).  The semantics are those of include/armour_b200.h and DESIGN.md section 3 ("Closed-loop
-// episodes"); the host loop that sequences these kernels around the device build and solve is rollout_run in armour_capi.cu.
+// Closed-loop replanning episodes on the device (armour_batch_rollout*, armour_armtd_batch_rollout*) and the exact clearance
+// of arm configurations (armour_batch_clearance*).  The semantics are those of include/armour_b200.h and DESIGN.md section 3
+// ("Closed-loop episodes"); the host loop that sequences these kernels around the device build and solve is rollout_run in
+// armour_capi.cu, templated over the planner like the batched solver over its NLP.
 //
-// Per replan: k_rollout_plan (compaction list -> dense planning inputs, waypoint, log rows), the existing build and solve on
-// the running worlds, k_rollout_advance (verdict -> executed segment, next state, audit samples), k_clearance over the audit
-// samples, k_rollout_finish (stop tests, stable compaction of the running worlds in ascending world index).
+// Per replan: k_rollout_plan (compaction list -> dense planning inputs, waypoint, log rows), the planner's build and solve on
+// the running worlds, k_rollout_advance (verdict -> executed segment, next state, audit samples; its trajectory class is a
+// template parameter), k_clearance over the audit samples, k_rollout_finish (stop tests, stable compaction of the running worlds
+// in ascending world index).
 #pragma once
 #include <climits>
 #include <cuda_runtime.h>
 #include <math_constants.h>
 
 #include "../../include/armour_b200.h"
+#include "armtd.cuh"
 #include "bezier.cuh"
 #include "device_constants.cuh"
 
 namespace armour {
 
 constexpr int ROLL_STATE = 3 * NF;  // q, qd, qdd
-constexpr int ROLL_PLAN = 4 * NF;   // q0, qd0, qdd0 (real time), k (rad): the Bezier of an executed plan
+constexpr int ROLL_PLAN = 4 * NF;   // q0, qd0, qdd0 (real time), k (rad): the Bezier of an executed plan; ARMTD: q0, qd0, 0, k_a
 constexpr int ROLL_THREADS = 128;
 constexpr int CLEAR_THREADS = 128;
 constexpr int FINISH_THREADS = 1024;
@@ -137,10 +140,38 @@ __device__ __forceinline__ void roll_eval_plan(const double* P, double s, double
     }
 }
 
+// Trajectory classes of k_rollout_advance: the scale of a solved k into the plan's last slot for batch position i and joint j,
+// the normalised time t_move of the segment split, and (q, qd, qdd) of a stored plan at normalised time s.
+// The main planner's: the Bezier of roll_eval_plan, k scaled by the robot model's k_range.
+struct RollBezier {
+    __device__ __forceinline__ double k_scale(int, int j) const { return c_robot.k_range[j]; }
+    __device__ __forceinline__ double s_move() const { return c_robot.t_plan / c_robot.duration; }
+    __device__ __forceinline__ void eval(const double* P, double s, double* q, double* qd, double* qdd) const {
+        roll_eval_plan(P, s, q, qd, qdd);
+    }
+};
+// The ARMTD comparison planner's: the constant-acceleration curve of armtd_curve over t in [0, 1] (t_move 0.5), k scaled by the
+// k_range of the replan ([i][NF], dense), the plan stored as (q0, qd0, 0, k_a).  The planner has no acceleration input: qdd is 0.
+struct RollConstAcc {
+    const double* k_range;
+    __device__ __forceinline__ double k_scale(int i, int j) const { return k_range[size_t(i) * NF + j]; }
+    __device__ __forceinline__ double s_move() const { return 0.5; }
+    __device__ __forceinline__ void eval(const double* P, double s, double* q, double* qd, double* qdd) const {
+        for (int j = 0; j < NF; j++) {
+            double a, b;
+            armtd_curve(P[j], P[NF + j], P[3 * NF + j], s, &a, &b);
+            if (q) q[j] = a;
+            if (qd) qd[j] = b;
+            if (qdd) qdd[j] = 0.0;
+        }
+    }
+};
+
 // the solve's verdict -> executed segment (the new plan over [0, t_move] or the current plan's braking half [t_move, 1]),
 // next state, current plan, counters, audit samples and the joint-limit audit
+template <class Traj>
 __global__ void k_rollout_advance(RolloutDev D, int r, int nrun, const int* __restrict__ list, const int* __restrict__ build_status,
-                                  int epoch) {
+                                  int epoch, Traj traj) {
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= nrun) return;
     const RobotConstants& R = c_robot;
@@ -158,13 +189,13 @@ __global__ void k_rollout_advance(RolloutDev D, int r, int nrun, const int* __re
     }
     double* P = D.plan + size_t(w) * ROLL_PLAN;
     double* st = D.state + size_t(w) * ROLL_STATE;
-    const double s_move = R.t_plan / R.duration;
+    const double s_move = traj.s_move();
     if (ok) {  // the new plan becomes the current plan
         for (int j = 0; j < NF; j++) {
             P[j] = st[j];
             P[NF + j] = st[NF + j];
             P[2 * NF + j] = st[2 * NF + j];
-            P[3 * NF + j] = R.k_range[j] * D.dk[size_t(i) * NF + j];
+            P[3 * NF + j] = traj.k_scale(i, j) * D.dk[size_t(i) * NF + j];
         }
     }
     const double s0 = ok ? 0.0 : s_move, s1 = ok ? s_move : 1.0;
@@ -173,7 +204,7 @@ __global__ void k_rollout_advance(RolloutDev D, int r, int nrun, const int* __re
     for (int m = 0; m < D.S; m++) {
         const double s = s0 + (s1 - s0) * double(m) / double(D.S - 1);
         double q[NF], qd[NF];
-        roll_eval_plan(P, s, q, qd, nullptr);
+        traj.eval(P, s, q, qd, nullptr);
         for (int j = 0; j < NF; j++) {
             D.samp[(size_t(i) * D.S + m) * NF + j] = q[j];
             if (!roll_continuous(j) && (q[j] < R.state_limits_lb[j] || q[j] > R.state_limits_ub[j])) lim = 1;
@@ -183,15 +214,15 @@ __global__ void k_rollout_advance(RolloutDev D, int r, int nrun, const int* __re
     D.limit[w] = lim;
     if (ok) {
         double q[NF], qd[NF], qdd[NF];
-        roll_eval_plan(P, s_move, q, qd, qdd);
+        traj.eval(P, s_move, q, qd, qdd);
         for (int j = 0; j < NF; j++) {
             st[j] = q[j];
             st[NF + j] = qd[j];
             st[2 * NF + j] = qdd[j];
         }
-    } else {  // braked to rest at s = 1: the current plan becomes the rest plan there (a constant Bezier)
+    } else {  // braked to rest at s = 1: the current plan becomes the rest plan there (constant in both trajectory classes)
         double q[NF];
-        roll_eval_plan(P, 1.0, q, nullptr, nullptr);
+        traj.eval(P, 1.0, q, nullptr, nullptr);
         for (int j = 0; j < NF; j++) {
             st[j] = q[j];
             st[NF + j] = 0.0;

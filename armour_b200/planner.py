@@ -23,6 +23,33 @@ def _dp(a):
     return a.ctypes.data_as(_lib.dp)
 
 
+def run_rollout(owner, fn, start, goal, obstacles, max_replans, goal_radius, lookahead, audit_samples, solver):
+    """One call of an episode entry point with host pointers (armour_batch_rollout or armour_armtd_batch_rollout: the same
+    arguments) for owner's context; solver: solver option name -> value, None keeps the default.  Returns the dict of
+    ReachSetEngine.rollout."""
+    start, goal = _f64(start).reshape(-1, NF), _f64(goal).reshape(-1, NF)
+    n = start.shape[0]
+    obs = _f64(obstacles)
+    obs = obs.reshape(n, -1, 12) if obs.size else np.zeros((n, 0, 12))
+    opt = _lib.RolloutOptions()
+    owner.lib.armour_rollout_options_default(C.byref(opt))
+    opt.max_replans, opt.goal_radius, opt.lookahead = int(max_replans), float(goal_radius), float(lookahead)
+    opt.audit_samples = int(audit_samples)
+    for name, v in solver.items():
+        if v is not None:
+            setattr(opt.solver, name, type(getattr(opt.solver, name))(v))
+    R = opt.max_replans
+    res = dict(outcome=np.zeros(n, np.int32), replans=np.zeros(n, np.int32), infeasible=np.zeros(n, np.int32),
+               final_state=np.zeros((n, 3 * NF)), min_clearance=np.zeros(n), log_state=np.zeros((max(R, 0), n, 3 * NF)),
+               log_q_des=np.zeros((max(R, 0), n, NF)), log_k=np.zeros((max(R, 0), n, NF)),
+               log_int=np.zeros((max(R, 0), n, 4), np.int32), log_clearance=np.zeros((max(R, 0), n)))
+    out = _lib.RolloutOut()
+    for name, a in res.items():
+        setattr(out, name, a.ctypes.data_as(_lib.ip if a.dtype == np.int32 else _lib.dp))
+    owner._check(fn(owner._h, n, _dp(start), _dp(goal), _dp(obs), obs.shape[1], C.byref(opt), C.byref(out)))
+    return res
+
+
 class ReachSetEngine:
     def __init__(self, max_problems=1, max_obstacles=40, device=0, robot_model=0, num_time_steps=128,
                  simplify_threshold=5e-4, k_range=None, cap_link=32, cap_torque=64, cap_work=768,
@@ -175,28 +202,9 @@ class ReachSetEngine:
         replans, infeasible [n], final_state [n, 21], min_clearance [n], log_state [R, n, 21], log_q_des, log_k [R, n, 7],
         log_int [R, n, 4] (feasible, first violated row, iterations, build status), log_clearance [R, n].  The context's
         reach sets afterwards are those of the last replan's sub-batch: build again before evaluating."""
-        start, goal = _f64(start).reshape(-1, NF), _f64(goal).reshape(-1, NF)
-        n = start.shape[0]
-        obs = _f64(obstacles)
-        obs = obs.reshape(n, -1, 12) if obs.size else np.zeros((n, 0, 12))
-        opt = _lib.RolloutOptions()
-        self.lib.armour_rollout_options_default(C.byref(opt))
-        opt.max_replans, opt.goal_radius, opt.lookahead = int(max_replans), float(goal_radius), float(lookahead)
-        opt.audit_samples = int(audit_samples)
-        for name, v in (("max_iter", max_iter), ("tol", tol), ("torque_tol", torque_tol), ("collision_tol", collision_tol),
-                        ("qp_sweeps", qp_sweeps)):
-            if v is not None:
-                setattr(opt.solver, name, type(getattr(opt.solver, name))(v))
-        R = opt.max_replans
-        res = dict(outcome=np.zeros(n, np.int32), replans=np.zeros(n, np.int32), infeasible=np.zeros(n, np.int32),
-                   final_state=np.zeros((n, 3 * NF)), min_clearance=np.zeros(n), log_state=np.zeros((max(R, 0), n, 3 * NF)),
-                   log_q_des=np.zeros((max(R, 0), n, NF)), log_k=np.zeros((max(R, 0), n, NF)),
-                   log_int=np.zeros((max(R, 0), n, 4), np.int32), log_clearance=np.zeros((max(R, 0), n)))
-        out = _lib.RolloutOut()
-        for name, a in res.items():
-            setattr(out, name, a.ctypes.data_as(_lib.ip if a.dtype == np.int32 else _lib.dp))
-        self._check(self.lib.armour_batch_rollout(self._h, n, _dp(start), _dp(goal), _dp(obs), obs.shape[1], C.byref(opt),
-                                                  C.byref(out)))
+        res = run_rollout(self, self.lib.armour_batch_rollout, start, goal, obstacles, max_replans, goal_radius, lookahead,
+                          audit_samples, dict(max_iter=max_iter, tol=tol, torque_tol=torque_tol, collision_tol=collision_tol,
+                                              qp_sweeps=qp_sweeps))
         self.nprob = 0
         return res
 

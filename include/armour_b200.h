@@ -253,6 +253,36 @@ int armour_batch_rollout_device(armour_ctx* ctx, int nworlds, const double* d_st
 /* The same with host pointers (the copies are part of the call). */
 int armour_batch_rollout(armour_ctx* ctx, int nworlds, const double* start, const double* goal, const double* obstacles, int nobs,
                          const armour_rollout_options* opt, const armour_rollout_out* out);
+/* Episodes of the ARMTD comparison planner (section "ARMTD comparison planner" below), on the same worlds, options, outputs and
+ * audit as the episodes above, on a context of armour_armtd_batch_ctx_create.  Replan r of world w, step by step:
+ *   1. planning state (q0, qd0): (start, 0) at r = 0, afterwards the end of the last executed segment.  The planner has no
+ *      acceleration input: the qdd slots of log_state and final_state are 0 (the 21-wide layout is kept so that
+ *      armour_rollout_out is shared);
+ *   2. q_des: as step 2 above (the same straight-line waypoint and the same clamp at the goal);
+ *   3. plan: k_range = max(pi / 24, |qd0| / 3) per joint (armour_b200.worlds.armtd_k_range) and the offline table of
+ *      armour_armtd_offline_jrs (this library's synthetic stand-in, not the reference's CORA table) for every running world,
+ *      armour_armtd_batch_build_device with the device's sincos (d_sincos NULL) + armour_armtd_batch_solve_device, from k = 0
+ *      with opt->solver as given (armour_rollout_options_default leaves its tol at the main planner's default; KPA's is 1e-7).
+ *      The verdict is KPA's finalize_solution (armour_armtd_batch_verdict_device), so the collision rows of the last link are not
+ *      checked, as in the reference.  A build that overflowed a table is an infeasible replan, logged with its build status;
+ *   4. executed segment: after a feasible plan the new plan over t in [0, 0.5], and it becomes the world's current plan;
+ *      otherwise the current plan's braking half t in [0.5, 1], after which the current plan is the rest plan at q_stop
+ *      (qd0 = 0, k_a = 0).  The trajectory is the constant-acceleration curve of KPA (the one armour_armtd_eval's joint-limit
+ *      rows bound): q0 + qd0 t + k_a t^2 / 2 for t <= 0.5, then q_peak + qd_peak tau - qd_peak tau^2 with tau = t - 0.5, braking
+ *      to rest at t = 1; k_a = k_range * k_opt.  The end points at t = 0.5 and t = 1 are computed by the expressions of those
+ *      rows (q_peak, q_dot_peak, q_stop).  A plan is stored as (q0, qd0, 0, k_a); the initial current plan is the rest plan at
+ *      the start;
+ *   5. next state: (q, qd, 0) at the segment's end;
+ *   6. audit and stop: steps 6 and 7 above unchanged (all num_joints links by the separating-axis test, the raw position and
+ *      speed limits; collision, limit, arrived, budget in this order).
+ * Compaction, log rows and the context's reach sets afterwards: as above.  Rollout scratch grows by 4 207 doubles per world
+ * (the table and k_range of the dense batch).  Errors: ARMOUR_ERR_STATE on a context of the main planner and for
+ * nworlds > max_problems, ARMOUR_ERR_OBSTACLES for nobs > max_obstacles, ARMOUR_ERR_ARG for bad options and null inputs. */
+int armour_armtd_batch_rollout_device(armour_ctx* ctx, int nworlds, const double* d_start, const double* d_goal,
+                                      const double* d_obstacles, int nobs, const armour_rollout_options* opt,
+                                      const armour_rollout_out* d_out);
+int armour_armtd_batch_rollout(armour_ctx* ctx, int nworlds, const double* start, const double* goal, const double* obstacles,
+                               int nobs, const armour_rollout_options* opt, const armour_rollout_out* out);
 /* Exact clearance of nconf arm configurations q [nconf][7]: the link boxes of the context's robot model against obstacle set
  * world[i] of obstacles [nsets][nobs][12] (world NULL: set 0 for all) by the audit's separating-axis test.  clearance[nconf]
  * = the smallest over links and obstacles, which[nconf] (may be NULL) = l * nobs + o of the pair attaining it (ties: the lowest),
@@ -388,6 +418,16 @@ int armour_armtd_batch_build(armour_ctx* ctx, int nprob, const double* q0, const
                              const double* k_range, const double* obstacles, int nobs);
 int armour_armtd_batch_build_device(armour_ctx* ctx, int nprob, const double* d_q0, const double* d_qd0, const double* d_jrs,
                                     const double* d_k_range, const double* d_obstacles, int nobs, const double* d_sincos);
+/* The offline table as this library generates it: a SYNTHETIC STAND-IN for the reference's offline tables (MATLAB / CORA output
+ * that is not in the reference tree), NOT the reference's CORA table.  qd0, k_range [n][7] -> jrs [n][6][7][100] in the layout the
+ * builds take: per joint and interval the centre and slope of cos / sin of q(t) - q0 = qd0 t + k_range k t^2 / 2 (braking to rest
+ * after t = 0.5, the curve of armour_armtd_batch_rollout) at the interval's mid-time, and the radius 1.1 * the largest residual
+ * over 9 x 33 samples of (t, k) + 1e-6.  It restates armour_b200.worlds.armtd_offline_jrs_batch operation for operation; the
+ * device's sincos stands in for numpy's cos / sin, so entries differ from numpy's by a few ulp.  The episodes build from this
+ * table at every replan; these calls let a logged replan be rebuilt from exactly that table.  ARMTD contexts only
+ * (ARMOUR_ERR_STATE otherwise), n >= 1, no limit from max_problems. */
+int armour_armtd_offline_jrs(armour_ctx* ctx, int n, const double* qd0, const double* k_range, double* jrs);
+int armour_armtd_offline_jrs_device(armour_ctx* ctx, int n, const double* d_qd0, const double* d_k_range, double* d_jrs);
 /* eval_g / eval_jac_g of every problem at k (either output may be NULL) */
 int armour_armtd_batch_eval(armour_ctx* ctx, int nprob, const double* k, double* g, double* values);
 int armour_armtd_batch_eval_device(armour_ctx* ctx, int nprob, const double* d_k, double* d_g, double* d_values);
