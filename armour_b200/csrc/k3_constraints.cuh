@@ -782,6 +782,14 @@ k_constraints(Batch B, const double* __restrict__ kin, double* __restrict__ g, d
         const int tt = slicer ? tid / (3 * NJ) : 0;
         const int li = tt * NJ + l;  // table of the chunk
         const int2 lt = slicer ? reinterpret_cast<const int2*>(img)[li] : make_int2(0, 0);
+        {
+            // the chunk's candidate records end where link table 0 starts: ask L2 for all of them now, so that the row phase,
+            // which starts after the slices, finds them there
+            const size_t r0 = reinterpret_cast<size_t>(img + B.img_hdr());
+            const size_t r1 = reinterpret_cast<size_t>(imgd + __ldg(reinterpret_cast<const int*>(img)));
+            for (size_t a = r0 + size_t(tid) * 128; a < r1; a += size_t(K3_LINK_THREADS) * 128)
+                asm volatile("prefetch.global.L2 [%0];" ::"l"(a));
+        }
         if (slicer) {
             double value = reinterpret_cast<const double*>(img + B.img_lc())[li * 3 + e];
             double grad[NF] = {0, 0, 0, 0, 0, 0, 0};
